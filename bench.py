@@ -27,6 +27,10 @@ main entry), batch 8 per GPU, weak scaling.  ``workloads`` carries the same numb
                   BASELINE configs[0] (model_ad, batch 2).
 ``--impl reference`` times that CPU port alone (batch 2 per step -- stated in config.workload -- honouring --steps/--warmup)
                   and prints the same line shape with "impl": "reference".
+``--dump-outputs DIR`` writes what the last timed step of each measured workload computed -- the losses and model outputs
+                  it returns and the parameters, gradients and buffers it updates in place -- as DIR/<workload>.<name>.npy
+                  (float32, or float64 for integer buffers).  Inputs, weights and dropout masks are seeded, so two builds
+                  run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -58,6 +62,9 @@ WORKLOADS = {
     "mnet": ("Mnet", dict(), 2, "Mnet / MiSePyNet baseline (kfold_train_Mnet.py) train step"),
 }
 CPU_SAMPLE_BATCH = 2      # BASELINE configs[0] / the reference's default --batch_size
+OUTPUT_NAMES = ("logits", "d_mri_logits", "d_pet_logits")      # model_ad / model_CNN_ad return all three, the others logits
+LOSS_NAMES = ("loss_total", "loss_ce", "loss_ad")
+DUMP_BYTES = 64 * 10 ** 6                                      # --dump-outputs: all .npy files together stay below this
 
 
 def conv_flops_per_subject(shape, dim=128, towers=2, first_layer=True, other_layers=True):
@@ -116,6 +123,42 @@ def library_hash():
     with open(_lib.LIB_PATH, "rb") as f:
         so = hashlib.sha256(f.read()).hexdigest()[:16]
     return {"so_sha256_16": so, "sources_sha256_16": build.source_hash()[:16], "built_from": build.recorded_hash()[:16]}
+
+
+def step_arrays(model, outs, step_losses):
+    """Host copies of what one train step gave its caller: the losses and model outputs it returned, and the parameters,
+    gradients and buffers (BatchNorm statistics) it left in the model.  Integer buffers become float64, the rest float32."""
+    def host(t):
+        t = t.detach()
+        return (t.float() if t.is_floating_point() else t.double()).cpu().numpy()
+
+    arrays = {name: host(t) for name, t in zip(LOSS_NAMES, step_losses) if t is not None}
+    arrays.update({name: host(t) for name, t in zip(OUTPUT_NAMES, outs)})
+    for k, p in model.named_parameters():
+        arrays[f"param.{k}"] = host(p)
+        if p.grad is not None:
+            arrays[f"grad.{k}"] = host(p.grad)
+    arrays.update({f"buffer.{k}": host(b) for k, b in model.named_buffers()})
+    return arrays
+
+
+def write_dump(path, arrays):
+    """Write ``{name: array}`` as path/<name>.npy.  Past DUMP_BYTES every array keeps the same fraction of its elements,
+    at positions (of the flattened array, ascending) drawn from a generator seeded with the array's name: runs with the
+    same arguments store the same positions."""
+    import zlib
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    per_file = 128 + 8                               # .npy header, and the one element a tiny array keeps
+    total = sum(a.nbytes for a in arrays.values())
+    frac = min(1.0, (DUMP_BYTES - per_file * len(arrays)) / max(total, 1))
+    for name, a in arrays.items():
+        if frac < 1.0:
+            keep = max(1, int(a.size * frac))
+            pos = np.random.default_rng(zlib.crc32(name.encode())).choice(a.size, keep, replace=False)
+            a = a.reshape(-1)[np.sort(pos)]
+        np.save(os.path.join(path, name + ".npy"), a)
+    return {"dir": path, "arrays": len(arrays), "sampled": frac < 1.0}
 
 
 class ClockSampler:
@@ -319,14 +362,16 @@ class Job:
 
 
 def measure(job, workload, B, steps, warmup, mode="graph", optimizer="fused", want_e2e=True, want_roofline=False,
-            sustained_steps=0, sample_clocks=False):
-    """All legs for one workload at per-GPU batch B.  Returns a dict (rank 0 fills the clock record)."""
+            sustained_steps=0, sample_clocks=False, dump=False):
+    """All legs for one workload at per-GPU batch B.  Returns a dict (rank 0 fills the clock record; with ``dump``, rank 0
+    adds ``step_arrays`` of the last timed step under "dump")."""
     from transmf_ad_b200 import _lib
     from transmf_ad_b200.dp import FlatGradReducer
     from transmf_ad_b200.models import mymodel as M
     from transmf_ad_b200.synthetic import make_labels, make_volumes, procedural_state
     rank, world, dev = job.rank, job.world, job.dev
     kind, kwargs, towers, desc = WORKLOADS[workload]
+    torch.manual_seed(0)                                                     # dropout masks: the same in every run
     if kind == "Mnet":
         from transmf_ad_b200.models.MiSePyNet import Mnet
         model = Mnet()
@@ -367,12 +412,17 @@ def measure(job, workload, B, steps, warmup, mode="graph", optimizer="fused", wa
         ce = ce_fn(outs[0], label)                           # kfold_train_single.py:105
         return ce, None, ce
 
+    last = {}                                                # eager mode with dump: what the latest step returned
+
     def train_step(batch, read_losses):                      # the reference's eager loop
         mri, pet, label = batch
         opt.zero_grad()
         outs = model(mri) if towers == 1 else model(mri, pet)
         outs = outs if isinstance(outs, tuple) else (outs,)
         ce, ad, total = losses(outs, label)
+        if dump:                                             # detached: a kept autograd graph breaks the graph capture
+            last["outs"] = tuple(o.detach() for o in outs)
+            last["losses"] = tuple(None if t is None else t.detach() for t in (total, ce, ad))
         vals = None
         if read_losses:                                      # the reference's two .item() syncs (:127-128)
             vals = (ce.item(), ad.item() if ad is not None else 0.0)
@@ -418,6 +468,12 @@ def measure(job, workload, B, steps, warmup, mode="graph", optimizer="fused", wa
     res = {"workload": workload, "desc": desc, "batch_per_gpu": B, "value": world * B / (ms_per_step * 1e-3),
            "ms_per_step": ms_per_step, "gpu_launches": int(launches), "clocks": clocks, "steps": steps,
            "launches_per_step": int(launches // max(steps, 1))}
+    if dump and rank == 0:
+        if graph_mode:
+            outs, step_losses = graphed.outputs, graphed.losses
+        else:
+            outs, step_losses = last["outs"], last["losses"]
+        res["dump"] = step_arrays(model, outs if isinstance(outs, tuple) else (outs,), step_losses)
 
     # ---- end-to-end: pinned host buffers, H2D inside the timed region, loss reads ------------------------------------
     if want_e2e:
@@ -565,7 +621,13 @@ def main():
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the eager_dropin / sustained / c4 sub-records")
     ap.add_argument("--sustained-steps", type=int, default=2000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the last timed step computed as DIR/<workload>.<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path; --impl reference times the CPU port")
     if args.impl == "reference":
         run_reference_arm(args, int(os.environ.get("RANK", "0")))
         return
@@ -575,12 +637,17 @@ def main():
     rank, world = job.rank, job.world
     B = args.batch
     head_name = "ad" if args.workload == "both" else args.workload
+    dump = args.dump_outputs is not None
     head = measure(job, head_name, B, args.steps, args.warmup, args.mode, args.optimizer, want_e2e=True,
                    want_roofline=(not args.no_roofline) and head_name != "mnet", sample_clocks=True,
-                   sustained_steps=(args.sustained_steps if (world == 1 and not args.no_extras and args.mode == "graph") else 0))
+                   sustained_steps=(args.sustained_steps if (world == 1 and not args.no_extras and args.mode == "graph") else 0),
+                   dump=dump)
+    dumped = {f"{head_name}.{k}": v for k, v in head.pop("dump", {}).items()}
     others = {}
     if args.workload == "both":
-        r = measure(job, "cnn_ad", B, args.steps, args.warmup, args.mode, args.optimizer, want_e2e=True, want_roofline=False)
+        r = measure(job, "cnn_ad", B, args.steps, args.warmup, args.mode, args.optimizer, want_e2e=True, want_roofline=False,
+                    dump=dump)
+        dumped.update({f"cnn_ad.{k}": v for k, v in r.pop("dump", {}).items()})
         others["cnn_ad"] = {k: r[k] for k in ("desc", "batch_per_gpu", "value", "ms_per_step", "e2e", "launches_per_step")}
     extras = {}
     if not args.no_extras and world == 1 and args.mode == "graph":
@@ -609,6 +676,8 @@ def main():
                                   "its kernels are ATen's)"}
 
     if rank == 0:
+        if dump:
+            print(f"[bench] --dump-outputs: {write_dump(args.dump_outputs, dumped)}", file=sys.stderr)
         graph_mode = args.mode == "graph"
         line = {
             "metric": METRIC, "value": head["value"], "unit": "subjects/s", "n_gpus": world, "steps": args.steps,
