@@ -107,6 +107,24 @@ int tmf_conv1_bwd_fused_presplit(int ng, const void* const* dout, const void* co
                                  const float* const* bcoef, float* const* dw, int B, int D, int H, int W, int cout,
                                  float slope, void* ws, size_t ws_bytes, void* stream);
 
+/* Block-1 gradient with respect to the input image (saliency maps, integrated gradients, input-space attacks): the
+ * BatchNorm + LeakyReLU + MaxPool3d(2,2) backward "apply" (dy recomputed from the stored y exactly as
+ * tmf_bn_act_pool_bwd_apply computes it with pool = TMF_POOL_MAX; never written to HBM on the tcgen05 path) followed by
+ * the data gradient of conv1.0:  dx[p] = sum_tap sum_co dy[p - off(tap)][co] * w[co][tap]  (zero padding 1).
+ * dout: bf16 pooled gradient [B,D/2,H/2,W/2,Cout]; y: bf16 conv1.0 output [B,D,H,W,Cout]; coef / bcoef as below;
+ * w: fp32 conv1.0 weight (Cout,1,3,3,3); dx: fp32 [B,D,H,W] (= (B,1,D,H,W)), overwritten, every element written once in a
+ * fixed summation order (no atomics: bitwise reproducible, and a tower's result does not depend on ng).
+ * impl: TMF_CONV_UMMA (tcgen05, Cout = 32, W <= 128; the weight as bf16 hi + lo halves, fp32-level accuracy),
+ * TMF_CONV_DIRECT (CUDA cores: tmf_bn_act_pool_bwd_apply into the workspace, then an fp32 direct kernel; Cout a multiple
+ * of 8 in [8,64]) or TMF_CONV_AUTO (tcgen05 where supported, else direct).  `ws`: caller-owned, 256-byte aligned scratch
+ * of at least tmf_conv1_dgrad_fused_workspace_bytes(...) bytes; may be NULL when that returns 0.
+ * reference models/networks.py:22-25 (autograd backward of Conv3d(1,32,3,p1) / BatchNorm3d / LeakyReLU / MaxPool3d
+ * with respect to the image) */
+int tmf_conv1_dgrad_fused(int ng, const void* const* dout, const void* const* y, const float* const* coef,
+                          const float* const* bcoef, const float* const* w, float* const* dx, int B, int D, int H, int W,
+                          int cout, float slope, int impl, void* ws, size_t ws_bytes, void* stream);
+int64_t tmf_conv1_dgrad_fused_workspace_bytes(int ng, int impl, int B, int D, int H, int W, int cout);
+
 /* 3x3x3 (pad 1) or 1x1x1 convolution, bf16 NDHWC input a[B,D,H,W,Cin], packed bf16 weights wf[tap][Cout][Cin],
  * optional fp32 bias, bf16 output y[B,D,H,W,Cout], optional stats (as above; NULL array = none).
  * Also used for dgrad (a = dy, wf = flipped/transposed pack, bias = stats = NULL).

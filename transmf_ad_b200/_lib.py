@@ -27,6 +27,7 @@ SIGNATURES = {
     "tmf_conv1_bwd_fused": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp, C.c_size_t, _vp],
     "tmf_conv1_bwd_split_x": [_i, _pp, _i, _i, _i, _i, _i, _vp, C.c_size_t, _vp],
     "tmf_conv1_bwd_fused_presplit": [_i, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp, C.c_size_t, _vp],
+    "tmf_conv1_dgrad_fused": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _i, _vp, C.c_size_t, _vp],
     "tmf_conv3d_fwd": [_i, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "tmf_conv3d_wgrad": [_i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, C.c_size_t, _vp],
     "tmf_bn_finalize": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i64, _f, _f, _i, _vp],
@@ -76,7 +77,8 @@ PLAIN = {"tmf_last_error": (C.c_char_p, []), "tmf_version": (_i, []), "tmf_check
          "tmf_conv3d_wgrad_workspace_bytes": (_i64, [_i] * 9),
          "tmf_conv3d_umma_plan_info": (_i, [_i] * 8 + [C.POINTER(C.c_int)]),
          "tmf_conv3d_col_plan_info": (_i, [_i] * 7 + [C.POINTER(C.c_int)]),
-         "tmf_conv1_bwd_fused_workspace_bytes": (_i64, [_i] * 6), "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
+         "tmf_conv1_bwd_fused_workspace_bytes": (_i64, [_i] * 6), "tmf_conv1_dgrad_fused_workspace_bytes": (_i64, [_i] * 7),
+         "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
 
 _lib = None
 _device_checked = False

@@ -233,9 +233,6 @@ class SNetFunction(torch.autograd.Function):
         if not isinstance(run, SNetRun):
             run = SNetRun(bool(run), True)
         training = run.training
-        if run.grad_enabled and any(ctx.needs_input_grad[4:4 + ng]):
-            raise RuntimeError("sNet: gradients with respect to the input volumes are not implemented (conv1.0 has no "
-                               "dgrad kernel); detach the inputs or compute saliency with the reference modules")
         xs = [_f32c(a) for a in args[:ng]]
         params = args[ng:]
         assert len(params) == ng * 7 * 4
@@ -246,7 +243,9 @@ class SNetFunction(torch.autograd.Function):
             if tuple(x.shape) != tuple(xs[0].shape):
                 raise RuntimeError("MRI and PET volumes must have the same shape")
         dev = xs[0].device
-        need_grad = run.grad_enabled and any(ctx.needs_input_grad[4 + ng:])
+        need_wgrad = run.grad_enabled and any(ctx.needs_input_grad[4 + ng:])
+        need_xgrad = run.grad_enabled and any(ctx.needs_input_grad[4:4 + ng])     # saliency: d / d input volume
+        need_grad = need_wgrad or need_xgrad
         impl = conv_impl()
         P = lambda t, l, k: params[(t * 7 + l) * 4 + k]
         if not training and not need_grad and run.folds is not None and os.environ.get("TMF_EVAL_FOLD", "1") != "0":
@@ -322,7 +321,7 @@ class SNetFunction(torch.autograd.Function):
         # and 4.295 ms without -- the parallel branch costs the kernels it overlaps what it saves the backward pass.
         ctx.c1split = None
         cout0, pool0 = spec.layers[0][1], spec.layers[0][3]
-        if (need_grad and pool0 == L.POOL_MAX and impl != L.CONV_DIRECT and len(spec.layers) > 1
+        if (need_wgrad and pool0 == L.POOL_MAX and impl != L.CONV_DIRECT and len(spec.layers) > 1
                 and os.environ.get("TMF_C1B_PRESPLIT", "0") != "0"):
             nws0 = int(L.load().tmf_conv1_bwd_fused_workspace_bytes(ng, B, D, H, W, cout0))
             if nws0 > 0:
@@ -343,6 +342,8 @@ class SNetFunction(torch.autograd.Function):
         ctx.sync_group, ctx.sync_world = run.sync_group, sync_world
         ctx.params = params if need_grad else None          # references only (gradient slots of the flat DP buffer)
         ctx.impl = impl
+        ctx.need_wgrad = need_wgrad
+        ctx.x_dtypes = [a.dtype for a in args[:ng]]
         outs = tuple(o.permute(0, 4, 1, 2, 3) for o in act)      # logical (B,C,d,h,w), channels-last memory
         return outs if ng > 1 else outs[0]
 
@@ -407,6 +408,11 @@ class SNetFunction(torch.autograd.Function):
             dout.append(g)
         dout_fp32 = 1
         pgrads = [None] * (ng * 7 * 4)
+        need_w = ctx.need_wgrad
+        # frozen weights (saliency): no weight-gradient launches, no parameter .grad; BatchNorm's parameter gradients
+        # still come out of tmf_bn_bwd_finalize (next to bcoef, which the input gradient needs) into scratch
+        xg = [t for t in range(ng) if ctx.needs_input_grad[4 + t]]
+        dxs = [None] * ng
         for l in range(len(spec.layers) - 1, -1, -1):
             cin, cout, ks, pool = spec.layers[l]
             act, y, coef, wd, (Dl, Hl, Wl), ymax = saved[l]
@@ -421,9 +427,12 @@ class SNetFunction(torch.autograd.Function):
                 L.call("tmf_bn_act_pool_bwd_reduce", ng, L.ptrs(dout), dout_fp32, L.ptrs(y), L.ptrs(coef), L.ptrs(sums),
                        B, Dl, Hl, Wl, cout, pool, slope, tag=f"tmf_bn_act_pool_bwd_reduce@L{l}")
             PG = lambda t, k: ctx.params[(t * 7 + l) * 4 + k]
-            dbias = [grad_out(PG(t, 1)) for t in range(ng)]
-            dgamma = [grad_out(PG(t, 2)) for t in range(ng)]
-            dbeta = [grad_out(PG(t, 3)) for t in range(ng)]
+            if need_w:
+                dbias = [grad_out(PG(t, 1)) for t in range(ng)]
+                dgamma = [grad_out(PG(t, 2)) for t in range(ng)]
+                dbeta = [grad_out(PG(t, 3)) for t in range(ng)]
+            else:
+                dbias, dgamma, dbeta = (list(s.unbind(0)) for s in torch.empty((3, ng, cout), dtype=torch.float32, device=dev))
             bcoef = list(torch.empty((ng, 2 * cout), dtype=torch.float32, device=dev).unbind(0))
             L.call("tmf_bn_bwd_finalize", ng, L.ptrs(sums), L.ptrs(coef), L.ptrs(dgamma), L.ptrs(dbeta),
                    L.ptrs(dbias), L.ptrs(bcoef), cout, count, int(training))
@@ -434,7 +443,22 @@ class SNetFunction(torch.autograd.Function):
                 scratch_g = list(torch.empty((3 * ng, cout), dtype=torch.float32, device=dev).unbind(0))
                 L.call("tmf_bn_bwd_finalize", ng, L.ptrs(sums), L.ptrs(coef), L.ptrs(scratch_g[:ng]), L.ptrs(scratch_g[ng:2 * ng]),
                        L.ptrs(scratch_g[2 * ng:]), L.ptrs(bcoef), cout, count * ctx.sync_world, int(training))
-            dw = [grad_out(PG(t, 0)) for t in range(ng)]
+            if l == 0 and xg:
+                if dout_fp32:
+                    raise RuntimeError("sNet backward: the input gradient needs a bf16 pooled gradient into block 1")
+                w0 = [PG(t, 0) for t in xg]
+                dx = [torch.empty((B, 1, Dl, Hl, Wl), dtype=torch.float32, device=dev) for _ in xg]
+                nws = int(L.load().tmf_conv1_dgrad_fused_workspace_bytes(len(xg), ctx.impl, B, Dl, Hl, Wl, cout))
+                ws = torch.empty(nws, dtype=torch.uint8, device=dev) if nws > 0 else None
+                L.call("tmf_conv1_dgrad_fused", len(xg), L.ptrs([dout[t] for t in xg]), L.ptrs([y[t] for t in xg]),
+                       L.ptrs([coef[t] for t in xg]), L.ptrs([bcoef[t] for t in xg]), L.ptrs(w0), L.ptrs(dx),
+                       B, Dl, Hl, Wl, cout, slope, ctx.impl, L.ptr(ws), nws)
+                for t, d in zip(xg, dx):
+                    dxs[t] = d if ctx.x_dtypes[t] == torch.float32 else d.to(ctx.x_dtypes[t])
+            if l == 0 and not need_w:
+                saved[l] = None
+                continue
+            dw = [grad_out(PG(t, 0)) for t in range(ng)] if need_w else None
             fused_ws = 0
             if l == 0 and pool == L.POOL_MAX and not dout_fp32 and ctx.impl != L.CONV_DIRECT:
                 fused_ws = int(L.load().tmf_conv1_bwd_fused_workspace_bytes(ng, B, Dl, Hl, Wl, cout))
@@ -462,18 +486,20 @@ class SNetFunction(torch.autograd.Function):
                 L.call("tmf_conv1_wgrad", ng, L.ptrs(dy), L.ptrs(act), L.ptrs(dw), B, Dl, Hl, Wl, cout, ctx.impl,
                        L.ptr(ws), nws)
             else:
-                ws = wgrad_workspace(ng, ctx.impl, B, Dl, Hl, Wl, cin, cout, ks, dev)
-                L.call("tmf_conv3d_wgrad", ng, L.ptrs(dy), L.ptrs(act), L.ptrs(dw), B, Dl, Hl, Wl, cin, cout, ks,
-                       ctx.impl, L.ptr(ws), 0 if ws is None else ws.numel(), tag=f"tmf_conv3d_wgrad@L{l}")
+                if need_w:
+                    ws = wgrad_workspace(ng, ctx.impl, B, Dl, Hl, Wl, cin, cout, ks, dev)
+                    L.call("tmf_conv3d_wgrad", ng, L.ptrs(dy), L.ptrs(act), L.ptrs(dw), B, Dl, Hl, Wl, cin, cout, ks,
+                           ctx.impl, L.ptr(ws), 0 if ws is None else ws.numel(), tag=f"tmf_conv3d_wgrad@L{l}")
                 da = [torch.empty((B, Dl, Hl, Wl, cin), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
                 L.call("tmf_conv3d_fwd", ng, L.ptrs(dy), L.ptrs(wd), L.ptrs(None), L.ptrs(da), L.ptrs(None),
                        B, Dl, Hl, Wl, cout, cin, ks, ctx.impl, tag=f"tmf_conv3d_dgrad@L{l}")
                 dout, dout_fp32 = da, 0
-            SNetFunction._layer_grads(ctx, pgrads, l, dw, dbias, dgamma, dbeta)
+            if need_w:
+                SNetFunction._layer_grads(ctx, pgrads, l, dw, dbias, dgamma, dbeta)
             saved[l] = None
         ctx.saved = None
         ctx.params = None
-        return (None, None, None, None) + (None,) * ng + tuple(pgrads)
+        return (None, None, None, None) + tuple(dxs) + tuple(pgrads)
 
     @staticmethod
     def _layer_grads(ctx, pgrads, l, dw, dbias, dgamma, dbeta):
