@@ -173,6 +173,21 @@ int tmf_bn_act_pool_fwd(int ng, const void* const* y, const float* const* coef, 
 int tmf_bn_act_pool_fwd_keepmax(int ng, const void* const* y, const float* const* coef, void* const* out,
                                 void* const* ymax, int out_fp32, int B, int D, int H, int W, int C, float slope,
                                 void* stream);
+/* Dual-output variants of the two passes above for a block boundary whose output is exposed (module hooks on the sNet
+ * blocks, Grad-CAM): out (bf16, the next conv's operand) and ymax are the same bits as tmf_bn_act_pool_fwd /
+ * tmf_bn_act_pool_fwd_keepmax write with out_fp32 = 0, and out32 (fp32, same layout) receives the value before rounding,
+ * i.e. the fp32 number whose round-to-nearest bf16 is out.  networks.py:25,34,43,52 (the nn.Sequential block outputs). */
+int tmf_bn_act_pool_fwd_dual(int ng, const void* const* y, const float* const* coef, void* const* out,
+                             float* const* out32, int B, int D, int H, int W, int C, int pool, float slope, void* stream);
+int tmf_bn_act_pool_fwd_keepmax_dual(int ng, const void* const* y, const float* const* coef, void* const* out,
+                                     float* const* out32, void* const* ymax, int B, int D, int H, int W, int C, float slope,
+                                     void* stream);
+/* n elements (a multiple of 8) bf16 -> fp32 (exact) and fp32 -> bf16 (round to nearest even), per tower: the gradient at
+ * an exposed block boundary (the bf16 dgrad output widened for autograd; an fp32 gradient narrowed for block 1's fused
+ * backward kernels). */
+int tmf_widen_bf16(int ng, const void* const* src, float* const* dst, int64_t n, void* stream);
+int tmf_narrow_f32(int ng, const float* const* src, void* const* dst, int64_t n, void* stream);
+
 /* sums[TMF_STAT_ROWS][2*C] (double partial rows) = {sum dz, sum dz*xhat} of a max-pool layer from ymax and dout (both at pooled extents Do,Ho,Wo):
  * same result as tmf_bn_act_pool_bwd_reduce(pool = TMF_POOL_MAX) up to summation order. */
 int tmf_bn_maxpool_bwd_reduce_kept(int ng, const void* const* dout, int dout_fp32, const void* const* ymax,
@@ -283,6 +298,19 @@ int tmf_token_pool_bwd(const float* dmean, const float* dmax, const int32_t* arg
  * 1-element device tensor lambda (no host sync), or alpha = -lambda.  reference
  * models/gradient_reversal/functional.py:11-16 */
 int tmf_scale(const float* x, float* y, float alpha, const float* alpha_dev, int64_t n, void* stream);
+
+/* ---- Grad-CAM on an sNet block (Selvaraju et al. 2017; pytorch-grad-cam conventions) ---------------------------------
+ * A, G: fp32 [B,d,h,w,C] per tower (block activation and its gradient, channels-last).  alpha[b,c] = mean_p G[b,p,c] (double,
+ * per-chunk partial rows in `ws` added in index order: no atomics, bitwise reproducible, a tower's bits do not depend on ng);
+ * cam[b,p] = ReLU(sum_c alpha[b,c] A[b,p,c]).  upsample != 0: trilinear to D x H x W (F.interpolate(mode="trilinear",
+ * align_corners=False)); else the map is d x h x w.  normalize != 0: (cam - min) / (max - min + 1e-7) per sample over the
+ * returned map (a map that is zero everywhere stays zero).  cam: fp32 [B, D,H,W] (or [B,d,h,w]), overwritten.  C a multiple
+ * of 4 in [4,1024], A / G 16-byte aligned; `ws`: caller-owned, 256-byte aligned, at least tmf_gradcam_workspace_bytes(...)
+ * bytes (which returns -1 for an unsupported problem). */
+int64_t tmf_gradcam_workspace_bytes(int ng, int B, int d, int h, int w, int C, int D, int H, int W, int upsample,
+                                    int normalize);
+int tmf_gradcam(int ng, const float* const* A, const float* const* G, float* const* cam, int B, int d, int h, int w, int C,
+                int D, int H, int W, int upsample, int normalize, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- inference (SURVEY.md section 8f row 2; reference kfold_train_adversarial.py:144-187) ------------------------------------
  * Eval-mode BatchNorm3d folded into the conv operands: scale = gamma*rsqrt(running_var + eps); wf (bf16

@@ -112,6 +112,7 @@ struct ActPoolArgs {
   GroupPtr<__nv_bfloat16> dy;         // bwd apply output
   GroupPtr<double> sums;              // bwd reduce output
   GroupPtr<__nv_bfloat16> ymax;       // fwd (max pool, optional): the pre-BN value behind each window's maximum
+  GroupPtr<float> out32;              // fwd, dual-output variants: the fp32 value whose bf16 rounding is `out`
   int B, D, H, W, C, pool, fp32io;
   int Do, Ho, Wo;                     // forward output dims (floor)
   int Dc, Hc, Wc;                     // ceil dims (windows that touch any input voxel)
@@ -142,8 +143,9 @@ __device__ __forceinline__ void store8f(void* base, int64_t elem_off, int fp32, 
 // maximum (first maximum in (d,h,w) scan order, torch's rule).  The backward reduction of a max-pool layer needs y
 // only there (dz is zero elsewhere), so it can run on ymax + dout at pooled resolution instead of re-reading all of y:
 // block 1 re-read 925 MB per step for two per-channel sums.
-template <bool KEEP>
-__global__ void __launch_bounds__(256, KEEP ? 3 : 4) bn_act_pool_fwd_kernel(ActPoolArgs p) {
+// DUAL: also store the fp32 value o in out32 (same layout as out); out (bf16) and ymax are the same bits as without it.
+template <bool KEEP, bool DUAL = false>
+__global__ void __launch_bounds__(256, DUAL ? 2 : (KEEP ? 3 : 4)) bn_act_pool_fwd_kernel(ActPoolArgs p) {
   pdl_entry();
   const int g = blockIdx.z;
   const int CQ = p.C >> 3;
@@ -207,7 +209,9 @@ __global__ void __launch_bounds__(256, KEEP ? 3 : 4) bn_act_pool_fwd_kernel(ActP
         for (int j = 0; j < 8; ++j) o[j] *= 0.125f;
       }
     }
-    store8f(p.out.p[g], ((((int64_t)n * p.Do + dd) * p.Ho + ho) * p.Wo + wo) * p.C + c0, p.fp32io, o);
+    const int64_t ooff = ((((int64_t)n * p.Do + dd) * p.Ho + ho) * p.Wo + wo) * p.C + c0;
+    store8f(p.out.p[g], ooff, p.fp32io, o);
+    if (DUAL) store8f(p.out32.p[g], ooff, 1, o);
    }
   }
 }
@@ -658,6 +662,36 @@ int tmf_bn_act_pool_fwd_keepmax(int ng, const void* const* y, const float* const
     return 1;
   dim3 grid(plan_units(B, p.Do, p.Ho, 148 * 8, &p.nch, &p.hcr), 1, ng);
   launch_k(bn_act_pool_fwd_kernel<true>, grid, 256, 0, (cudaStream_t)stream, p);
+  TMF_LAUNCH_CHECK();
+  return 0;
+}
+
+int tmf_bn_act_pool_fwd_dual(int ng, const void* const* y, const float* const* coef, void* const* out,
+                             float* const* out32, int B, int D, int H, int W, int C, int pool, float slope, void* stream) {
+  TMF_CHECK_NG(ng);
+  ActPoolArgs p{};
+  if (fill_args(p, B, D, H, W, C, pool, slope, 0)) return 1;
+  if (!load_group(p.y, (const __nv_bfloat16* const*)y, ng, true, "y") || !load_group(p.coef, coef, ng, true, "coef") ||
+      !load_group(p.out, (void* const*)out, ng, true, "out") || !load_group(p.out32, out32, ng, true, "out32"))
+    return 1;
+  dim3 grid(plan_units(B, p.Do, p.Ho, 148 * 8, &p.nch, &p.hcr), 1, ng);
+  launch_k(bn_act_pool_fwd_kernel<false, true>, grid, 256, 0, (cudaStream_t)stream, p);
+  TMF_LAUNCH_CHECK();
+  return 0;
+}
+
+int tmf_bn_act_pool_fwd_keepmax_dual(int ng, const void* const* y, const float* const* coef, void* const* out,
+                                     float* const* out32, void* const* ymax, int B, int D, int H, int W, int C, float slope,
+                                     void* stream) {
+  TMF_CHECK_NG(ng);
+  ActPoolArgs p{};
+  if (fill_args(p, B, D, H, W, C, TMF_POOL_MAX, slope, 0)) return 1;
+  if (!load_group(p.y, (const __nv_bfloat16* const*)y, ng, true, "y") || !load_group(p.coef, coef, ng, true, "coef") ||
+      !load_group(p.out, (void* const*)out, ng, true, "out") || !load_group(p.out32, out32, ng, true, "out32") ||
+      !load_group(p.ymax, (__nv_bfloat16* const*)ymax, ng, true, "ymax"))
+    return 1;
+  dim3 grid(plan_units(B, p.Do, p.Ho, 148 * 8, &p.nch, &p.hcr), 1, ng);
+  launch_k(bn_act_pool_fwd_kernel<true, true>, grid, 256, 0, (cudaStream_t)stream, p);
   TMF_LAUNCH_CHECK();
   return 0;
 }

@@ -87,6 +87,16 @@ class SNetSpec:
         self.dim = dim
 
 
+class SNetSegment:
+    """Layers [l0, l1) of an sNet, passed to ``SNetFunction.apply`` in the place of the spec: a segmented run (module hooks on
+    the blocks, Grad-CAM; DESIGN section 3.7) chains one autograd node per segment, split at the exposed block outputs.
+    A segment with l0 > 0 consumes ``src``, the bf16 NDHWC twins of its fp32 inputs (what the previous segment returned);
+    a segment with l1 < 7 returns the fp32 block outputs followed by their bf16 twins (not differentiable)."""
+
+    def __init__(self, spec, l0, l1, src=None):
+        self.spec, self.l0, self.l1, self.src = spec, l0, l1, src
+
+
 class ConvPack:
     """bf16 operand packs of one Conv3d weight -- wf[tap][Cout][Cin] (forward) and wd[taps-1-tap][Cin][Cout] (dgrad) -- kept
     across steps.  They are fresh while ``weight._version`` is the one they were packed from: torch in-place updates
@@ -233,15 +243,26 @@ class SNetFunction(torch.autograd.Function):
         if not isinstance(run, SNetRun):
             run = SNetRun(bool(run), True)
         training = run.training
-        xs = [_f32c(a) for a in args[:ng]]
+        seg = spec if isinstance(spec, SNetSegment) else None
+        if seg is not None:
+            spec = seg.spec
+        l0, l1 = (seg.l0, seg.l1) if seg is not None else (0, len(spec.layers))
+        tap_out = l1 < len(spec.layers)
         params = args[ng:]
         assert len(params) == ng * 7 * 4
-        B, cin0, D, H, W = xs[0].shape
-        if cin0 != 1:
-            raise RuntimeError(f"sNet expects single-channel volumes (B,1,D,H,W); got {tuple(xs[0].shape)}")
-        for x in xs:
-            if tuple(x.shape) != tuple(xs[0].shape):
-                raise RuntimeError("MRI and PET volumes must have the same shape")
+        if l0 == 0:
+            xs = [_f32c(a) for a in args[:ng]]
+            B, cin0, D, H, W = xs[0].shape
+            if cin0 != 1:
+                raise RuntimeError(f"sNet expects single-channel volumes (B,1,D,H,W); got {tuple(xs[0].shape)}")
+            for x in xs:
+                if tuple(x.shape) != tuple(xs[0].shape):
+                    raise RuntimeError("MRI and PET volumes must have the same shape")
+        else:
+            xs = seg.src                                    # bf16 twins of the fp32 block outputs args[:ng]
+            B, D, H, W, cin0 = xs[0].shape
+            if cin0 != spec.layers[l0][0] or any(tuple(x.shape) != tuple(xs[0].shape) for x in xs):
+                raise RuntimeError(f"sNet segment from layer {l0}: unexpected input {tuple(xs[0].shape)}")
         dev = xs[0].device
         need_wgrad = run.grad_enabled and any(ctx.needs_input_grad[4 + ng:])
         need_xgrad = run.grad_enabled and any(ctx.needs_input_grad[4:4 + ng])     # saliency: d / d input volume
@@ -249,14 +270,15 @@ class SNetFunction(torch.autograd.Function):
         impl = conv_impl()
         P = lambda t, l, k: params[(t * 7 + l) * 4 + k]
         if not training and not need_grad and run.folds is not None and os.environ.get("TMF_EVAL_FOLD", "1") != "0":
-            return SNetFunction._eval_forward(ctx, spec, run, buffers, ng, xs, P, impl)
+            return SNetFunction._eval_forward(ctx, spec, run, buffers, ng, xs, P, impl, l0, l1)
         if training:
             bump_param_epoch()                              # running statistics are about to change
         saved = []
         act = xs
         dims = (D, H, W)
         sync_world = _sync_world(run.sync_group) if training else 1
-        for l, (cin, cout, ks, pool) in enumerate(spec.layers):
+        for l in range(l0, l1):
+            cin, cout, ks, pool = spec.layers[l]
             Dl, Hl, Wl = dims
             count = B * Dl * Hl * Wl
             bn_eps, bn_momentum, slope = run.hyper[l]
@@ -298,13 +320,22 @@ class SNetFunction(torch.autograd.Function):
             Do, Ho, Wo = _pooled(Dl, Hl, Wl, pool)
             out = [torch.empty((B, Do, Ho, Wo, cout), dtype=torch.float32 if last else torch.bfloat16, device=dev)
                    for _ in range(ng)]
+            dual = tap_out and l == l1 - 1                  # exposed block output: fp32 value + the bf16 operand
+            out32 = [torch.empty((B, Do, Ho, Wo, cout), dtype=torch.float32, device=dev) for _ in range(ng)] if dual else None
             ymax = None
             if need_grad and pool == L.POOL_MAX and keep_ymax():
                 # max-pool layers keep the pre-BN value behind every window maximum: the backward reduction then reads
                 # 1/8 of the voxels instead of all of y
                 ymax = [torch.empty((B, Do, Ho, Wo, cout), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
-                L.call("tmf_bn_act_pool_fwd_keepmax", ng, L.ptrs(y), L.ptrs(coef), L.ptrs(out), L.ptrs(ymax), int(last),
-                       B, Dl, Hl, Wl, cout, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
+                if dual:
+                    L.call("tmf_bn_act_pool_fwd_keepmax_dual", ng, L.ptrs(y), L.ptrs(coef), L.ptrs(out), L.ptrs(out32),
+                           L.ptrs(ymax), B, Dl, Hl, Wl, cout, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
+                else:
+                    L.call("tmf_bn_act_pool_fwd_keepmax", ng, L.ptrs(y), L.ptrs(coef), L.ptrs(out), L.ptrs(ymax), int(last),
+                           B, Dl, Hl, Wl, cout, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
+            elif dual:
+                L.call("tmf_bn_act_pool_fwd_dual", ng, L.ptrs(y), L.ptrs(coef), L.ptrs(out), L.ptrs(out32), B, Dl, Hl, Wl,
+                       cout, pool, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
             else:
                 L.call("tmf_bn_act_pool_fwd", ng, L.ptrs(y), L.ptrs(coef), L.ptrs(out), int(last), B, Dl, Hl, Wl, cout,
                        pool, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
@@ -321,7 +352,7 @@ class SNetFunction(torch.autograd.Function):
         # and 4.295 ms without -- the parallel branch costs the kernels it overlaps what it saves the backward pass.
         ctx.c1split = None
         cout0, pool0 = spec.layers[0][1], spec.layers[0][3]
-        if (need_wgrad and pool0 == L.POOL_MAX and impl != L.CONV_DIRECT and len(spec.layers) > 1
+        if (need_wgrad and l0 == 0 and pool0 == L.POOL_MAX and impl != L.CONV_DIRECT and len(spec.layers) > 1
                 and os.environ.get("TMF_C1B_PRESPLIT", "0") != "0"):
             nws0 = int(L.load().tmf_conv1_bwd_fused_workspace_bytes(ng, B, D, H, W, cout0))
             if nws0 > 0:
@@ -344,17 +375,30 @@ class SNetFunction(torch.autograd.Function):
         ctx.impl = impl
         ctx.need_wgrad = need_wgrad
         ctx.x_dtypes = [a.dtype for a in args[:ng]]
+        ctx.l0, ctx.l1 = l0, l1
+        if tap_out:
+            return SNetFunction._tap_outputs(ctx, out32, act)
         outs = tuple(o.permute(0, 4, 1, 2, 3) for o in act)      # logical (B,C,d,h,w), channels-last memory
         return outs if ng > 1 else outs[0]
 
     @staticmethod
-    def _eval_forward(ctx, spec, run, buffers, ng, xs, P, impl):
+    def _tap_outputs(ctx, out32, twins):
+        """A segment that ends at an exposed block output: the fp32 outputs (B,C,d,h,w, channels-last memory) for autograd
+        and the caller's hooks, then their bf16 twins for the next segment."""
+        ctx.mark_non_differentiable(*twins)
+        ctx.set_materialize_grads(False)
+        return tuple(o.permute(0, 4, 1, 2, 3) for o in out32) + tuple(twins)
+
+    @staticmethod
+    def _eval_forward(ctx, spec, run, buffers, ng, xs, P, impl, l0=0, l1=7):
         """Inference (val_step, reference kfold_train_adversarial.py:144-161): no statistics, no saved activations; the
         BatchNorm of every layer is folded into the conv operands once per weight / running-statistics state."""
-        B, _, D, H, W = xs[0].shape
+        B, D, H, W = (xs[0].shape[0],) + tuple(xs[0].shape[2:]) if l0 == 0 else tuple(xs[0].shape[:4])
         dev = xs[0].device
         act, dims = xs, (D, H, W)
-        for l, (cin, cout, ks, pool) in enumerate(spec.layers):
+        tap_out = l1 < len(spec.layers)
+        for l in range(l0, l1):
+            cin, cout, ks, pool = spec.layers[l]
             Dl, Hl, Wl = dims
             bn_eps, _, slope = run.hyper[l]
             folds = [run.folds[t][l] for t in range(ng)]
@@ -380,6 +424,12 @@ class SNetFunction(torch.autograd.Function):
             Do, Ho, Wo = _pooled(Dl, Hl, Wl, pool)
             out = [torch.empty((B, Do, Ho, Wo, cout), dtype=torch.float32 if last else torch.bfloat16, device=dev)
                    for _ in range(ng)]
+            if tap_out and l == l1 - 1:
+                out32 = [torch.empty((B, Do, Ho, Wo, cout), dtype=torch.float32, device=dev) for _ in range(ng)]
+                L.call("tmf_bn_act_pool_fwd_dual", ng, L.ptrs(y), L.ptrs([fo.ident for fo in folds]), L.ptrs(out),
+                       L.ptrs(out32), B, Dl, Hl, Wl, cout, pool, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
+                ctx.saved = None
+                return SNetFunction._tap_outputs(ctx, out32, out)
             L.call("tmf_bn_act_pool_fwd", ng, L.ptrs(y), L.ptrs([fo.ident for fo in folds]), L.ptrs(out), int(last), B, Dl, Hl,
                    Wl, cout, pool, slope, tag=f"tmf_bn_act_pool_fwd@L{l}")
             act, dims = out, (Do, Ho, Wo)
@@ -390,8 +440,9 @@ class SNetFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, *grads):
         spec, ng, B, training = ctx.spec, ctx.ng, ctx.B, ctx.training
+        l0, l1 = ctx.l0, ctx.l1
         saved = ctx.saved
-        if saved is None or len(saved) != len(spec.layers):
+        if saved is None or len(saved) != l1 - l0:
             raise RuntimeError("sNet backward: the saved activations are gone -- backward through this forward ran "
                                "already (they are freed layer by layer; retain_graph / double backward are not "
                                "supported), or the forward ran without autograd recording")
@@ -399,9 +450,9 @@ class SNetFunction(torch.autograd.Function):
         dout = []
         for t in range(ng):
             g = grads[t]
-            cout = spec.layers[-1][1]
+            cout = spec.layers[l1 - 1][1]
             if g is None:
-                Dl, Hl, Wl = _pooled(*saved[-1][4], spec.layers[-1][3])
+                Dl, Hl, Wl = _pooled(*saved[-1][4], spec.layers[l1 - 1][3])
                 g = torch.zeros((B, Dl, Hl, Wl, cout), dtype=torch.float32, device=dev)
             else:
                 g = _f32c(g.permute(0, 2, 3, 4, 1))
@@ -413,11 +464,16 @@ class SNetFunction(torch.autograd.Function):
         # still come out of tmf_bn_bwd_finalize (next to bcoef, which the input gradient needs) into scratch
         xg = [t for t in range(ng) if ctx.needs_input_grad[4 + t]]
         dxs = [None] * ng
-        for l in range(len(spec.layers) - 1, -1, -1):
+        for l in range(l1 - 1, l0 - 1, -1):
             cin, cout, ks, pool = spec.layers[l]
-            act, y, coef, wd, (Dl, Hl, Wl), ymax = saved[l]
+            act, y, coef, wd, (Dl, Hl, Wl), ymax = saved[l - l0]
             count = B * Dl * Hl * Wl
             slope = ctx.hyper[l][2]
+            if l == 0 and dout_fp32:
+                # a segment of block 1 alone: its fused backward kernels read a bf16 pooled gradient
+                d16 = [torch.empty(d.shape, dtype=torch.bfloat16, device=dev) for d in dout]
+                L.call("tmf_narrow_f32", ng, L.ptrs(dout), L.ptrs(d16), dout[0].numel())
+                dout, dout_fp32 = d16, 0
             sums = L.stat_buffers(ng, cout, dev)
             if ymax is not None:
                 L.call("tmf_bn_maxpool_bwd_reduce_kept", ng, L.ptrs(dout), dout_fp32, L.ptrs(ymax), L.ptrs(coef),
@@ -456,7 +512,7 @@ class SNetFunction(torch.autograd.Function):
                 for t, d in zip(xg, dx):
                     dxs[t] = d if ctx.x_dtypes[t] == torch.float32 else d.to(ctx.x_dtypes[t])
             if l == 0 and not need_w:
-                saved[l] = None
+                saved[l - l0] = None
                 continue
             dw = [grad_out(PG(t, 0)) for t in range(ng)] if need_w else None
             fused_ws = 0
@@ -475,7 +531,7 @@ class SNetFunction(torch.autograd.Function):
                     L.call("tmf_conv1_bwd_fused", ng, L.ptrs(dout), L.ptrs(y), L.ptrs(coef), L.ptrs(bcoef), L.ptrs(act),
                            L.ptrs(dw), B, Dl, Hl, Wl, cout, slope, L.ptr(ws), fused_ws)
                 SNetFunction._layer_grads(ctx, pgrads, l, dw, dbias, dgamma, dbeta)
-                saved[l] = None
+                saved[l - l0] = None
                 continue
             dy = [torch.empty((B, Dl, Hl, Wl, cout), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
             L.call("tmf_bn_act_pool_bwd_apply", ng, L.ptrs(dout), dout_fp32, L.ptrs(y), L.ptrs(coef), L.ptrs(bcoef),
@@ -490,13 +546,20 @@ class SNetFunction(torch.autograd.Function):
                     ws = wgrad_workspace(ng, ctx.impl, B, Dl, Hl, Wl, cin, cout, ks, dev)
                     L.call("tmf_conv3d_wgrad", ng, L.ptrs(dy), L.ptrs(act), L.ptrs(dw), B, Dl, Hl, Wl, cin, cout, ks,
                            ctx.impl, L.ptr(ws), 0 if ws is None else ws.numel(), tag=f"tmf_conv3d_wgrad@L{l}")
-                da = [torch.empty((B, Dl, Hl, Wl, cin), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
-                L.call("tmf_conv3d_fwd", ng, L.ptrs(dy), L.ptrs(wd), L.ptrs(None), L.ptrs(da), L.ptrs(None),
-                       B, Dl, Hl, Wl, cout, cin, ks, ctx.impl, tag=f"tmf_conv3d_dgrad@L{l}")
-                dout, dout_fp32 = da, 0
+                if l > l0 or xg:                            # a segment's first layer: only for an input that wants it
+                    da = [torch.empty((B, Dl, Hl, Wl, cin), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
+                    L.call("tmf_conv3d_fwd", ng, L.ptrs(dy), L.ptrs(wd), L.ptrs(None), L.ptrs(da), L.ptrs(None),
+                           B, Dl, Hl, Wl, cout, cin, ks, ctx.impl, tag=f"tmf_conv3d_dgrad@L{l}")
+                    dout, dout_fp32 = da, 0
+                if l == l0 and xg:
+                    # gradient with respect to the exposed fp32 block output: the bf16 dgrad output, widened
+                    da32 = [torch.empty(d.shape, dtype=torch.float32, device=dev) for d in da]
+                    L.call("tmf_widen_bf16", ng, L.ptrs(da), L.ptrs(da32), da[0].numel())
+                    for t in xg:
+                        dxs[t] = da32[t].permute(0, 4, 1, 2, 3)
             if need_w:
                 SNetFunction._layer_grads(ctx, pgrads, l, dw, dbias, dgamma, dbeta)
-            saved[l] = None
+            saved[l - l0] = None
         ctx.saved = None
         ctx.params = None
         return (None, None, None, None) + tuple(dxs) + tuple(pgrads)
@@ -721,6 +784,10 @@ class EncoderFunction(torch.autograd.Function):
         L.call("tmf_encoder_proj_bwd", L.ptr(dq), L.ptr(dkv), L.ptr(dxp), L.ptr(x3), L.ptr(ln1_w), L.ptr(mean1), L.ptr(rstd1),
                L.ptr(wq), L.ptr(wkv), L.ptr(dx), L.ptr(dctx), L.ptr(d_ln1_w), L.ptr(d_ln1_b), Mx, Mc, L.ptr(ctx.pack),
                L.ptr(ws), nws)
+        if not any(ctx.needs_input_grad[9:]):
+            # frozen weights (saliency, Grad-CAM): no weight-gradient launch; the LayerNorm parameter gradients above come
+            # out of the input-gradient kernels anyway
+            return (dx.reshape(x3.shape), dctx.reshape(c3.shape)) + (None,) * 21
         table = (ctypes_ptr_array([dq, h1, d_wq, dkv, c3, d_wkv, da, o, d_wo, d_bo, dp, h2, d_w1, d_b1, dg]))
         if os.environ.get("TMF_ENC_SIDE", "1") != "0":
             # all five weight gradients feed nothing downstream in this backward pass: off the critical path
@@ -820,3 +887,31 @@ class GradientReversalFunction(torch.autograd.Function):
 
 def revgrad(x, alpha):
     return GradientReversalFunction.apply(x, alpha)
+
+
+# ==============================================================================================================
+# Grad-CAM   (csrc/gradcam.cu)
+# ==============================================================================================================
+def gradcam(acts, grads, size=None, normalize=True):
+    """Grad-CAM maps of one or more towers' block activations ``acts`` and their gradients ``grads`` (fp32, logical
+    (B,C,d,h,w)): ReLU(sum_c mean_p(G)[c] * A[c]), trilinearly upsampled to ``size`` = (D,H,W) when given
+    (``F.interpolate(mode="trilinear", align_corners=False)``), normalised per sample to [0,1] when ``normalize``.
+    Returns one fp32 (B,1,D,H,W) (or (B,1,d,h,w)) map per tower; both towers of a pair run in one launch sequence."""
+    A = [_f32c(a.detach().permute(0, 2, 3, 4, 1)) for a in acts]
+    G = [_f32c(g.detach().permute(0, 2, 3, 4, 1)) for g in grads]
+    B, d, h, w, C = A[0].shape
+    if any(t.shape != A[0].shape for t in A + G):
+        raise ValueError("gradcam: every activation and gradient must have the same shape")
+    D, H, W = tuple(size) if size is not None else (d, h, w)
+    ups = int(size is not None)
+    dev = A[0].device
+    cams = [torch.empty((B, 1, D, H, W), dtype=torch.float32, device=dev) for _ in A]
+    for i in range(0, len(A), 2):
+        ng = min(2, len(A) - i)
+        nws = int(L.load().tmf_gradcam_workspace_bytes(ng, B, d, h, w, C, D, H, W, ups, int(normalize)))
+        if nws < 0:
+            raise ValueError(f"gradcam: unsupported problem B={B} {d}x{h}x{w} C={C} -> {D}x{H}x{W}")
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        L.call("tmf_gradcam", ng, L.ptrs(A[i:i + ng]), L.ptrs(G[i:i + ng]), L.ptrs(cams[i:i + ng]), B, d, h, w, C, D, H, W,
+               ups, int(normalize), L.ptr(ws), nws)
+    return cams

@@ -7,6 +7,11 @@ children are *parameter containers only* -- their forward is never called.  All 
 """
 from __future__ import annotations
 
+import contextlib
+import copy
+import warnings
+import weakref
+
 import torch
 from torch import nn
 
@@ -41,6 +46,8 @@ class sNet(nn.Module):
         self._spec = TF.SNetSpec(dim)
         self._packs = [TF.ConvPack() for _ in range(7)]      # cached bf16 operand packs of the conv weights
         self._folds = [TF.EvalFold() for _ in range(7)]      # eval mode: BatchNorm folded into the conv operands
+        self._cam_tap = None                                  # transmf_ad_b200.interpret.grad_cam: block index to expose
+        self._cam_act = None
 
     def _units(self):
         """[(conv, bn)] in execution order."""
@@ -98,17 +105,146 @@ class sNet(nn.Module):
 
     def forward(self, mri):
         params, bufs = self._params_and_buffers()
+        taps = _tapped_boundaries([self])
+        if taps:
+            return _segmented_forward([self], [mri], params, [bufs], taps)[0]
         return TF.SNetFunction.apply(self._spec, self._run(), [bufs], 1, mri, *params)
 
 
 def snet_pair_forward(net_a: sNet, net_b: sNet, xa, xb):
-    """Run two towers of identical shape as one grouped launch sequence (grid.z = tower)."""
+    """Run two towers of identical shape as one grouped launch sequence (grid.z = tower).  Forward pre-hooks and forward
+    hooks of the towers fire as ``nn.Module.__call__`` would fire them; towers with backward hooks go through it."""
     if (net_a._spec.dim != net_b._spec.dim or net_a.training != net_b.training or tuple(xa.shape) != tuple(xb.shape)
-            or net_a._hyper() != net_b._hyper()):
+            or net_a._hyper() != net_b._hyper() or _has_backward_hooks(net_a) or _has_backward_hooks(net_b)):
         return net_a(xa), net_b(xb)
+    xa, xb = _fire_pre_hooks(net_a, xa), _fire_pre_hooks(net_b, xb)
     pa, ba = net_a._params_and_buffers()
     pb, bb = net_b._params_and_buffers()
-    return TF.SNetFunction.apply(net_a._spec, net_a._run(net_b), [ba, bb], 2, xa, xb, *pa, *pb)
+    taps = _tapped_boundaries([net_a, net_b])
+    if taps:
+        fa, fb = _segmented_forward([net_a, net_b], [xa, xb], pa + pb, [ba, bb], taps)
+    else:
+        fa, fb = TF.SNetFunction.apply(net_a._spec, net_a._run(net_b), [ba, bb], 2, xa, xb, *pa, *pb)
+    return _fire_hooks(net_a, xa, fa), _fire_hooks(net_b, xb, fb)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# block outputs for module hooks and Grad-CAM   (DESIGN section 3.7)
+# ---------------------------------------------------------------------------------------------------------------
+BLOCKS = ("conv1", "conv2", "conv3", "conv4")
+BLOCK_END = (0, 2, 4, 6)              # last sNet layer of each block; boundary k = output of block k (3: the tower output)
+_WARNED = weakref.WeakSet()
+
+
+def _has_backward_hooks(m):
+    return bool(m._backward_hooks or m._backward_pre_hooks)
+
+
+def _fire_pre_hooks(m, x, block=False):
+    """``nn.Module.__call__``'s forward pre-hooks on the single positional argument x; a block's hooks may only observe."""
+    for hid, hook in list(m._forward_pre_hooks.items()):
+        if hid in m._forward_pre_hooks_with_kwargs:
+            res = hook(m, (x,), {})
+            res = None if res is None else res[0]
+        else:
+            res = hook(m, (x,))
+        if res is not None:
+            if block:
+                raise NotImplementedError(f"a forward pre-hook on sNet.{_block_name(m)} returned a replacement input: the block "
+                                          f"runs inside fused kernels, so its hooks may only observe")
+            x = res[0] if isinstance(res, tuple) else res
+    return x
+
+
+def _fire_hooks(m, x, out, block=False):
+    """``nn.Module.__call__``'s forward hooks with (module, (x,), out); a block's hooks may only observe."""
+    for hid, hook in list(m._forward_hooks.items()):
+        res = hook(m, (x,), {}, out) if hid in m._forward_hooks_with_kwargs else hook(m, (x,), out)
+        if res is not None:
+            if block:
+                raise NotImplementedError(f"a forward hook on sNet.{_block_name(m)} returned a replacement output: the block "
+                                          f"runs inside fused kernels, so its hooks may only observe")
+            out = res
+    return out
+
+
+def _block_name(m):
+    return getattr(m, "_tmf_block_name", "conv?")
+
+
+def _tapped_boundaries(nets):
+    """Block outputs the hooks on the towers' blocks (and a pending Grad-CAM) need as real tensors: a hook on block k taps
+    its input (boundary k-1) and its output (boundary k).  Refuses what cannot be honoured and warns, once per module, about
+    hooks on modules inside a block (their tensors are fused away and never exist)."""
+    taps = set()
+    for net in nets:
+        if net._cam_tap is not None:
+            taps.add(net._cam_tap)
+        for k, name in enumerate(BLOCKS):
+            blk = getattr(net, name)
+            if _has_backward_hooks(blk):
+                raise NotImplementedError(f"backward hooks on sNet.{name} are not supported (the block runs inside fused "
+                                          f"kernels): register a tensor hook on its output from a forward hook "
+                                          f"(output.register_hook) or use torch.autograd.grad with respect to that output")
+            if blk._forward_hooks or blk._forward_pre_hooks:
+                blk._tmf_block_name = name
+                taps.update((k - 1, k) if k > 0 else (k,))
+            for child in blk._modules.values():
+                if (child._forward_hooks or child._forward_pre_hooks or _has_backward_hooks(child)) and child not in _WARNED:
+                    _WARNED.add(child)
+                    warnings.warn(f"a hook on {type(child).__name__} inside sNet.{name} never fires: the block's layers run "
+                                  f"as fused kernels and their intermediate tensors do not exist. Hook the blocks "
+                                  f"({', '.join(BLOCKS)}) or the sNet itself", UserWarning, stacklevel=4)
+    return taps
+
+
+def segment_plan(taps):
+    """Layer ranges [(l0, l1)] of a segmented run: split after each tapped block (the tower output is always exposed)."""
+    cuts = sorted(BLOCK_END[k] + 1 for k in taps if k < len(BLOCKS) - 1) + [BLOCK_END[-1] + 1]
+    return list(zip([0] + cuts[:-1], cuts))
+
+
+def _segmented_forward(nets, xs, params, bufs, taps):
+    """The towers as a chain of ``SNetFunction`` nodes split after every tapped block: each block output is an fp32 tensor
+    on the autograd path (its bf16 twin feeds the next segment), and the blocks' hooks fire on it."""
+    spec, ng = nets[0]._spec, len(nets)
+    run = nets[0]._run(nets[1] if ng == 2 else None)
+    cam = nets[0]._cam_tap
+    if cam is not None:
+        # Grad-CAM: everything up to the exposed block runs without autograd (no backward launches upstream of it)
+        run_nograd = copy.copy(run)
+        run_nograd.grad_enabled = False
+    cuts = [l1 for _, l1 in segment_plan(taps)]
+    bound = {-1: list(xs)}
+    for t, net in enumerate(nets):
+        if net.conv1._forward_pre_hooks:
+            _fire_pre_hooks(net.conv1, xs[t], block=True)
+    cur, src, l0 = list(xs), None, 0
+    for l1 in cuts:
+        upstream = cam is not None and l1 <= BLOCK_END[cam] + 1
+        with torch.no_grad() if upstream else contextlib.nullcontext():
+            res = TF.SNetFunction.apply(TF.SNetSegment(spec, l0, l1, src), run_nograd if upstream else run, bufs, ng,
+                                        *cur, *params)
+        res = res if isinstance(res, tuple) else (res,)
+        k = BLOCK_END.index(l1 - 1)
+        outs, src = list(res[:ng]), list(res[ng:]) or None
+        if cam == k:
+            outs = [o.detach().requires_grad_(True) for o in outs]
+            for net, o in zip(nets, outs):
+                net._cam_act = o
+        bound[k] = outs
+        versions = [o._version for o in outs]
+        for t, net in enumerate(nets):
+            blk = getattr(net, BLOCKS[k])
+            if blk._forward_hooks:
+                _fire_hooks(blk, bound[k - 1][t], outs[t], block=True)
+            if k + 1 < len(BLOCKS) and getattr(net, BLOCKS[k + 1])._forward_pre_hooks:
+                _fire_pre_hooks(getattr(net, BLOCKS[k + 1]), outs[t], block=True)
+        if src is not None and [o._version for o in outs] != versions:
+            raise RuntimeError(f"a hook modified the output of sNet.{BLOCKS[k]} in place; the next block would read the "
+                               f"value from before the change. Hooks on sNet blocks may only observe (clone to modify)")
+        cur, l0 = outs, l1
+    return cur
 
 
 def tokens_of(feat):
