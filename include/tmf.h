@@ -311,6 +311,26 @@ int64_t tmf_gradcam_workspace_bytes(int ng, int B, int d, int h, int w, int C, i
                                     int normalize);
 int tmf_gradcam(int ng, const float* const* A, const float* const* G, float* const* cam, int B, int d, int h, int w, int C,
                 int D, int H, int W, int upsample, int normalize, void* ws, size_t ws_bytes, void* stream);
+/* Grad-CAM's resampling pass on caller maps: lo fp32 [ng][B][d][h][w] (contiguous) -> out[g] fp32 [B][D][H][W], trilinear
+ * (align_corners=False; D,H,W = d,h,w copies the map exactly) and, with normalize != 0, (x - min) / (max - min + 1e-7) per
+ * sample.  `ws`: at least tmf_map_resample_workspace_bytes(...) bytes (0 without normalize; -1: unsupported problem). */
+int64_t tmf_map_resample_workspace_bytes(int ng, int B, int d, int h, int w, int D, int H, int W, int normalize);
+int tmf_map_resample(int ng, const float* lo, float* const* out, int B, int d, int h, int w, int D, int H, int W, int normalize,
+                     void* ws, size_t ws_bytes, void* stream);
+
+/* ---- attention maps of the fusion transformer (DESIGN section 3.8) ------------------------------------------------------
+ * tmf_attn_scores: per-head product of the attention core's operands (q / kv as for tmf_attn_fwd; dh in {16, 32, 64}, any
+ * Nq, Nk), written out as fp32 [B, heads, Nq, Nk]:
+ *   mode 0: a = q,  s = dots = scale * q_h k_h^T,  p = attn = exp(dots - lse)   (lse from tmf_attn_fwd, any implementation)
+ *   mode 1: a = dout (dL/d out, [B,Nq,h*dh]),  s = dattn = dout_h v_h^T  (dL/d attn of out = attn v; lse and p unused)
+ * Three-MMA bf16 hi/lo split with fp32 accumulation, as the tensor-core forward: dots carries the forward's scores bit for
+ * bit.  a / kv 16-byte aligned, s / p 8-byte aligned; every element written once (bitwise reproducible).
+ * tmf_attn_relevance: M[b,i,j] = mean_h w with w = attn (dattn == NULL) or max(attn * dattn, 0) (Chefer et al. 2021),
+ * r[b,j] = mean_i M[b,i,j] (accumulate != 0: added to r).  M [B,Nq,Nk] (may be NULL), r [B,Nk]; fixed summation order. */
+int tmf_attn_scores(int mode, const float* a, const float* kv, const float* lse, float* s, float* p, int B, int Nq, int Nk,
+                    int heads, int dh, float scale, void* stream);
+int tmf_attn_relevance(const float* attn, const float* dattn, float* M, float* r, int B, int heads, int Nq, int Nk,
+                       int accumulate, void* stream);
 
 /* ---- inference (SURVEY.md section 8f row 2; reference kfold_train_adversarial.py:144-187) ------------------------------------
  * Eval-mode BatchNorm3d folded into the conv operands: scale = gamma*rsqrt(running_var + eps); wf (bf16

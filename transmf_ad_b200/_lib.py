@@ -39,6 +39,9 @@ SIGNATURES = {
     "tmf_widen_bf16": [_i, _pp, _pp, _i64, _vp],
     "tmf_narrow_f32": [_i, _pp, _pp, _i64, _vp],
     "tmf_gradcam": [_i, _pp, _pp, _pp] + [_i] * 10 + [_vp, C.c_size_t, _vp],
+    "tmf_map_resample": [_i, _vp, _pp] + [_i] * 8 + [_vp, C.c_size_t, _vp],
+    "tmf_attn_scores": [_i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp],
+    "tmf_attn_relevance": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "tmf_bn_maxpool_bwd_reduce_kept": [_i, _pp, _i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp],
     "tmf_bn_bwd_finalize": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i64, _i, _vp],
     "tmf_bn_act_pool_bwd_apply": [_i, _pp, _i, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _f, _vp],
@@ -83,7 +86,7 @@ PLAIN = {"tmf_last_error": (C.c_char_p, []), "tmf_version": (_i, []), "tmf_check
          "tmf_conv3d_umma_plan_info": (_i, [_i] * 8 + [C.POINTER(C.c_int)]),
          "tmf_conv3d_col_plan_info": (_i, [_i] * 7 + [C.POINTER(C.c_int)]),
          "tmf_conv1_bwd_fused_workspace_bytes": (_i64, [_i] * 6), "tmf_conv1_dgrad_fused_workspace_bytes": (_i64, [_i] * 7),
-         "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_gradcam_workspace_bytes": (_i64, [_i] * 11), "tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
+         "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_gradcam_workspace_bytes": (_i64, [_i] * 11), "tmf_map_resample_workspace_bytes": (_i64, [_i] * 9),"tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
 
 _lib = None
 _device_checked = False

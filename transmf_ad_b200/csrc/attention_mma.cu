@@ -64,12 +64,12 @@ struct Lay {
   static constexpr int NT = DH / 8;                     // n8 tiles over the head dimension
 };
 
-// Stage `nvalid` token rows (DH floats at src + r * row_stride) as bf16 hi / lo planes; rows [nvalid, 160) are zero.  Loads are
+// Stage `nvalid` token rows (DH floats at src + r * row_stride) as bf16 hi / lo planes; rows [nvalid, NR) are zero.  Loads are
 // issued ten at a time per thread before any is used (dh = 32: the whole plane in ONE round trip).
-template <int DH>
+template <int DH, int NR = AM_NMAX>
 __device__ __forceinline__ void stage_split(uint8_t* hi, uint8_t* lo, const float* __restrict__ src, int64_t row_stride,
                                             int nvalid) {
-  constexpr int C4 = DH / 4, TOTAL = AM_NMAX * C4, U = 10;     // 160 * DH / 4 float4 = U * 128 threads * (DH / 32)
+  constexpr int C4 = DH / 4, TOTAL = NR * C4, U = 10;          // 160 * DH / 4 float4 = U * 128 threads * (DH / 32)
   for (int i0 = threadIdx.x; i0 < TOTAL; i0 += U * AM_THREADS) {
     float4 v[U];
 #pragma unroll
@@ -427,6 +427,132 @@ __global__ void __launch_bounds__(AM_THREADS) attn_mma_bwd_kernel(AttnArgs p) {
   }
 }
 
+// =====================================================================================================================
+// attention maps (DESIGN section 3.8): the per-head product A_h B_h^T that the kernels above keep in registers, written out.
+//   mode 0 ("probs"): A = q, B = k  ->  s = dots = scale * q_h k_h^T,  p = attn = exp(dots - lse)
+//   mode 1 ("grad"):  A = dO, B = v ->  s = dattn = dO_h v_h^T          (the exact dL/dattn of out = attn v)
+// Both [B, heads, Nq, Nk] fp32.  A CTA = one (batch, head), 64 query rows, one 64-key tile (blockIdx.z): the key range is
+// tiled, so Nk has no envelope (and Nk = 150 gives three times the CTAs of the forward).  The product is the forward's (same fragments, same k16 order, fp32 accumulation), so
+// dots carries the bits of the forward's scaled scores and attn those of the P the backward recomputes.  Every element is
+// written once by one thread: no atomics.
+// =====================================================================================================================
+constexpr int SC_KEYS = 64;                                     // keys per CTA
+struct ScoreArgs {
+  const float* a; const float* kv; const float* lse;
+  float* s; float* p;
+  int Nq, Nk, heads, mode;
+  float scale;
+};
+
+template <int DH>
+__global__ void __launch_bounds__(AM_THREADS) attn_scores_kernel(ScoreArgs p) {
+  pdl_entry();
+  extern __shared__ __align__(16) uint8_t smraw[];
+  using L = Lay<DH>;
+  const int inner = p.heads * DH;
+  const int b = blockIdx.x / p.heads, h = blockIdx.x % p.heads;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+  const int k0 = blockIdx.z * SC_KEYS, nk = min(SC_KEYS, p.Nk - k0);
+  const float* bsrc = p.kv + ((int64_t)b * p.Nk + k0) * 2 * inner + (p.mode == 0 ? 0 : inner) + h * DH;
+  stage_split<DH, SC_KEYS>(smraw, smraw + L::PLANE, bsrc, 2 * inner, nk);
+  __syncthreads();
+  const int r0 = blockIdx.y * AM_ROWS + warp * 16;
+  if (r0 >= p.Nq) return;
+  uint32_t ah[L::KS][4], al[L::KS][4];
+  load_a_frags<DH>(p.a + ((int64_t)b * p.Nq + r0) * inner + h * DH, inner, p.Nq - r0, ah, al);
+  float lr[2] = {0.f, 0.f};
+  if (p.mode == 0) {
+#pragma unroll
+    for (int hf = 0; hf < 2; ++hf) {
+      const int i = r0 + g + 8 * hf;
+      lr[hf] = (i < p.Nq) ? __ldg(p.lse + (int64_t)blockIdx.x * p.Nq + i) : 0.f;
+    }
+  }
+  const uint32_t kb = (uint32_t)__cvta_generic_to_shared(smraw) + off_nk<DH>(lane);
+  const int64_t base = (int64_t)blockIdx.x * p.Nq * p.Nk;       // (b * heads + h) * Nq * Nk
+  const bool pairs = (p.Nk & 1) == 0;                            // rows start 8-byte aligned: float2 stores
+  const int nchunk = (nk + 15) >> 4;
+  for (int jp = 0; jp < nchunk; ++jp) {
+    float c[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
+    mma_tile_nk<DH>(c, ah, al, kb, 16 * jp);
+#pragma unroll
+    for (int j = 0; j < 2; ++j)
+#pragma unroll
+      for (int hf = 0; hf < 2; ++hf) {
+        const int i = r0 + g + 8 * hf, col = k0 + 16 * jp + 8 * j + 2 * t;
+        if (i >= p.Nq || col >= p.Nk) continue;
+        float v0 = c[j][2 * hf], v1 = c[j][2 * hf + 1];
+        const int64_t o = base + (int64_t)i * p.Nk + col;
+        const bool two = col + 1 < p.Nk;
+        if (p.mode == 0) {
+          v0 *= p.scale;
+          v1 *= p.scale;
+          const float e0 = __expf(v0 - lr[hf]), e1 = __expf(v1 - lr[hf]);
+          if (pairs && two) {
+            *reinterpret_cast<float2*>(p.p + o) = make_float2(e0, e1);
+          } else {
+            p.p[o] = e0;
+            if (two) p.p[o + 1] = e1;
+          }
+        }
+        if (pairs && two) {
+          *reinterpret_cast<float2*>(p.s + o) = make_float2(v0, v1);
+        } else {
+          p.s[o] = v0;
+          if (two) p.s[o + 1] = v1;
+        }
+      }
+  }
+}
+
+template <int DH>
+static int launch_scores(const ScoreArgs& p, int B, cudaStream_t st) {
+  const size_t smem = 2 * (size_t)Lay<DH>::PLANE;                // one hi / lo plane pair (rows >= SC_KEYS unused)
+  dim3 grid(B * p.heads, ceil_div(p.Nq, AM_ROWS), ceil_div(p.Nk, SC_KEYS));
+  launch_k(attn_scores_kernel<DH>, grid, AM_THREADS, smem, st, p);
+  TMF_LAUNCH_CHECK();
+  return 0;
+}
+
+// M[b,i,j] = (1/heads) sum_h w,  w = attn (dattn == NULL) or max(attn * dattn, 0);  r[b,j] (+)= (1/Nq) sum_i M[b,i,j].
+// A block = 32 key columns of one sample (coalesced rows) x 8 row slices; heads, rows of a slice and the slices are added
+// in index order.
+constexpr int RV_COLS = 32, RV_SLICES = 8;
+__global__ void __launch_bounds__(RV_COLS * RV_SLICES) attn_relevance_kernel(const float* __restrict__ attn,
+                                                                           const float* __restrict__ dattn, float* M, float* r,
+                                                                           int heads, int Nq, int Nk, int accumulate) {
+  pdl_entry();
+  __shared__ float part[RV_SLICES][RV_COLS];
+  const int b = blockIdx.y, cx = threadIdx.x % RV_COLS, sl = threadIdx.x / RV_COLS;
+  const int j = blockIdx.x * RV_COLS + cx;
+  float acc = 0.f;
+  if (j < Nk) {
+    const int64_t hstride = (int64_t)Nq * Nk;
+    for (int i = sl; i < Nq; i += RV_SLICES) {
+      const int64_t o = ((int64_t)b * heads * Nq + i) * Nk + j;
+      float m = 0.f;
+      for (int hh = 0; hh < heads; ++hh) {
+        float w = __ldg(attn + o + hh * hstride);
+        if (dattn != nullptr) w = fmaxf(w * __ldg(dattn + o + hh * hstride), 0.f);
+        m += w;
+      }
+      m /= (float)heads;
+      if (M != nullptr) M[((int64_t)b * Nq + i) * Nk + j] = m;
+      acc += m;
+    }
+  }
+  part[sl][cx] = acc;
+  __syncthreads();
+  if (sl == 0 && j < Nk) {
+    float s = 0.f;
+#pragma unroll
+    for (int k = 0; k < RV_SLICES; ++k) s += part[k][cx];
+    s /= (float)Nq;
+    float* dst = r + (int64_t)b * Nk + j;
+    *dst = accumulate ? *dst + s : s;
+  }
+}
+
 static int impl_choice() {
   static int v = -1;
   if (v < 0) {
@@ -487,3 +613,37 @@ int attn_mma_bwd(const AttnArgs& p, cudaStream_t st) {
 }  // namespace tmf
 
 extern "C" int tmf_attn_impl_default(void) { return tmf::amma::impl_choice(); }
+
+extern "C" int tmf_attn_scores(int mode, const float* a, const float* kv, const float* lse, float* s, float* p, int B, int Nq,
+                               int Nk, int heads, int dh, float scale, void* stream) {
+  using namespace tmf;
+  TMF_REQUIRE(mode == 0 || mode == 1, "tmf_attn_scores: mode must be 0 (probs) or 1 (grad); got %d", mode);
+  TMF_REQUIRE(dh == 16 || dh == 32 || dh == 64, "tmf_attn_scores: dim_head must be 16, 32 or 64 (got %d)", dh);
+  TMF_REQUIRE(B >= 1 && Nq >= 1 && Nk >= 1 && heads >= 1, "tmf_attn_scores: bad shape B=%d Nq=%d Nk=%d heads=%d", B, Nq, Nk,
+              heads);
+  TMF_REQUIRE((int64_t)B * heads * Nq * Nk < (1ll << 40), "tmf_attn_scores: problem too large");
+  TMF_REQUIRE(a != nullptr && kv != nullptr && s != nullptr && (mode == 1 || (lse != nullptr && p != nullptr)),
+              "tmf_attn_scores: missing operand (mode %d needs a, kv, s%s)", mode, mode == 0 ? ", lse, p" : "");
+  TMF_REQUIRE(((uintptr_t)a & 15) == 0 && ((uintptr_t)kv & 15) == 0 && ((uintptr_t)s & 7) == 0 && ((uintptr_t)p & 7) == 0,
+              "tmf_attn_scores: a / kv must be 16-byte and s / p 8-byte aligned");
+  amma::ScoreArgs sa{};
+  sa.a = a; sa.kv = kv; sa.lse = lse; sa.s = s; sa.p = p;
+  sa.Nq = Nq; sa.Nk = Nk; sa.heads = heads; sa.mode = mode; sa.scale = scale;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dh == 32) return amma::launch_scores<32>(sa, B, st);
+  if (dh == 16) return amma::launch_scores<16>(sa, B, st);
+  return amma::launch_scores<64>(sa, B, st);
+}
+
+extern "C" int tmf_attn_relevance(const float* attn, const float* dattn, float* M, float* r, int B, int heads, int Nq, int Nk,
+                                  int accumulate, void* stream) {
+  using namespace tmf;
+  TMF_REQUIRE(B >= 1 && heads >= 1 && Nq >= 1 && Nk >= 1, "tmf_attn_relevance: bad shape B=%d heads=%d Nq=%d Nk=%d", B, heads,
+              Nq, Nk);
+  TMF_REQUIRE(attn != nullptr && r != nullptr, "tmf_attn_relevance: attn and r are required");
+  dim3 grid(ceil_div(Nk, amma::RV_COLS), B);
+  launch_k(amma::attn_relevance_kernel, grid, amma::RV_COLS * amma::RV_SLICES, 0, (cudaStream_t)stream, attn, dattn, M, r,
+           heads, Nq, Nk, accumulate);
+  TMF_LAUNCH_CHECK();
+  return 0;
+}

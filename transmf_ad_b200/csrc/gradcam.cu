@@ -361,4 +361,43 @@ int tmf_gradcam(int ng, const float* const* A, const float* const* G, float* con
   return 0;
 }
 
+// Any low-resolution maps (the fusion transformer's token relevance, DESIGN section 3.8) through Grad-CAM's resampling pass:
+// the same plan and the same cam_resample_kernel launches, so a map comes out with the bits tmf_gradcam gives it.
+static size_t map_resample_bytes(int ng, int B, int d, int h, int w, int D, int H, int W, int normalize) {
+  const CamPlan pl = cam_plan(ng, B, d, h, w, 4, D, H, W, 1, normalize);
+  return normalize ? (size_t)ng * B * pl.nres * 2 * sizeof(float) : 0;
+}
+
+int64_t tmf_map_resample_workspace_bytes(int ng, int B, int d, int h, int w, int D, int H, int W, int normalize) {
+  if (ng < 1 || ng > TMF_MAX_GROUPS || B < 1 || d < 1 || h < 1 || w < 1 || D < 1 || H < 1 || W < 1) return -1;
+  return (int64_t)map_resample_bytes(ng, B, d, h, w, D, H, W, normalize);
+}
+
+int tmf_map_resample(int ng, const float* lo, float* const* out, int B, int d, int h, int w, int D, int H, int W, int normalize,
+                     void* ws, size_t ws_bytes, void* stream) {
+  TMF_CHECK_NG(ng);
+  TMF_REQUIRE(lo != nullptr, "tmf_map_resample: lo is NULL");
+  TMF_REQUIRE(B >= 1 && d >= 1 && h >= 1 && w >= 1 && D >= 1 && H >= 1 && W >= 1,
+              "tmf_map_resample: bad extent B=%d %dx%dx%d -> %dx%dx%d", B, d, h, w, D, H, W);
+  TMF_REQUIRE((int64_t)d * h * w < (1ll << 31) && (int64_t)D * H * W < (1ll << 31), "tmf_map_resample: extent too large");
+  const size_t need = map_resample_bytes(ng, B, d, h, w, D, H, W, normalize);
+  TMF_REQUIRE(!normalize || (ws != nullptr && ws_bytes >= need),
+              "tmf_map_resample: workspace of %zu bytes < %zu (tmf_map_resample_workspace_bytes)", ws_bytes, need);
+  const CamPlan pl = cam_plan(ng, B, d, h, w, 4, D, H, W, 1, normalize);
+  CamArgs a{};
+  if (!load_group(a.out, out, ng, true, "out")) return 1;
+  a.lo = const_cast<float*>(lo);
+  a.mm = normalize ? (float*)ws : nullptr;
+  a.B = B; a.d = d; a.h = h; a.w = w; a.D = D; a.H = H; a.W = W;
+  a.P = pl.P; a.nparts = pl.nres; a.nout = pl.nout;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (normalize) {
+    launch_k(cam_resample_kernel<true, false>, dim3(pl.nres, B, ng), CAM_THREADS, 0, st, a, 1);
+    TMF_LAUNCH_CHECK();
+  }
+  launch_k(cam_resample_kernel<true, true>, dim3(pl.nres, B, ng), CAM_THREADS, 0, st, a, normalize);
+  TMF_LAUNCH_CHECK();
+  return 0;
+}
+
 }  // extern "C"

@@ -659,10 +659,11 @@ def layer_norm(x, gamma, beta, residual=None, eps=LN_EPS):
 
 
 class AttentionCoreFunction(torch.autograd.Function):
-    """softmax(q k^T * scale) v per head on short token sequences; q (B,Nq,h*dh), kv (B,Nk,2*h*dh)."""
+    """softmax(q k^T * scale) v per head on short token sequences; q (B,Nq,h*dh), kv (B,Nk,2*h*dh).  With an ``AttnTap``
+    it also returns the reference's ``dots`` and ``attn`` (DESIGN section 3.8)."""
 
     @staticmethod
-    def forward(ctx, q, kv, heads, scale):
+    def forward(ctx, q, kv, heads, scale, tap=None):
         q, kv = _f32c(q), _f32c(kv)
         B, Nq, inner = q.shape
         Nk = kv.shape[1]
@@ -672,21 +673,148 @@ class AttentionCoreFunction(torch.autograd.Function):
         L.call("tmf_attn_fwd", L.ptr(q), L.ptr(kv), L.ptr(out), L.ptr(lse), B, Nq, Nk, heads, dh, float(scale))
         ctx.save_for_backward(q, kv, out, lse)
         ctx.heads, ctx.scale = heads, float(scale)
-        return out
+        ctx.tap = tap
+        if tap is None:
+            return out
+        dots, attn = attn_scores(q, kv, heads, scale, lse)
+        tap.arm(kv, heads, None)
+        ctx.mark_non_differentiable(dots)
+        ctx.set_materialize_grads(False)
+        return out, dots, attn
 
     @staticmethod
-    def backward(ctx, dout):
+    def backward(ctx, dout, ddots=None, dattn=None):
         q, kv, out, lse = ctx.saved_tensors
         B, Nq, inner = q.shape
         Nk = kv.shape[1]
+        if ctx.tap is not None:
+            ctx.tap.check(dattn)
         dq, dkv = torch.empty_like(q), torch.empty_like(kv)
+        if dout is None:
+            dout = torch.zeros_like(out)
         L.call("tmf_attn_bwd", L.ptr(_f32c(dout)), L.ptr(q), L.ptr(kv), L.ptr(out), L.ptr(lse), L.ptr(dq), L.ptr(dkv),
                B, Nq, Nk, ctx.heads, inner // ctx.heads, ctx.scale)
-        return dq, dkv, None, None
+        return dq, dkv, None, None, None
 
 
-def attention_core(q, kv, heads, scale):
-    return AttentionCoreFunction.apply(q, kv, heads, scale)
+def attention_core(q, kv, heads, scale, tap=None):
+    return AttentionCoreFunction.apply(q, kv, heads, scale, tap)
+
+
+# ==============================================================================================================
+# Attention probabilities for module hooks and attention maps   (csrc/attention_mma.cu, DESIGN section 3.8)
+# ==============================================================================================================
+def attn_scores(q, kv, heads, scale, lse):
+    """(dots, attn), fp32 (B, heads, Nq, Nk): scale * q_h k_h^T and exp(dots - lse), with the attention core's operands."""
+    B, Nq, inner = q.shape
+    Nk = kv.shape[1]
+    dots = torch.empty((B, heads, Nq, Nk), dtype=torch.float32, device=q.device)
+    attn = torch.empty_like(dots)
+    L.call("tmf_attn_scores", 0, L.ptr(q), L.ptr(kv), L.ptr(lse), L.ptr(dots), L.ptr(attn), B, Nq, Nk, heads, inner // heads,
+           float(scale))
+    return dots, attn
+
+
+def attn_scores_grad(dout, kv, heads):
+    """dL/d attn = dO_h v_h^T, fp32 (B, heads, Nq, Nk), from dL/d out (B, Nq, heads*dh)."""
+    dout = _f32c(dout)
+    B, Nq, inner = dout.shape
+    Nk = kv.shape[1]
+    dattn = torch.empty((B, heads, Nq, Nk), dtype=torch.float32, device=dout.device)
+    L.call("tmf_attn_scores", 1, L.ptr(dout), L.ptr(kv), L.ptr(None), L.ptr(dattn), L.ptr(None), B, Nq, Nk, heads,
+           inner // heads, 1.0)
+    return dattn
+
+
+def attn_relevance(attn, dattn=None, r=None, accumulate=False):
+    """Head-averaged map M = mean_h attn (or mean_h max(attn * dattn, 0)), (B, Nq, Nk), and the key relevance
+    r = mean_i M, (B, Nk), written into ``r`` when given (added to it with ``accumulate``).  Returns (M, r)."""
+    attn = _f32c(attn.detach())
+    B, heads, Nq, Nk = attn.shape
+    if dattn is not None:
+        dattn = _f32c(dattn.detach())
+        if dattn.shape != attn.shape:
+            raise ValueError("attn_relevance: attn and dattn must have the same shape")
+    M = torch.empty((B, Nq, Nk), dtype=torch.float32, device=attn.device)
+    acc = r is not None and accumulate
+    if r is None:
+        r = torch.empty((B, Nk), dtype=torch.float32, device=attn.device)
+    elif tuple(r.shape) != (B, Nk) or r.dtype != torch.float32 or not r.is_contiguous():
+        raise ValueError(f"attn_relevance: r must be a contiguous fp32 ({B}, {Nk}) tensor")
+    L.call("tmf_attn_relevance", L.ptr(attn), L.ptr(dattn), L.ptr(M), L.ptr(r), B, heads, Nq, Nk, int(acc))
+    return M, r
+
+
+def map_resample(lo, size, normalize=True):
+    """``lo``: fp32 (ng, B, d, h, w) maps -> ng fp32 (B, 1, D, H, W) maps, trilinear (align_corners=False) to ``size``
+    and normalised per sample to [0, 1] when ``normalize``: Grad-CAM's resampling pass (csrc/gradcam.cu)."""
+    lo = _f32c(lo)
+    ng, B, d, h, w = lo.shape
+    D, H, W = (int(s) for s in size)
+    outs = [torch.empty((B, 1, D, H, W), dtype=torch.float32, device=lo.device) for _ in range(ng)]
+    for i in range(0, ng, 2):
+        n = min(2, ng - i)
+        nws = int(L.load().tmf_map_resample_workspace_bytes(n, B, d, h, w, D, H, W, int(normalize)))
+        if nws < 0:
+            raise ValueError(f"map_resample: unsupported problem B={B} {d}x{h}x{w} -> {D}x{H}x{W}")
+        ws = torch.empty(max(nws, 1), dtype=torch.uint8, device=lo.device)
+        L.call("tmf_map_resample", n, L.ptr(lo[i:i + n]), L.ptrs(outs[i:i + n]), B, d, h, w, D, H, W, int(normalize),
+               L.ptr(ws), nws)
+    return outs
+
+
+class AttnTap:
+    """What ties an attention node that exposes ``attn`` to the ``AttnTapFunction`` node behind its output.  The tap node's
+    backward turns the gradient of the output into dL/d attn (``tmf_attn_scores`` mode 1) and hands it to autograd; the
+    attention node's backward then checks that the gradient it receives for ``attn`` is that very tensor, unmodified --
+    the probabilities may only be observed, never feed anything else."""
+
+    def __init__(self):
+        self.kv = self.heads = self.chain = None
+        self.dattn, self.version = None, None
+        self.stash = None
+
+    def arm(self, kv, heads, chain):
+        """``chain(dy) -> (dO, stash)``: the gradient of the attention output from that of the node's output (fused encoder:
+        its chain backward, whose results ``stash`` the encoder's backward reuses; attention core: the identity)."""
+        self.kv, self.heads, self.chain = kv, heads, chain
+
+    def grad(self, dy):
+        dout, self.stash = self.chain(dy) if self.chain is not None else (dy, None)
+        self.dattn = attn_scores_grad(dout, self.kv, self.heads)
+        self.version = self.dattn._version
+        self.kv = self.chain = None
+        return self.dattn
+
+    def check(self, dattn):
+        if dattn is not None and (dattn is not self.dattn or dattn._version != self.version):
+            # this backward pass ends here: join the weight-gradient work that encoders behind this one already put on the
+            # side stream (the engine callback that would have joined it is dropped with the pass)
+            join_side_streams()
+            raise NotImplementedError("attention probabilities may only be observed: a gradient other than the one the "
+                                      "model's own output gives reached `attn` (a tensor hook on it returned or modified a "
+                                      "gradient, or `attn` entered a loss). Clone `attn` to compute with it")
+        self.dattn = None
+
+
+class AttnTapFunction(torch.autograd.Function):
+    """Identity on an attention node's output ``y`` that also consumes its ``attn``: backward returns dy unchanged and
+    dL/d attn as ``attn``'s gradient, so that tensor hooks on ``attn`` see it."""
+
+    @staticmethod
+    def forward(ctx, y, attn, tap):
+        ctx.tap = tap
+        return y.view_as(y)
+
+    @staticmethod
+    def backward(ctx, dy):
+        return dy, ctx.tap.grad(dy), None
+
+
+def attn_tap(y, attn, tap):
+    if not (torch.is_grad_enabled() and attn.requires_grad):
+        return y
+    return AttnTapFunction.apply(y, attn, tap)
 
 
 # Side stream for work that is off the backward pass's critical path (the encoders' weight gradients): launched there, it
@@ -718,7 +846,7 @@ class EncoderFunction(torch.autograd.Function):
     params = (ln1_w, ln1_b, wq, wkv, wo, bo, ln2_w, ln2_b, w1, b1, w2, b2, lnf_w, lnf_b)."""
 
     @staticmethod
-    def forward(ctx, x, context, heads, scale, add_input, eps1, eps2, epsf, pack_cache, *params):
+    def forward(ctx, x, context, heads, scale, add_input, eps1, eps2, epsf, pack_cache, tap, *params):
         ln1_w, ln1_b, wq, wkv, wo, bo, ln2_w, ln2_b, w1, b1, w2, b2, lnf_w, lnf_b = [_f32c(t) for t in params]
         x3, c3 = _f32c(x), _f32c(context)
         B, Nq, dim = x3.shape
@@ -757,10 +885,39 @@ class EncoderFunction(torch.autograd.Function):
         ctx.pack = pack
         ctx.param_refs = params                              # references only: gradient slots of the flat DP buffer
         ctx.cfg = (heads, float(scale), bool(add_input), B, Nq, Nk, dim, mlp)
-        return y.reshape(x.shape)
+        ctx.tap = tap
+        if tap is None:
+            return y.reshape(x.shape)
+        # attention maps (DESIGN section 3.8): the probabilities behind o, one more launch
+        dots, attn = attn_scores(q, kv, heads, scale, lse)
+        chain_in = (g, a, pre, wo, w1, w2, ln2_w, lnf_w, mean2, rstd2, meanf, rstdf)
+        cfg = ctx.cfg
+        tap.arm(kv, heads, lambda dy: EncoderFunction._chain_bwd(cfg, params, pack, chain_in, dy))
+        ctx.mark_non_differentiable(dots)
+        ctx.set_materialize_grads(False)
+        return y.reshape(x.shape), dots, attn
 
     @staticmethod
-    def backward(ctx, dy):
+    def _chain_bwd(cfg, P, pack, saved, dy):
+        """tmf_encoder_chain_bwd: the gradients of the attention output (dout), of the residual input (dxp) and of the rows
+        behind them, plus the gradients of the two LayerNorms it covers."""
+        g, a, pre, wo, w1, w2, ln2_w, lnf_w, mean2, rstd2, meanf, rstdf = saved
+        heads, scale, add_input, B, Nq, Nk, dim, mlp = cfg
+        Mx = B * Nq
+        dev = g.device
+        E = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+        d_ln2_w, d_ln2_b, d_lnf_w, d_lnf_b = grad_out(P[6]), grad_out(P[7]), grad_out(P[12]), grad_out(P[13])
+        ws, nws = L.scratch(dev)
+        dy2 = _f32c(dy).reshape(Mx, dim)
+        dg, dp, da, dout, dxp = E(Mx, dim), E(Mx, mlp), E(Mx, dim), E(B, Nq, dim), E(Mx, dim)
+        L.call("tmf_encoder_chain_bwd", L.ptr(dy2), L.ptr(g), L.ptr(a), L.ptr(pre), L.ptr(wo), L.ptr(w1), L.ptr(w2), L.ptr(ln2_w),
+               L.ptr(lnf_w), L.ptr(mean2), L.ptr(rstd2), L.ptr(meanf), L.ptr(rstdf), L.ptr(dg), L.ptr(dp), L.ptr(da),
+               L.ptr(dout), L.ptr(dxp), L.ptr(d_lnf_w), L.ptr(d_lnf_b), L.ptr(d_ln2_w), L.ptr(d_ln2_b), Mx, mlp,
+               int(add_input), L.ptr(pack), L.ptr(ws), nws)
+        return dout, (dy, dg, dp, da, dout, dxp, d_ln2_w, d_ln2_b, d_lnf_w, d_lnf_b)
+
+    @staticmethod
+    def backward(ctx, dy, ddots=None, dattn=None):
         (x3, c3, h1, mean1, rstd1, q, kv, o, lse, a, h2, mean2, rstd2, pre, f, g, meanf, rstdf,
          ln1_w, wq, wkv, wo, ln2_w, w1, w2, lnf_w) = ctx.saved_tensors
         heads, scale, add_input, B, Nq, Nk, dim, mlp = ctx.cfg
@@ -769,14 +926,27 @@ class EncoderFunction(torch.autograd.Function):
         E = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
         P = ctx.param_refs
         G = lambda i: grad_out(P[i])
-        d_ln1_w, d_ln1_b, d_wq, d_wkv, d_wo, d_bo, d_ln2_w, d_ln2_b, d_w1, d_b1, d_w2, d_b2, d_lnf_w, d_lnf_b = [G(i) for i in range(14)]
-        ws, nws = L.scratch(dev)
-        dy2 = _f32c(dy).reshape(Mx, dim)
-        dg, dp, da, dout, dxp = E(Mx, dim), E(Mx, mlp), E(Mx, dim), E(B, Nq, dim), E(Mx, dim)
-        L.call("tmf_encoder_chain_bwd", L.ptr(dy2), L.ptr(g), L.ptr(a), L.ptr(pre), L.ptr(wo), L.ptr(w1), L.ptr(w2), L.ptr(ln2_w),
-               L.ptr(lnf_w), L.ptr(mean2), L.ptr(rstd2), L.ptr(meanf), L.ptr(rstdf), L.ptr(dg), L.ptr(dp), L.ptr(da),
-               L.ptr(dout), L.ptr(dxp), L.ptr(d_lnf_w), L.ptr(d_lnf_b), L.ptr(d_ln2_w), L.ptr(d_ln2_b), Mx, mlp,
-               int(add_input), L.ptr(ctx.pack), L.ptr(ws), nws)
+        stash = None
+        if ctx.tap is not None:
+            ctx.tap.check(dattn)
+            stash, ctx.tap.stash = ctx.tap.stash, None
+            if dy is None:
+                dy = torch.zeros((B, Nq, dim), dtype=torch.float32, device=dev)
+        if stash is not None and stash[0] is dy:
+            # the tap node ran the chain backward on this very gradient to get dL/d attn: its results are reused
+            _, dg, dp, da, dout, dxp, d_ln2_w, d_ln2_b, d_lnf_w, d_lnf_b = stash
+            d_ln1_w, d_ln1_b, d_wq, d_wkv, d_wo, d_bo = [G(i) for i in range(6)]
+            d_w1, d_b1, d_w2, d_b2 = [G(i) for i in range(8, 12)]
+            ws, nws = L.scratch(dev)
+        else:
+            d_ln1_w, d_ln1_b, d_wq, d_wkv, d_wo, d_bo, d_ln2_w, d_ln2_b, d_w1, d_b1, d_w2, d_b2, d_lnf_w, d_lnf_b = [G(i) for i in range(14)]
+            ws, nws = L.scratch(dev)
+            dy2 = _f32c(dy).reshape(Mx, dim)
+            dg, dp, da, dout, dxp = E(Mx, dim), E(Mx, mlp), E(Mx, dim), E(B, Nq, dim), E(Mx, dim)
+            L.call("tmf_encoder_chain_bwd", L.ptr(dy2), L.ptr(g), L.ptr(a), L.ptr(pre), L.ptr(wo), L.ptr(w1), L.ptr(w2), L.ptr(ln2_w),
+                   L.ptr(lnf_w), L.ptr(mean2), L.ptr(rstd2), L.ptr(meanf), L.ptr(rstdf), L.ptr(dg), L.ptr(dp), L.ptr(da),
+                   L.ptr(dout), L.ptr(dxp), L.ptr(d_lnf_w), L.ptr(d_lnf_b), L.ptr(d_ln2_w), L.ptr(d_ln2_b), Mx, mlp,
+                   int(add_input), L.ptr(ctx.pack), L.ptr(ws), nws)
         dq, dkv = E(B, Nq, dim), E(B, Nk, 2 * dim)
         L.call("tmf_attn_bwd", L.ptr(dout), L.ptr(q), L.ptr(kv), L.ptr(o), L.ptr(lse), L.ptr(dq), L.ptr(dkv), B, Nq, Nk, heads,
                dim // heads, scale)
@@ -784,10 +954,10 @@ class EncoderFunction(torch.autograd.Function):
         L.call("tmf_encoder_proj_bwd", L.ptr(dq), L.ptr(dkv), L.ptr(dxp), L.ptr(x3), L.ptr(ln1_w), L.ptr(mean1), L.ptr(rstd1),
                L.ptr(wq), L.ptr(wkv), L.ptr(dx), L.ptr(dctx), L.ptr(d_ln1_w), L.ptr(d_ln1_b), Mx, Mc, L.ptr(ctx.pack),
                L.ptr(ws), nws)
-        if not any(ctx.needs_input_grad[9:]):
+        if not any(ctx.needs_input_grad[10:]):
             # frozen weights (saliency, Grad-CAM): no weight-gradient launch; the LayerNorm parameter gradients above come
             # out of the input-gradient kernels anyway
-            return (dx.reshape(x3.shape), dctx.reshape(c3.shape)) + (None,) * 21
+            return (dx.reshape(x3.shape), dctx.reshape(c3.shape)) + (None,) * 22
         table = (ctypes_ptr_array([dq, h1, d_wq, dkv, c3, d_wkv, da, o, d_wo, d_bo, dp, h2, d_w1, d_b1, dg]))
         if os.environ.get("TMF_ENC_SIDE", "1") != "0":
             # all five weight gradients feed nothing downstream in this backward pass: off the critical path
@@ -806,7 +976,7 @@ class EncoderFunction(torch.autograd.Function):
             _SIDE_PENDING.append(ev)
         else:
             L.call("tmf_encoder_wgrad", table, L.ptr(f), L.ptr(d_w2), L.ptr(d_b2), Mx, Mc, mlp, L.ptr(ws), nws)
-        return (dx.reshape(x3.shape), dctx.reshape(c3.shape), None, None, None, None, None, None, None,
+        return (dx.reshape(x3.shape), dctx.reshape(c3.shape), None, None, None, None, None, None, None, None,
                 d_ln1_w, d_ln1_b, d_wq, d_wkv, d_wo, d_bo, d_ln2_w, d_ln2_b, d_w1, d_b1, d_w2, d_b2, d_lnf_w, d_lnf_b)
 
 
@@ -819,8 +989,9 @@ def encoder_supported(dim, inner, mlp):
     return os.environ.get("TMF_ENC_FUSED", "1") != "0" and bool(L.load().tmf_encoder_supported(int(dim), int(inner), int(mlp)))
 
 
-def encoder(x, context, heads, scale, add_input, eps1, eps2, epsf, params, pack_cache=None):
-    return EncoderFunction.apply(x, context, heads, scale, add_input, eps1, eps2, epsf, pack_cache, *params)
+def encoder(x, context, heads, scale, add_input, eps1, eps2, epsf, params, pack_cache=None, tap=None):
+    """The fused encoder; with an ``AttnTap`` it returns (y, dots, attn) (DESIGN section 3.8)."""
+    return EncoderFunction.apply(x, context, heads, scale, add_input, eps1, eps2, epsf, pack_cache, tap, *params)
 
 
 class TokenPoolFunction(torch.autograd.Function):

@@ -1,17 +1,21 @@
-"""Interpretability on the sNet towers: Grad-CAM (Selvaraju et al., 2017) on a block of every tower of a model.
+"""Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, and head-averaged or
+gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the fusion transformer.
 
 Input gradients (saliency maps) need nothing from here: ``mri.requires_grad_(True)`` and plain autograd work on every model
-(INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c).
+(INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c), and so do
+module hooks on ``Attention.attend`` (section 3d).
 """
 from __future__ import annotations
+
+from collections import namedtuple
 
 import torch
 
 from . import functional as TF
-from .models.networks import BLOCKS, sNet
+from .models.networks import BLOCKS, CrossTransformer, CrossTransformer_MOD_AVG, sNet
 
 
-def _target_index(target, B, device):
+def _target_index(target, B, device, who="grad_cam"):
     if isinstance(target, int) and not isinstance(target, bool):
         return torch.full((B,), target, dtype=torch.long, device=device)
     if torch.is_tensor(target) and target.dim() <= 1 and not target.is_floating_point() and target.dtype != torch.bool:
@@ -20,7 +24,7 @@ def _target_index(target, B, device):
             t = t.expand(B)
         if t.numel() == B:
             return t
-    raise ValueError(f"grad_cam: target must be a class index or an integer tensor of shape ({B},); got {target!r}")
+    raise ValueError(f"{who}: target must be a class index or an integer tensor of shape ({B},); got {target!r}")
 
 
 def grad_cam(model, inputs, target, layer="conv3", upsample=True, normalize=True):
@@ -65,3 +69,96 @@ def grad_cam(model, inputs, target, layer="conv3", upsample=True, normalize=True
             t._cam_tap, t._cam_act = None, None
     size = tuple(inputs[0].shape[2:]) if upsample else None
     return TF.gradcam(acts, grads, size=size, normalize=normalize)
+
+
+CrossAttention = namedtuple("CrossAttention", ["maps", "mri", "pet"])
+
+
+def cross_attention(model, inputs, target=None, upsample=True, normalize=True):
+    """Cross-modal attention maps of the fusion transformer of ``model`` (``CrossTransformer_MOD_AVG``: ``model_ad``,
+    ``model_transformer``; ``CrossTransformer``: ``model_transformer_res``).
+
+    Per encoder call, M[b,i,j] = mean_h attn (``target=None``: forward only) or mean_h max(attn * dL/d attn, 0) for the
+    objective ``sum_b logits[b, target_b]`` of the model's first output (gradient-weighted, Chefer et al. 2021); a key
+    token's relevance is r[b,j] = mean_i M[b,i,j].  Returns ``CrossAttention(maps, mri, pet)``:
+      ``maps``: per layer, the (mri_enc, pet_enc) pair of fp32 (B, Nq, Nk) maps M;
+      ``pet`` / ``mri``: fp32 (B,1,D,H,W) volume maps (``upsample``; else the tower output's (B,1,d,h,w)), normalised per
+      sample to [0,1] (``normalize``).  ``CrossTransformer_MOD_AVG``: the PET map sums, over layers, the key relevance of
+      ``mri_enc`` (where MRI queries looked in PET) and the MRI map that of ``pet_enc``.  ``CrossTransformer``: both
+      encoders attend to cat([mri, pet]); the MRI map sums r[:, :N], the PET map r[:, N:], over layers and encoders.
+    Key token n is the sNet output voxel (x, y, z) with n = (x*h + y)*w + z (``tokens_of``).
+
+    The model runs in its current mode.  The towers run without autograd and their outputs become leaves, so no sNet
+    backward runs; no parameter receives a ``.grad``, no weight-gradient kernel runs, and ``requires_grad`` flags are
+    restored afterwards."""
+    fusers = [m for m in model.modules() if isinstance(m, (CrossTransformer, CrossTransformer_MOD_AVG))]
+    if not fusers:
+        raise ValueError("cross_attention: the model has no fusion transformer (CrossTransformer or CrossTransformer_MOD_AVG)")
+    if len(fusers) > 1:
+        raise ValueError("cross_attention: the model has more than one fusion transformer")
+    fuser = fusers[0]
+    if isinstance(fuser, CrossTransformer) and fuser.share:
+        raise ValueError("cross_attention: CrossTransformer(share=True) is not supported")
+    towers = [m for m in model.modules() if isinstance(m, sNet)]
+    inputs = tuple(inputs) if isinstance(inputs, (tuple, list)) else (inputs,)
+    if len(inputs) != 2 or not all(torch.is_tensor(x) and x.dim() == 5 for x in inputs):
+        raise ValueError("cross_attention: inputs must be the (mri, pet) pair of (B,1,D,H,W) volumes")
+    B = inputs[0].shape[0]
+    encs = [enc for pair in fuser.layers for enc in pair]              # reference order: mri_enc, pet_enc per layer
+    probs, grid = {}, {}
+    weighted = target is not None
+
+    def keep_attn(i):
+        def hook(module, args, attn):
+            probs.setdefault(i, attn)
+        return hook
+
+    def leaf(module, args, out):
+        grid["dhw"] = tuple(out.shape[2:])
+        return out.detach().requires_grad_(True) if weighted else None
+
+    flags = [(p, p.requires_grad) for p in model.parameters()]
+    handles = []
+    try:
+        for p, _ in flags:
+            p.requires_grad_(False)
+        for i, enc in enumerate(encs):
+            handles.append(enc.layers[0][0].fn.attend.register_forward_hook(keep_attn(i)))
+        for t in towers:
+            handles.append(t.register_forward_hook(leaf))
+        with torch.enable_grad() if weighted else torch.no_grad():
+            outs = model(*inputs)
+            if len(probs) != len(encs) or "dhw" not in grid:
+                raise RuntimeError("cross_attention: the fusion transformer or a tower did not run in the model's forward pass")
+            attns = [probs[i] for i in range(len(encs))]
+            grads = [None] * len(encs)
+            if weighted:
+                logits = outs[0] if isinstance(outs, (tuple, list)) else outs
+                idx = _target_index(target, B, logits.device, "cross_attention")
+                objective = logits.gather(1, idx.view(-1, 1)).sum()
+                grads = list(torch.autograd.grad(objective, attns))
+    finally:
+        for h in handles:
+            h.remove()
+        for p, f in flags:
+            p.requires_grad_(f)
+    d, h, w = grid["dhw"]
+    N = d * h * w
+    maps = []
+    if isinstance(fuser, CrossTransformer_MOD_AVG):
+        r = torch.empty((2, B, N), dtype=torch.float32, device=attns[0].device)     # [mri map, pet map]
+        for i, (a, g) in enumerate(zip(attns, grads)):
+            # mri_enc (even i): MRI queries, PET keys -> the PET map; pet_enc: the MRI map
+            M, _ = TF.attn_relevance(a, g, r[1 - i % 2], accumulate=i >= 2)
+            maps.append(M)
+        r = r.view(2, B, d, h, w)
+    else:
+        rr = torch.empty((B, 2 * N), dtype=torch.float32, device=attns[0].device)
+        for i, (a, g) in enumerate(zip(attns, grads)):
+            M, _ = TF.attn_relevance(a, g, rr, accumulate=i > 0)
+            maps.append(M)
+        r = torch.stack([rr[:, :N], rr[:, N:]]).view(2, B, d, h, w)
+    size = tuple(inputs[0].shape[2:]) if upsample else (d, h, w)
+    mri, pet = TF.map_resample(r, size, normalize)
+    pairs = [(maps[2 * l], maps[2 * l + 1]) for l in range(len(maps) // 2)]
+    return CrossAttention(pairs, mri, pet)

@@ -316,7 +316,13 @@ class Attention(nn.Module):
             context = torch.cat((x, context), dim=1)
         q = TF.linear(x, self.to_q.weight)
         kv = TF.linear(context, self.to_kv.weight)
-        out = TF.attention_core(q, kv, self.heads, self.scale)
+        if _attend_hooked(self.attend):
+            tap = TF.AttnTap()
+            out, dots, attn = TF.attention_core(q, kv, self.heads, self.scale, tap)
+            out = TF.attn_tap(out, attn, tap)
+            _fire_attend_hooks(self.attend, dots, attn)
+        else:
+            out = TF.attention_core(q, kv, self.heads, self.scale)
         proj, drop = self.to_out[0], self.to_out[1]
         if _dropout_active(drop):
             y = drop(TF.linear(out, proj.weight, proj.bias))
@@ -375,18 +381,83 @@ class Transformer(nn.Module):
         return (A.to_out[0].bias is not None and F.net[0].bias is not None and F.net[3].bias is not None and
                 TF.encoder_supported(dim, A.to_q.weight.shape[0], F.net[0].weight.shape[0]) and context.shape[-1] == dim)
 
+    def _dead_hook_scan(self, fused):
+        """Warn, once per module, about hooks on children whose forward never runs: the nn.Linear / nn.LayerNorm / nn.GELU
+        parameter containers, an inactive nn.Dropout and, on the fused path, PreNorm / Attention / FeedForward as well."""
+        for pair in self.layers:
+            for pre in pair:
+                mods = [pre.norm, *pre.fn.children()] + (list(pre.fn.net) if isinstance(pre.fn, FeedForward) else
+                                                         list(pre.fn.to_out))
+                if fused:
+                    mods += [pre, pre.fn]
+                for m in mods:
+                    if m is getattr(pre.fn, "attend", None):
+                        continue
+                    if isinstance(m, nn.Dropout) and not fused and _dropout_active(m):
+                        continue
+                    _warn_dead_hook(m)
+        _warn_dead_hook(self.norm)
+
     def forward(self, x, context=None, add_input=False):
         """``add_input`` fuses the caller's outer residual ``enc(x) + x`` into the final LayerNorm kernel."""
         if self._can_fuse(x, context):
             attn, ff = self.layers[0]          # the whole encoder in 3 launches (csrc/enc_fused.cu)
-            return TF.encoder(x, context, attn.fn.heads, attn.fn.scale, add_input, attn.norm.eps, ff.norm.eps,
-                              self.norm.eps, self._fused_params(), pack_cache=self._enc_pack)
+            self._dead_hook_scan(True)
+            tap = TF.AttnTap() if _attend_hooked(attn.fn.attend) else None
+            y = TF.encoder(x, context, attn.fn.heads, attn.fn.scale, add_input, attn.norm.eps, ff.norm.eps,
+                           self.norm.eps, self._fused_params(), pack_cache=self._enc_pack, tap=tap)
+            if tap is None:
+                return y
+            y, dots, probs = y
+            y = TF.attn_tap(y, probs, tap)
+            _fire_attend_hooks(attn.fn.attend, dots, probs)
+            return y
+        self._dead_hook_scan(False)
         x_in = x
         for attn, ff in self.layers:
             x = attn(x, context=context, residual=x)
             x = ff(x, residual=x)
         return TF.layer_norm(x, self.norm.weight, self.norm.bias, residual=x_in if add_input else None,
                              eps=self.norm.eps)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# attention probabilities for module hooks and attention maps   (DESIGN section 3.8)
+# ---------------------------------------------------------------------------------------------------------------
+def _attend_hooked(attend):
+    """Whether ``Attention.attend`` has hooks to fire: the attention node then also returns ``dots`` / ``attn``."""
+    if _has_backward_hooks(attend):
+        raise NotImplementedError("backward hooks on Attention.attend are not supported (the softmax runs inside fused "
+                                  "kernels): register a tensor hook on `attn` from a forward hook (attn.register_hook), "
+                                  "or use torch.autograd.grad with respect to it")
+    return bool(attend._forward_hooks or attend._forward_pre_hooks)
+
+
+def _warn_dead_hook(m):
+    if (m._forward_hooks or m._forward_pre_hooks or _has_backward_hooks(m)) and m not in _WARNED:
+        _WARNED.add(m)
+        warnings.warn(f"a hook on {type(m).__name__} inside a fusion Transformer never fires: the encoder runs as fused "
+                      f"kernels and this module's forward is never called. Hook the attention probabilities at "
+                      f"Attention.attend, or the Transformer itself", UserWarning, stacklevel=5)
+
+
+def _fire_attend_hooks(attend, dots, attn):
+    """``nn.Module.__call__``'s hooks of the reference's ``attn = self.attend(dots)``: pre-hooks get (dots,), forward hooks
+    (module, (dots,), attn); they may only observe."""
+    versions = (dots._version, attn._version)
+    for hid, hook in list(attend._forward_pre_hooks.items()):
+        res = hook(attend, (dots,), {}) if hid in attend._forward_pre_hooks_with_kwargs else hook(attend, (dots,))
+        if res is not None:
+            raise NotImplementedError("a forward pre-hook on Attention.attend returned a replacement input: the softmax "
+                                      "runs inside fused kernels, so its hooks may only observe")
+    for hid, hook in list(attend._forward_hooks.items()):
+        res = hook(attend, (dots,), {}, attn) if hid in attend._forward_hooks_with_kwargs else hook(attend, (dots,), attn)
+        if res is not None:
+            raise NotImplementedError("a forward hook on Attention.attend returned a replacement output: the softmax runs "
+                                      "inside fused kernels, so its hooks may only observe")
+    if (dots._version, attn._version) != versions:
+        raise RuntimeError("a hook modified the attention scores or probabilities in place; the model used the values "
+                           "from before the change. Hooks on Attention.attend may only observe (clone to modify)")
 
 
 class _TokenGAP(nn.Module):
