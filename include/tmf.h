@@ -318,6 +318,40 @@ int64_t tmf_map_resample_workspace_bytes(int ng, int B, int d, int h, int w, int
 int tmf_map_resample(int ng, const float* lo, float* const* out, int B, int d, int h, int w, int D, int H, int W, int normalize,
                      void* ws, size_t ws_bytes, void* stream);
 
+/* ---- layer-wise relevance propagation through the sNet towers (DESIGN section 3.9) --------------------------------------
+ * rule TMF_LRP_EPSILON: s = R / stab(y) (y: the stored folded pre-activation, bias included); TMF_LRP_ZPLUS: s = R / stab(z+)
+ * with z+ = conv(a, w+) (no bias) and the redistribution through w+ = max(w_folded, 0).  stab(z) = z + eps*sign(z), sign(0) =
+ * +1; s = 0 where stab(z) == 0.  Totals: fp32 [B][8] per tower (column `col` written), per-CTA partial rows added in index
+ * order (no atomics: bitwise reproducible, a tower's bits do not depend on ng).
+ * tmf_lrp_fold_pack: eval BatchNorm folded into the conv weight as tmf_fold_bn_pack does (positive part for zplus): wf
+ * [tap][Cout][Cin] and wd [taps-1-tap][Cin][Cout] bf16 packs, w32 fp32 (Cout,Cin,k,k,k) and the folded bias (each of wf / wd
+ * / w32 may be NULL).
+ * tmf_lrp_ratio: R = up_a * up_c (pooled [B][D/p][H/p][W/p][C]; fp32 with up_fp32, else bf16) routed through the pool
+ * (max: to the first maximum of y in (d,h,w) scan order; avg: in proportion to LeakyReLU(y), stabilised window sum; none)
+ * and divided by stab(zp ? zp : y) (bf16 [B][D][H][W][C]) -> s bf16 [B][D][H][W][C], zero where no complete window covers
+ * a voxel; totals[:, col] = sum of R.  C a multiple of 8; 16-byte aligned tensors; ws of tmf_lrp_ratio_workspace_bytes.
+ * tmf_lrp_conv1: block 1.  s from the pooled a1 / c1 (bf16 [B][D/2][H/2][W/2][Cout]), y (and zp) as tmf_lrp_ratio with
+ * pool = max, then R_x = x * conv_transpose(s, w) with w the fp32 rule weight (Cout,1,3,3,3) and x fp32 [B][D][H][W]:
+ * rx fp32 [B][D][H][W]; totals[:, 6] = sum a1 * c1, totals[:, 7] = sum R_x.  impl as tmf_conv1_dgrad_fused
+ * (tmf_lrp_conv1_impl resolves TMF_CONV_AUTO); ws of tmf_lrp_conv1_workspace_bytes.
+ * tmf_lrp_normalize: map[g][b] /= max |map[g][b]| (unchanged where that is 0), per of [B][per] fp32. */
+#define TMF_LRP_EPSILON 0
+#define TMF_LRP_ZPLUS 1
+int tmf_lrp_fold_pack(int ng, const float* const* w, const float* const* conv_bias, const float* const* gamma,
+                      const float* const* beta, const float* const* running_mean, const float* const* running_var,
+                      void* const* wf, void* const* wd, float* const* w32, float* const* bias_out, int cout, int cin,
+                      int ksize, float eps, int rule, void* stream);
+int64_t tmf_lrp_ratio_workspace_bytes(int ng, int B, int D, int H, int W, int C, int pool);
+int tmf_lrp_ratio(int ng, const void* const* up_a, const void* const* up_c, int up_fp32, const void* const* y,
+                  const void* const* zp, void* const* s, float* const* totals, int col, int B, int D, int H, int W, int C,
+                  int pool, float slope, float eps, void* ws, size_t ws_bytes, void* stream);
+int tmf_lrp_conv1_impl(int ng, int impl, int B, int D, int H, int W, int cout);
+int64_t tmf_lrp_conv1_workspace_bytes(int ng, int impl, int B, int D, int H, int W, int cout);
+int tmf_lrp_conv1(int ng, const void* const* a1, const void* const* c1, const void* const* y, const void* const* zp,
+                  const float* const* w, const float* const* x, float* const* rx, float* const* totals, int B, int D, int H,
+                  int W, int cout, float eps, int impl, void* ws, size_t ws_bytes, void* stream);
+int tmf_lrp_normalize(int ng, float* const* map, int B, int64_t per, void* stream);
+
 /* ---- attention maps of the fusion transformer (DESIGN section 3.8) ------------------------------------------------------
  * tmf_attn_scores: per-head product of the attention core's operands (q / kv as for tmf_attn_fwd; dh in {16, 32, 64}, any
  * Nq, Nk), written out as fp32 [B, heads, Nq, Nk]:

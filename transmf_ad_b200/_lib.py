@@ -14,6 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libtmf_sm100a.so")
 
 POOL_NONE, POOL_MAX, POOL_AVG = 0, 1, 2
+LRP_EPSILON, LRP_ZPLUS = 0, 1
 CONV_AUTO, CONV_DIRECT, CONV_UMMA = 0, 1, 2
 
 _vp, _i, _i64, _f = C.c_void_p, C.c_int, C.c_int64, C.c_float
@@ -40,6 +41,10 @@ SIGNATURES = {
     "tmf_narrow_f32": [_i, _pp, _pp, _i64, _vp],
     "tmf_gradcam": [_i, _pp, _pp, _pp] + [_i] * 10 + [_vp, C.c_size_t, _vp],
     "tmf_map_resample": [_i, _vp, _pp] + [_i] * 8 + [_vp, C.c_size_t, _vp],
+    "tmf_lrp_fold_pack": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _f, _i, _vp],
+    "tmf_lrp_ratio": [_i, _pp, _pp, _i, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp, C.c_size_t, _vp],
+    "tmf_lrp_conv1": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _i, _vp, C.c_size_t, _vp],
+    "tmf_lrp_normalize": [_i, _pp, _i, _i64, _vp],
     "tmf_attn_scores": [_i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp],
     "tmf_attn_relevance": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "tmf_bn_maxpool_bwd_reduce_kept": [_i, _pp, _i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp],
@@ -86,7 +91,9 @@ PLAIN = {"tmf_last_error": (C.c_char_p, []), "tmf_version": (_i, []), "tmf_check
          "tmf_conv3d_umma_plan_info": (_i, [_i] * 8 + [C.POINTER(C.c_int)]),
          "tmf_conv3d_col_plan_info": (_i, [_i] * 7 + [C.POINTER(C.c_int)]),
          "tmf_conv1_bwd_fused_workspace_bytes": (_i64, [_i] * 6), "tmf_conv1_dgrad_fused_workspace_bytes": (_i64, [_i] * 7),
-         "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_gradcam_workspace_bytes": (_i64, [_i] * 11), "tmf_map_resample_workspace_bytes": (_i64, [_i] * 9),"tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
+         "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_gradcam_workspace_bytes": (_i64, [_i] * 11), "tmf_map_resample_workspace_bytes": (_i64, [_i] * 9),
+         "tmf_lrp_ratio_workspace_bytes": (_i64, [_i] * 7), "tmf_lrp_conv1_workspace_bytes": (_i64, [_i] * 7),
+         "tmf_lrp_conv1_impl": (_i, [_i] * 7), "tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
 
 _lib = None
 _device_checked = False

@@ -200,6 +200,12 @@ __device__ __forceinline__ uint4 pack8(const float* f) {
   return v;
 }
 
+// LRP's stabilised ratio (lrp.cu, conv1_dgrad.cu): r / (z + eps*sign(z)) with sign(0) = +1, and 0 where that denominator is 0
+__device__ __forceinline__ float lrp_div(float r, float z, float eps) {
+  const float st = __fadd_rn(z, z >= 0.f ? eps : -eps);
+  return st != 0.f ? __fdiv_rn(r, st) : 0.f;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

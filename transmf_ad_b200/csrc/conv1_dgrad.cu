@@ -39,6 +39,7 @@ constexpr uint32_t C1D_OFF_X = C1D_OFF_ACC + 4u * C1D_HB * 128u * 4u;
 constexpr uint32_t C1D_OFF_COEF = C1D_OFF_X + 2u * 2u * 9u * C1D_XW * 4u;   // per channel A, Bc, scale, shift (fp32)
 constexpr uint32_t C1D_OFF_BAR = C1D_OFF_COEF + 4u * 32u * 4u;
 constexpr uint32_t C1D_SMEM = 1024u + C1D_OFF_BAR + 64u;
+constexpr uint32_t C1D_SMEM_LRP = C1D_SMEM + 4u * C1D_THREADS;   // + one relevance partial sum per thread
 
 struct C1DParams {
   const __nv_bfloat16* y[TMF_MAX_GROUPS];
@@ -50,6 +51,12 @@ struct C1DParams {
   int B, D, H, W, DP, HP, WC, nbands, chunk;
   uint32_t idesc;
   float slope;
+  // LRP front (tmf_lrp_conv1): dout = c1, y, zp (or NULL) and a1 build s; dx = R_x = x * (W^T s); part: per-CTA partial sums
+  const __nv_bfloat16* a1[TMF_MAX_GROUPS];
+  const __nv_bfloat16* zp[TMF_MAX_GROUPS];
+  const float* x[TMF_MAX_GROUPS];
+  float* part[TMF_MAX_GROUPS];
+  float eps;
 };
 
 __device__ __forceinline__ uint32_t c1d_sw64(int r, int j) { return (uint32_t)r * 64u + (uint32_t)((j ^ ((r >> 1) & 3)) << 4); }
@@ -63,6 +70,9 @@ __device__ __forceinline__ uint32_t c1d_beq(uint32_t a, uint32_t b) {
 }
 __device__ __forceinline__ uint32_t c1d_get(const uint4& v, int i) { return i == 0 ? v.x : (i == 1 ? v.y : (i == 2 ? v.z : v.w)); }
 
+// LRP = false: the saliency front (dy from the BatchNorm / LeakyReLU / MaxPool backward apply); LRP = true: the relevance
+// front (s = a1 * c1 / stab(z) at each window's first maximum of y, zero elsewhere) and an epilogue that writes x * (W^T s).
+template <bool LRP>
 __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const __grid_constant__ C1DParams p) {
   pdl_entry();
   extern __shared__ uint8_t smem_raw[];
@@ -111,7 +121,7 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
   for (int i = threadIdx.x; i < 4 * C1D_HB * 128; i += C1D_THREADS) acc[i] = 0.f;
   for (int i = threadIdx.x; i < 2 * 2 * 9 * C1D_XW; i += C1D_THREADS) xch[i] = 0.f;
   float* cf = reinterpret_cast<float*>(gen + C1D_OFF_COEF);                   // in shared memory: 32 registers fewer per builder
-  if (threadIdx.x < 32) {
+  if (!LRP && threadIdx.x < 32) {
     const int c = threadIdx.x;
     const float sc = p.coef[g][c], sh = p.coef[g][32 + c], mu = p.coef[g][64 + c], is = p.coef[g][96 + c];
     const float m1 = p.bcoef[g][c], m2 = p.bcoef[g][32 + c];
@@ -126,6 +136,7 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(gen + C1D_OFF_BAR + 48);
+  float bsum = 0.f, esum = 0.f;                          // LRP: relevance entering block 1 (owned windows) / R_x written
 
   if (warp == 4) {
     // =========================================== MMA issuer =============================================
@@ -169,6 +180,7 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
       if (u >= 2) mbar_wait(mma_done + 8 * grp, (uint32_t)((u >> 1) - 1) & 1u);   // the stage's previous unit is consumed
       const bool exd = 2 * j + 1 < p.D, exh = 2 * k + 1 < p.H;
       const bool pool_ok = j < Do && k < Ho;
+      const bool own = j >= j0 && j < j1 && 2 * k >= h0 && 2 * k < h0 + C1D_HB;      // LRP: windows this CTA accounts for
       const __nv_bfloat16* yu = yg + ((((int64_t)n * p.D + 2 * j) * p.H + 2 * k) * p.W) * 32 + c0;
       const __nv_bfloat16* gu = p.dout[g] + ((((int64_t)n * Do + j) * Ho + k) * Wo) * 32 + c0;
       for (int task = tb; task < p.WC * 4; task += C1D_BGROUP) {
@@ -182,6 +194,49 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
           const int off = wo * 64 + ((q & 4) ? sD : 0) + ((q & 2) ? sH : 0) + ((q & 1) ? 32 : 0);
           raw[q] = ex ? __ldg(reinterpret_cast<const uint4*>(yu + off)) : make_uint4(0u, 0u, 0u, 0u);
         }
+        if constexpr (LRP) {
+          float R[8], sv[8];
+          int wq[8];
+#pragma unroll
+          for (int c = 0; c < 8; ++c) R[c] = 0.f;
+          if (win_ok) {
+            float av[8], cv[8];
+            unpack8(__ldg(reinterpret_cast<const uint4*>(p.a1[g] + (gu - p.dout[g]) + wo * 32)), av);
+            unpack8(__ldg(reinterpret_cast<const uint4*>(gu + wo * 32)), cv);
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+              R[c] = __fmul_rn(av[c], cv[c]);
+              if (own) bsum = __fadd_rn(bsum, R[c]);
+            }
+          }
+#pragma unroll
+          for (int c = 0; c < 8; ++c) {
+            const auto ybf = [&](int q) {
+              const uint32_t v = c1d_get(raw[q], c >> 1);
+              return (c & 1) ? bf16_hi(v) : bf16_lo(v);
+            };
+            float m = ybf(0);
+            wq[c] = 0;
+#pragma unroll
+            for (int q = 1; q < 8; ++q) {
+              const float v = ybf(q);
+              if (v > m) { m = v; wq[c] = q; }
+            }
+            if (p.zp[g] != nullptr && win_ok) {
+              const int q = wq[c];
+              const int off = wo * 64 + ((q & 4) ? sD : 0) + ((q & 2) ? sH : 0) + ((q & 1) ? 32 : 0);
+              m = __bfloat162float(p.zp[g][(yu - yg) + off + c]);
+            }
+            sv[c] = win_ok ? lrp_div(R[c], m, p.eps) : 0.f;
+          }
+#pragma unroll
+          for (int q = 0; q < 8; ++q) {
+            raw[q].x = pack_bf16(wq[0] == q ? sv[0] : 0.f, wq[1] == q ? sv[1] : 0.f);
+            raw[q].y = pack_bf16(wq[2] == q ? sv[2] : 0.f, wq[3] == q ? sv[3] : 0.f);
+            raw[q].z = pack_bf16(wq[4] == q ? sv[4] : 0.f, wq[5] == q ? sv[5] : 0.f);
+            raw[q].w = pack_bf16(wq[6] == q ? sv[6] : 0.f, wq[7] == q ? sv[7] : 0.f);
+          }
+        } else {
         float go[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) go[i] = 0.f;
@@ -215,6 +270,7 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
             const uint32_t pk = pack_bf16(__uint_as_float(lo_u32(o2)), __uint_as_float(hi_u32(o2)));
             if (j2 == 0) raw[q].x = pk; else if (j2 == 1) raw[q].y = pk; else if (j2 == 2) raw[q].z = pk; else raw[q].w = pk;
           }
+        }
         }
 #pragma unroll
         for (int q = 0; q < 8; ++q) {
@@ -278,18 +334,39 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
           const bool wr = pd >= pw0 && pd < pw1 && w < p.W;
           float* dst = dxg + (((int64_t)n * p.D + pd) * p.H + h0) * p.W + w;
           for (int hr = 0; hr < C1D_HB; ++hr) {
-            if (wr && h0 + hr < p.H) dst[(int64_t)hr * p.W] = ap[hr * 128];
+            if (wr && h0 + hr < p.H) {
+              if constexpr (LRP) {
+                const float v = __fmul_rn(p.x[g][(dst - dxg) + (int64_t)hr * p.W], ap[hr * 128]);
+                dst[(int64_t)hr * p.W] = v;
+                esum = __fadd_rn(esum, v);
+              } else {
+                dst[(int64_t)hr * p.W] = ap[hr * 128];
+              }
+            }
             ap[hr * 128] = 0.f;
           }
         }
       }
     }
   }
+  float* red = reinterpret_cast<float*>(gen + C1D_OFF_BAR + 64);
+  if constexpr (LRP) red[threadIdx.x] = warp >= 5 ? bsum : (warp < 4 ? esum : 0.f);
   tc_fence_before();
   __syncthreads();
   if (warp == 4) {
     tc_fence_after();
     tmem_dealloc(tmem_base, 256);
+  }
+  if constexpr (LRP) {
+    if (threadIdx.x == 0) {
+      // fixed order: builders by thread index, then the epilogue columns by w
+      float sb = 0.f, se = 0.f;
+      for (int i = 160; i < C1D_THREADS; ++i) sb = __fadd_rn(sb, red[i]);
+      for (int i = 0; i < 128; ++i) se = __fadd_rn(se, red[i]);
+      float* pr = p.part[g] + ((int64_t)n * gridDim.x + blockIdx.x) * 2;
+      pr[0] = sb;
+      pr[1] = se;
+    }
   }
 }
 
@@ -365,6 +442,24 @@ static size_t c1d_direct_ws(int ng, int B, int D, int H, int W, int cout) {
   return (size_t)ng * ((((size_t)B * D * H * W * cout * 2) + 255) & ~(size_t)255);
 }
 
+size_t lrp_ratio_ws(int ng, int B, int D, int H, int W, int C, int pool);
+int lrp_blocks(int64_t items);
+int lrp_sum_rows(int ng, float* const* part, float* const* totals, int B, int rows, int K, int col, cudaStream_t st);
+int lrp_xmul(int ng, const float* const* x, float* const* rx, float* const* totals, int col, int B, int64_t per, float* part,
+             cudaStream_t st);
+
+static size_t c1d_align(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// LRP on the CUDA-core path: [s (bf16, per tower)] [ratio partial rows] [x-multiply partial rows]
+static size_t c1d_lrp_direct_ws(int ng, int B, int D, int H, int W, int cout) {
+  return c1d_direct_ws(ng, B, D, H, W, cout) + lrp_ratio_ws(ng, B, D, H, W, cout, TMF_POOL_MAX) +
+         c1d_align((size_t)ng * B * lrp_blocks((int64_t)D * H * W) * sizeof(float));
+}
+
+// The tcgen05 LRP instance plans its grid as for two towers whatever ng is: the per-CTA partial rows of the totals then
+// cover the same voxels, and a tower's totals do not depend on whether it runs alone or paired.
+static C1DPlan c1d_lrp_plan(int B, int D, int H) { return c1d_plan(TMF_MAX_GROUPS, B, D, H); }
+
 }  // namespace tmf
 
 using namespace tmf;
@@ -412,10 +507,10 @@ int tmf_conv1_dgrad_fused(int ng, const void* const* dout, const void* const* y,
     p.slope = slope;
     static bool attr_done = false;
     if (!attr_done) {
-      TMF_CUDA(cudaFuncSetAttribute(conv1_dgrad_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C1D_SMEM));
+      TMF_CUDA(cudaFuncSetAttribute(conv1_dgrad_umma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C1D_SMEM));
       attr_done = true;
     }
-    launch_k(conv1_dgrad_umma_kernel, dim3(pl.nbands * pl.nchunks, B, ng), C1D_THREADS, C1D_SMEM, st, p);
+    launch_k(conv1_dgrad_umma_kernel<false>, dim3(pl.nbands * pl.nchunks, B, ng), C1D_THREADS, C1D_SMEM, st, p);
     TMF_LAUNCH_CHECK();
     return 0;
   }
@@ -439,6 +534,93 @@ int tmf_conv1_dgrad_fused(int ng, const void* const* dout, const void* const* y,
   launch_k(conv1_dgrad_direct_kernel, grid, 256, 0, st, gdy, gw, gdx, B, D, H, W, cout);
   TMF_LAUNCH_CHECK();
   return 0;
+}
+
+int tmf_lrp_ratio(int ng, const void* const* up_a, const void* const* up_c, int up_fp32, const void* const* y,
+                  const void* const* zp, void* const* s, float* const* totals, int col, int B, int D, int H, int W, int C,
+                  int pool, float slope, float eps, void* ws, size_t ws_bytes, void* stream);
+
+int tmf_lrp_conv1_impl(int ng, int impl, int B, int D, int H, int W, int cout) {
+  if (impl == TMF_CONV_AUTO) impl = c1d_umma_supported(ng, B, D, H, W, cout) ? TMF_CONV_UMMA : TMF_CONV_DIRECT;
+  return impl;
+}
+
+int64_t tmf_lrp_conv1_workspace_bytes(int ng, int impl, int B, int D, int H, int W, int cout) {
+  impl = tmf_lrp_conv1_impl(ng, impl, B, D, H, W, cout);
+  if (impl == TMF_CONV_DIRECT) return (int64_t)c1d_lrp_direct_ws(ng, B, D, H, W, cout);
+  const C1DPlan pl = c1d_lrp_plan(B, D, H);
+  return (int64_t)c1d_align((size_t)ng * B * pl.nbands * pl.nchunks * 2 * sizeof(float));
+}
+
+int tmf_lrp_conv1(int ng, const void* const* a1, const void* const* c1, const void* const* y, const void* const* zp,
+                  const float* const* w, const float* const* x, float* const* rx, float* const* totals, int B, int D, int H,
+                  int W, int cout, float eps, int impl, void* ws, size_t ws_bytes, void* stream) {
+  TMF_CHECK_NG(ng);
+  TMF_REQUIRE(B >= 1 && B <= 65535 && D >= 1 && H >= 1 && W >= 1, "lrp_conv1: empty problem (%d,%d,%d,%d)", B, D, H, W);
+  TMF_REQUIRE(eps >= 0.f, "lrp_conv1: eps must be >= 0");
+  impl = tmf_lrp_conv1_impl(ng, impl, B, D, H, W, cout);
+  cudaStream_t st = (cudaStream_t)stream;
+  for (int g = 0; g < ng; ++g) {
+    TMF_REQUIRE(a1 && c1 && y && w && x && rx && totals && a1[g] && c1[g] && y[g] && w[g] && x[g] && rx[g] && totals[g],
+                "lrp_conv1: NULL device pointer");
+    TMF_REQUIRE((((uintptr_t)a1[g] | (uintptr_t)c1[g] | (uintptr_t)y[g]) & 15) == 0,
+                "lrp_conv1: a1 / c1 / y must be 16-byte aligned");
+  }
+  const int64_t need = tmf_lrp_conv1_workspace_bytes(ng, impl, B, D, H, W, cout);
+  TMF_REQUIRE(ws != nullptr && ws_bytes >= (size_t)need && ((uintptr_t)ws & 255) == 0,
+              "lrp_conv1: needs a 256-byte aligned workspace of %lld bytes (got %zu)", (long long)need, ws_bytes);
+  if (impl == TMF_CONV_UMMA) {
+    TMF_REQUIRE(c1d_umma_supported(ng, B, D, H, W, cout), "lrp_conv1: tcgen05 path needs Cout = 32 and W <= 128 (got Cout=%d, W=%d)",
+                cout, W);
+    const C1DPlan pl = c1d_lrp_plan(B, D, H);
+    const int rows = pl.nbands * pl.nchunks;
+    C1DParams p{};
+    float* part[TMF_MAX_GROUPS] = {nullptr, nullptr};
+    for (int g = 0; g < ng; ++g) {
+      p.y[g] = (const __nv_bfloat16*)y[g];
+      p.dout[g] = (const __nv_bfloat16*)c1[g];
+      p.a1[g] = (const __nv_bfloat16*)a1[g];
+      p.zp[g] = zp != nullptr ? (const __nv_bfloat16*)zp[g] : nullptr;
+      p.w[g] = w[g];
+      p.x[g] = x[g];
+      p.dx[g] = rx[g];
+      part[g] = p.part[g] = (float*)ws + (size_t)g * B * rows * 2;
+    }
+    p.B = B; p.D = D; p.H = H; p.W = W;
+    p.DP = (D + 1) / 2; p.HP = (H + 1) / 2; p.WC = (W + 1) / 2;
+    p.nbands = pl.nbands; p.chunk = pl.chunk;
+    p.idesc = make_idesc_bf16(128, 32, 0, 0);
+    p.eps = eps;
+    static bool attr_done = false;
+    if (!attr_done) {
+      TMF_CUDA(cudaFuncSetAttribute(conv1_dgrad_umma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C1D_SMEM_LRP));
+      attr_done = true;
+    }
+    launch_k(conv1_dgrad_umma_kernel<true>, dim3(rows, B, ng), C1D_THREADS, C1D_SMEM_LRP, st, p);
+    TMF_LAUNCH_CHECK();
+    return lrp_sum_rows(ng, part, totals, B, rows, 2, 6, st);
+  }
+  TMF_REQUIRE(impl == TMF_CONV_DIRECT, "lrp_conv1: unknown impl %d", impl);
+  TMF_REQUIRE(cout >= 8 && cout <= 64 && cout % 8 == 0, "lrp_conv1: Cout must be a multiple of 8 in [8,64] (got %d)", cout);
+  // s at full resolution (the ratio pass with block 1's max-pool), then the fp32 direct data gradient, then x * c
+  const size_t per = c1d_direct_ws(1, B, D, H, W, cout);
+  const size_t rws = lrp_ratio_ws(ng, B, D, H, W, cout, TMF_POOL_MAX);
+  void* sp[TMF_MAX_GROUPS] = {nullptr, nullptr};
+  for (int g = 0; g < ng; ++g) sp[g] = (uint8_t*)ws + (size_t)g * per;
+  uint8_t* rbase = (uint8_t*)ws + (size_t)ng * per;
+  if (tmf_lrp_ratio(ng, a1, c1, 0, y, zp, sp, totals, 6, B, D, H, W, cout, TMF_POOL_MAX, 0.f, eps, rbase, rws, stream) != 0)
+    return 1;
+  GroupPtr<const __nv_bfloat16> gs;
+  GroupPtr<const float> gw;
+  GroupPtr<float> gx;
+  if (!load_group(gs, (const __nv_bfloat16* const*)sp, ng, true, "s") || !load_group(gw, w, ng, true, "w") ||
+      !load_group(gx, rx, ng, true, "rx"))
+    return 1;
+  const long long total = (long long)B * D * H * W;
+  dim3 grid((unsigned)std::min((total + 255) / 256, 148LL * 16), 1, ng);
+  launch_k(conv1_dgrad_direct_kernel, grid, 256, 0, st, gs, gw, gx, B, D, H, W, cout);
+  TMF_LAUNCH_CHECK();
+  return lrp_xmul(ng, x, rx, totals, 7, B, (int64_t)D * H * W, (float*)(rbase + rws), st);
 }
 
 }  // extern "C"

@@ -190,7 +190,7 @@ class SNetRun:
     the call site: inside ``Function.forward`` grad mode is always off), and the hyper-parameters read from the
     ``nn.BatchNorm3d`` / ``nn.LeakyReLU`` children -- per layer (eps, momentum, negative_slope)."""
 
-    def __init__(self, training, grad_enabled, hyper=None, packs=None, folds=None, sync_group=False):
+    def __init__(self, training, grad_enabled, hyper=None, packs=None, folds=None, sync_group=False, keep=None):
         self.training, self.grad_enabled = bool(training), bool(grad_enabled)
         self.hyper = hyper if hyper is not None else [(BN_EPS, BN_MOMENTUM, LRELU_SLOPE)] * 7
         self.packs = packs              # per tower: 7 ConvPack (index 0 unused: conv1.0 consumes the fp32 weight)
@@ -198,6 +198,8 @@ class SNetRun:
         # False: per-rank BatchNorm statistics (DDP semantics, the default).  None / a process group: the BatchNorm3d children
         # are nn.SyncBatchNorm (torch.nn.SyncBatchNorm.convert_sync_batchnorm(model)): statistics over the GLOBAL batch
         self.sync_group = sync_group
+        # per tower: a list (or None) that the folded eval path appends (input activation, y) to, layer by layer (LRP)
+        self.keep = keep
 
 
 def _sync_world(group):
@@ -413,6 +415,9 @@ class SNetFunction(torch.autograd.Function):
                 for fo, (_, sig) in zip(folds, state):
                     fo.sig = sig
             y = [torch.empty((B, Dl, Hl, Wl, cout), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
+            for t, kept in enumerate(run.keep or ()):
+                if kept is not None:
+                    kept.append((act[t], y[t]))
             bias = [fo.bias for fo in folds]
             if l == 0:
                 L.call("tmf_conv1_fwd", ng, L.ptrs(act), L.ptrs([fo.w32 for fo in folds]), L.ptrs(bias), L.ptrs(y), L.ptrs(None),
@@ -1086,3 +1091,111 @@ def gradcam(acts, grads, size=None, normalize=True):
         L.call("tmf_gradcam", ng, L.ptrs(A[i:i + ng]), L.ptrs(G[i:i + ng]), L.ptrs(cams[i:i + ng]), B, d, h, w, C, D, H, W,
                ups, int(normalize), L.ptr(ws), nws)
     return cams
+
+
+# ==============================================================================================================
+# Layer-wise relevance propagation   (csrc/lrp.cu, csrc/conv1_dgrad.cu; DESIGN section 3.9)
+# ==============================================================================================================
+LRP_RULES = {"epsilon": L.LRP_EPSILON, "zplus": L.LRP_ZPLUS}
+
+
+class LrpFold:
+    """One conv layer's eval-mode BatchNorm fold for an LRP rule (``tmf_lrp_fold_pack``): the bf16 forward pack ``wf`` (the
+    z+ convolution; rule zplus only), the bf16 dgrad pack ``wd`` (layers 1-6), the fp32 weight ``w32`` (layer 0) and the folded
+    bias.  Rebuilt on the signature ``EvalFold`` uses: parameter / running-statistics addresses and versions and the epoch."""
+
+    def __init__(self):
+        self.sig = None
+        self.wf = self.wd = self.w32 = self.bias = None
+
+    def refresh(self, l, rule, tensors, bn_eps):
+        w = tensors[0]
+        sig = (_PARAM_EPOCH[0],) + tuple((t.data_ptr(), t._version) for t in tensors)
+        if self.bias is None or self.bias.device != w.device:
+            cout, cin, k = w.shape[0], w.shape[1], w.shape[2]
+            self.bias = torch.empty(cout, dtype=torch.float32, device=w.device)
+            if l == 0:
+                self.w32 = torch.empty_like(w)
+            else:
+                self.wd = torch.empty((k ** 3, cin, cout), dtype=torch.bfloat16, device=w.device)
+                if rule == L.LRP_ZPLUS:
+                    self.wf = torch.empty((k ** 3, cout, cin), dtype=torch.bfloat16, device=w.device)
+            self.sig = None
+        if sig == self.sig:
+            return
+        cout, cin, k = w.shape[0], w.shape[1], w.shape[2]
+        L.call("tmf_lrp_fold_pack", 1, *[L.ptrs([t]) for t in tensors], L.ptrs([self.wf]), L.ptrs([self.wd]),
+               L.ptrs([self.w32]), L.ptrs([self.bias]), cout, cin, k, float(bn_eps), rule)
+        self.sig = sig
+
+
+def lrp_conv1_impl(B, D, H, W, cout, ng=1):
+    """The block-1 LRP implementation ``tmf_lrp_conv1`` takes for this problem: ``L.CONV_UMMA`` (tcgen05) or
+    ``L.CONV_DIRECT`` (CUDA cores: ``TMF_CONV_IMPL=direct``, rows wider than 128 voxels, Cout != 32)."""
+    return int(L.load().tmf_lrp_conv1_impl(ng, conv_impl(), B, D, H, W, cout))
+
+
+def lrp_towers(spec, hyper, folds, layer_params, kept, seeds, rule="epsilon", eps=1e-6):
+    """LRP sweep, layer 6 down to 0, through one or two towers of the same shape in one launch sequence.
+
+    ``folds[t]``: 7 ``LrpFold`` of tower t (cached by the caller); ``layer_params[t][l]``: (conv.weight, conv.bias, bn.weight,
+    bn.bias, running_mean, running_var); ``kept[t]``: the 7 (input activation, y) pairs the folded eval forward kept (layer 0:
+    the fp32 (B,1,D,H,W) volume); ``seeds[t]``: (a_T, g_T), fp32 (B,d,h,w,C) contiguous, whose product is the relevance at the
+    tower output.  Returns (maps, totals): per tower an fp32 (B,1,D,H,W) relevance map and an fp32 (B, 8) tensor of per-sample
+    relevance sums (the tower output, then entering layers 6 .. 0)."""
+    rc = LRP_RULES[rule]
+    ng = len(kept)
+    impl = conv_impl()
+    x = [k[0][0] for k in kept]
+    B, _, D, H, W = x[0].shape
+    dev = x[0].device
+    totals = list(torch.empty((ng, B, 8), dtype=torch.float32, device=dev).unbind(0))
+    c = None
+    for l in range(len(spec.layers) - 1, -1, -1):
+        cin, cout, ks, pool = spec.layers[l]
+        bn_eps, _, slope = hyper[l]
+        for t in range(ng):
+            folds[t][l].refresh(l, rc, layer_params[t][l], bn_eps)
+        fl = [folds[t][l] for t in range(ng)]
+        act = [k[l][0] for k in kept]
+        y = [k[l][1] for k in kept]
+        Dl, Hl, Wl = y[0].shape[1:4]
+        zp = None
+        if rc == L.LRP_ZPLUS:
+            zp = [torch.empty_like(v) for v in y]
+            zero = torch.zeros(cout, dtype=torch.float32, device=dev)
+            if l == 0:
+                L.call("tmf_conv1_fwd", ng, L.ptrs(act), L.ptrs([f.w32 for f in fl]), L.ptrs([zero] * ng), L.ptrs(zp),
+                       L.ptrs(None), B, Dl, Hl, Wl, cout, impl)
+            else:
+                L.call("tmf_conv3d_fwd", ng, L.ptrs(act), L.ptrs([f.wf for f in fl]), L.ptrs([zero] * ng), L.ptrs(zp),
+                       L.ptrs(None), B, Dl, Hl, Wl, cin, cout, ks, impl, tag=f"tmf_conv3d_fwd@L{l}")
+        if l == 0:
+            a1 = [k[1][0] for k in kept]
+            rx = [torch.empty((B, 1, D, H, W), dtype=torch.float32, device=dev) for _ in range(ng)]
+            nws = int(L.load().tmf_lrp_conv1_workspace_bytes(ng, impl, B, D, H, W, cout))
+            ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+            L.call("tmf_lrp_conv1", ng, L.ptrs(a1), L.ptrs(c), L.ptrs(y), L.ptrs(zp), L.ptrs([f.w32 for f in fl]), L.ptrs(x),
+                   L.ptrs(rx), L.ptrs(totals), B, D, H, W, cout, float(eps), impl, L.ptr(ws), nws)
+            return rx, totals
+        if l == len(spec.layers) - 1:
+            up_a, up_c, up32, col = [s[0] for s in seeds], [s[1] for s in seeds], 1, 0
+        else:
+            up_a, up_c, up32, col = [k[l + 1][0] for k in kept], c, 0, len(spec.layers) - 1 - l
+        s = [torch.empty_like(v) for v in y]
+        nws = int(L.load().tmf_lrp_ratio_workspace_bytes(ng, B, Dl, Hl, Wl, cout, pool))
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        L.call("tmf_lrp_ratio", ng, L.ptrs(up_a), L.ptrs(up_c), up32, L.ptrs(y), L.ptrs(zp), L.ptrs(s), L.ptrs(totals), col,
+               B, Dl, Hl, Wl, cout, pool, float(slope), float(eps), L.ptr(ws), nws, tag=f"tmf_lrp_ratio@L{l}")
+        c = [torch.empty((B, Dl, Hl, Wl, cin), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
+        L.call("tmf_conv3d_fwd", ng, L.ptrs(s), L.ptrs([f.wd for f in fl]), L.ptrs(None), L.ptrs(c), L.ptrs(None),
+               B, Dl, Hl, Wl, cout, cin, ks, impl, tag=f"tmf_conv3d_dgrad@L{l}")
+
+
+def lrp_normalize(maps):
+    """Divide each sample of each fp32 (B,1,D,H,W) map by its max |R|, in place (a map that is zero stays zero)."""
+    for i in range(0, len(maps), 2):
+        grp = maps[i:i + 2]
+        B = grp[0].shape[0]
+        L.call("tmf_lrp_normalize", len(grp), L.ptrs(grp), B, grp[0].numel() // B)
+    return maps

@@ -1,5 +1,6 @@
-"""Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, and head-averaged or
-gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the fusion transformer.
+"""Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, layer-wise relevance
+propagation (Bach et al., 2015) through the towers, and head-averaged or gradient-weighted (Chefer et al., 2021)
+cross-modal attention maps of the fusion transformer.
 
 Input gradients (saliency maps) need nothing from here: ``mri.requires_grad_(True)`` and plain autograd work on every model
 (INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c), and so do
@@ -162,3 +163,95 @@ def cross_attention(model, inputs, target=None, upsample=True, normalize=True):
     mri, pet = TF.map_resample(r, size, normalize)
     pairs = [(maps[2 * l], maps[2 * l + 1]) for l in range(len(maps) // 2)]
     return CrossAttention(pairs, mri, pet)
+
+
+LRP = namedtuple("LRP", ["maps", "totals"])
+
+
+def lrp(model, inputs, target, rule="epsilon", eps=1e-6, normalize=False):
+    """Layer-wise relevance propagation (Bach et al., 2015) through every sNet tower of ``model`` (eval mode), for the
+    objective f = ``sum_b logits[b, target_b]`` of the model's first output.
+
+    The relevance at a tower output a_T is R_T = a_T * df/da_T (gradient x input: LRP-0 through the piecewise-linear heads);
+    it is propagated through the seven conv units with BatchNorm folded into the convolutions (running statistics) and one
+    ``rule`` for all of them: ``"epsilon"`` (LRP-eps; ``eps=0`` is LRP-0: the denominator is the pre-activation, bias
+    included, stabilised as z + eps*sign(z)) or ``"zplus"`` (z+: the positive part of the folded weight, no bias).  LeakyReLU
+    passes relevance unchanged, max-pool sends it to the first maximum of each window, the final avg-pool splits it in
+    proportion to the activations.  ``inputs`` and ``target`` as for ``grad_cam``.
+
+    Returns ``LRP(maps, totals)``: per tower, in tower order (``model.modules()``), an fp32 (B,1,D,H,W) signed relevance map
+    (divided per sample by its max |R| with ``normalize``) and an fp32 (B, 8) tensor of per-sample relevance sums: at the
+    tower output (column 0), then entering layers 6 .. 0 (columns 1 .. 7; column 7 is the sum of the map before
+    normalisation).
+
+    The towers run once, without autograd; no sNet backward runs, no parameter receives a ``.grad``, no weight-gradient
+    kernel runs, BatchNorm buffers and the module mode are untouched and ``requires_grad`` flags are restored."""
+    if rule not in TF.LRP_RULES:
+        raise ValueError(f"lrp: rule must be one of {tuple(TF.LRP_RULES)}; got {rule!r}")
+    if isinstance(eps, bool) or not isinstance(eps, (int, float)) or not eps >= 0 or eps == float("inf"):
+        raise ValueError(f"lrp: eps must be a finite number >= 0; got {eps!r}")
+    towers = [m for m in model.modules() if isinstance(m, sNet)]
+    if not towers:
+        raise ValueError("lrp: the model has no sNet tower")
+    if any(m.training for m in towers):
+        raise ValueError("lrp: BatchNorm is folded with its running statistics; call model.eval() first")
+    inputs = tuple(inputs) if isinstance(inputs, (tuple, list)) else (inputs,)
+    if not inputs or not all(torch.is_tensor(x) and x.dim() == 5 and x.shape[1] == 1 for x in inputs):
+        raise ValueError("lrp: inputs must be (B,1,D,H,W) volumes")
+    B = inputs[0].shape[0]
+    idx = _target_index(target, B, inputs[0].device, "lrp")
+    leaves = {}
+
+    def leaf(module, args, out):
+        o = out.detach().requires_grad_(True)
+        leaves[module] = o
+        return o
+
+    flags = [(p, p.requires_grad) for p in model.parameters()]
+    handles = []
+    try:
+        for p, _ in flags:
+            p.requires_grad_(False)
+        for t in towers:
+            t._lrp_keep = []
+            handles.append(t.register_forward_hook(leaf))
+        with torch.enable_grad():
+            outs = model(*[x.detach() for x in inputs])
+            logits = outs[0] if isinstance(outs, (tuple, list)) else outs
+            objective = logits.gather(1, idx.to(logits.device).view(-1, 1)).sum()
+            acts = [leaves.get(t) for t in towers]
+            kept = [t._lrp_keep for t in towers]
+            if any(a is None for a in acts):
+                raise RuntimeError("lrp: a tower of the model did not run in its forward pass")
+            if any(len(k) != len(t._spec.layers) for k, t in zip(kept, towers)):
+                raise RuntimeError("lrp: the towers did not run the folded eval path (TMF_EVAL_FOLD=0?)")
+            grads = torch.autograd.grad(objective, acts, allow_unused=True)
+    finally:
+        for h in handles:
+            h.remove()
+        for p, f in flags:
+            p.requires_grad_(f)
+        for t in towers:
+            t._lrp_keep = None
+    seeds = [(TF._f32c(a.detach().permute(0, 2, 3, 4, 1)),
+              TF._f32c(torch.zeros_like(a) if g is None else g.permute(0, 2, 3, 4, 1))) for a, g in zip(acts, grads)]
+    maps, totals = [None] * len(towers), [None] * len(towers)
+    i = 0
+    while i < len(towers):
+        grp = [i]
+        if (i + 1 < len(towers) and towers[i + 1]._spec.dim == towers[i]._spec.dim
+                and kept[i + 1][0][0].shape == kept[i][0][0].shape and towers[i + 1]._hyper() == towers[i]._hyper()):
+            grp.append(i + 1)
+        folds = [towers[t]._lrp_folds.setdefault(rule, [TF.LrpFold() for _ in range(7)]) for t in grp]
+        params = []
+        for t in grp:
+            params.append([(conv.weight.detach(), conv.bias.detach(), bn.weight.detach(), bn.bias.detach(), bn.running_mean,
+                            bn.running_var) for conv, bn in towers[t]._units()])
+        m, tot = TF.lrp_towers(towers[i]._spec, towers[i]._hyper(), folds, params, [kept[t] for t in grp],
+                               [seeds[t] for t in grp], rule, eps)
+        for t, mm, tt in zip(grp, m, tot):
+            maps[t], totals[t] = mm, tt
+        i += len(grp)
+    if normalize:
+        TF.lrp_normalize(maps)
+    return LRP(maps, totals)

@@ -48,6 +48,8 @@ class sNet(nn.Module):
         self._folds = [TF.EvalFold() for _ in range(7)]      # eval mode: BatchNorm folded into the conv operands
         self._cam_tap = None                                  # transmf_ad_b200.interpret.grad_cam: block index to expose
         self._cam_act = None
+        self._lrp_keep = None          # transmf_ad_b200.interpret.lrp: a list the folded eval forward appends (a, y) to
+        self._lrp_folds = {}           # LRP rule -> 7 TF.LrpFold
 
     def _units(self):
         """[(conv, bn)] in execution order."""
@@ -77,7 +79,9 @@ class sNet(nn.Module):
         if any(sync) and not all(sync):
             raise NotImplementedError("sNet: either every BatchNorm3d is an nn.SyncBatchNorm or none")
         group = self._units()[0][1].process_group if all(sync) else False
-        return TF.SNetRun(self.training, torch.is_grad_enabled(), self._hyper(), packs, folds, sync_group=group)
+        keep = [self._lrp_keep] if other is None else [self._lrp_keep, other._lrp_keep]
+        return TF.SNetRun(self.training, torch.is_grad_enabled(), self._hyper(), packs, folds, sync_group=group,
+                          keep=keep if any(k is not None for k in keep) else None)
 
     def invalidate_packs(self):
         for pk in self._packs:
