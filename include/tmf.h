@@ -52,13 +52,9 @@ int tmf_version(void);
 int tmf_check_device(void);
 /* number of kernel launches issued through this library by the calling process so far */
 int64_t tmf_launch_count(void);
-/* programmatic dependent launch of the train-step kernels (default off; TMF_PDL=1 in the environment turns it on): each
- * kernel waits for its stream predecessors before its first global access, so results are identical either way */
-int tmf_set_pdl(int on);
 /* which attention kernels tmf_attn_fwd / tmf_attn_bwd try first (TMF_ATTN_IMPL, read once): 2 = tensor-core (attention_mma.cu,
  * default), 1 = register-tiled fp32 (attention.cu), 0 = row-per-warp fp32 (fusion_ops.cu) */
 int tmf_attn_impl_default(void);
-int tmf_get_pdl(void);
 /* TMF_STAT_ROWS, for callers that size statistics buffers without the header */
 int tmf_stat_rows(void);
 
@@ -98,14 +94,6 @@ int tmf_conv1_bwd_fused(int ng, const void* const* dout, const void* const* y, c
                         const float* const* bcoef, const float* const* x, float* const* dw, int B, int D, int H,
                         int W, int cout, float slope, void* ws, size_t ws_bytes, void* stream);
 int64_t tmf_conv1_bwd_fused_workspace_bytes(int ng, int B, int D, int H, int W, int cout);
-/* The same pass in two calls: the bf16 hi/lo split of the input image depends on x alone, so a caller that knows x early
- * (the forward pass) runs tmf_conv1_bwd_split_x() ahead of time, possibly on another stream, and later calls
- * tmf_conv1_bwd_fused_presplit() with the SAME workspace (stream-ordered after the split). */
-int tmf_conv1_bwd_split_x(int ng, const float* const* x, int B, int D, int H, int W, int cout, void* ws, size_t ws_bytes,
-                          void* stream);
-int tmf_conv1_bwd_fused_presplit(int ng, const void* const* dout, const void* const* y, const float* const* coef,
-                                 const float* const* bcoef, float* const* dw, int B, int D, int H, int W, int cout,
-                                 float slope, void* ws, size_t ws_bytes, void* stream);
 
 /* Block-1 gradient with respect to the input image (saliency maps, integrated gradients, input-space attacks): the
  * BatchNorm + LeakyReLU + MaxPool3d(2,2) backward "apply" (dy recomputed from the stored y exactly as

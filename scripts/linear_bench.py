@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Linear-layer microbenchmark (B200): tmf_linear_fwd / dgrad / wgrad at the fusion transformer's shapes (M = B*150
-tokens), CUDA events over `--iters` launches.  TMF_GEMM_IMPL=0 selects the generic gemm_kernel for comparison.
+tokens), CUDA events over `--iters` launches.  Every shape here runs gemm_ksplit_kernel; the generic gemm_kernel only
+takes shapes with an extent that is not a multiple of 4.
 
     python scripts/linear_bench.py [--iters 50] [--batch 8]
 """

@@ -10,7 +10,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "transmf_ad_b200", "libtmf_sm100a.so")
 COLS = [("UTC*MMA", r"UTC[A-Z]*MMA"), ("LDTM", r"LDTM"), ("UTMALDG", r"UTMALDG"), ("UBLKCP", r"UBLKCP"), ("UTCBAR", r"UTCBAR"),
         ("SYNCS", r"SYNCS"), ("HMMA", r"HMMA"), ("LDSM", r"LDSM"), ("LDGSTS", r"LDGSTS"), ("FFMA2/FADD2", r"F(FMA|ADD|MUL)2"),
-        ("HMNMX2/HSET2", r"(HMNMX2|HSET2)"), ("ACQBULK/PREEXIT", r"(ACQBULK|PREEXIT)"),
+        ("HMNMX2/HSET2", r"(HMNMX2|HSET2)"),
         ("float atomics", r"(ATOM|RED)[A-Z.]*\.(F32|F64|ADD\.F)"), ("int atomics (global)", r"(ATOMG|REDG|ATOM\.|RED\.)")]
 
 
@@ -37,8 +37,7 @@ def main():
           "cp.async.bulk (conv1.0 image windows), `UTCBAR` = tcgen05.commit, `SYNCS` = mbarrier operations; `HMMA` = legacy mma.sync (the 16-row "
           "token-panel GEMMs of the fused transformer encoder and the tensor-core attention kernels: bf16 hi/lo split products -- DESIGN.md "
           "sections 10.4 / 10.10 for why not tcgen05 there), `LDSM` = ldmatrix, `LDGSTS` = cp.async, `FFMA2/FADD2` = packed fp32 pairs, "
-          "`HMNMX2/HSET2` = packed bf16 max / compare (max-pool backward), `ACQBULK/PREEXIT` = griddepcontrol.wait / launch_dependents "
-          "(programmatic dependent launch entry of every train-step kernel; only active with TMF_PDL=1).\n")
+          "`HMNMX2/HSET2` = packed bf16 max / compare (max-pool backward).\n")
     print("Floating-point atomics: only the CUDA-core bring-up kernels (`conv_direct.cu`).  Integer atomics: last-block tickets and the Adam "
           "step ticket.\n")
     print("| kernel | " + " | ".join(c[0] for c in COLS) + " |")

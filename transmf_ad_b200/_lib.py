@@ -26,8 +26,6 @@ SIGNATURES = {
     "tmf_conv1_fwd": [_i, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _vp],
     "tmf_conv1_wgrad": [_i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _vp, C.c_size_t, _vp],
     "tmf_conv1_bwd_fused": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp, C.c_size_t, _vp],
-    "tmf_conv1_bwd_split_x": [_i, _pp, _i, _i, _i, _i, _i, _vp, C.c_size_t, _vp],
-    "tmf_conv1_bwd_fused_presplit": [_i, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp, C.c_size_t, _vp],
     "tmf_conv1_dgrad_fused": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _i, _vp, C.c_size_t, _vp],
     "tmf_conv3d_fwd": [_i, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _i, _i, _vp],
     "tmf_conv3d_wgrad": [_i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, C.c_size_t, _vp],
@@ -86,7 +84,7 @@ SIGNATURES = {
     "tmf_adam_step": [_vp, _i, _vp, _f, _f, _f, _f, _vp, _vp, _vp],
 }
 PLAIN = {"tmf_last_error": (C.c_char_p, []), "tmf_version": (_i, []), "tmf_check_device": (_i, []), "tmf_stat_rows": (_i, []), "tmf_scratch_bytes": (_i64, []), "tmf_encoder_supported": (_i, [_i, _i, _i]), "tmf_encoder_pack_bytes": (C.c_size_t, [_i]),
-         "tmf_launch_count": (_i64, []), "tmf_set_pdl": (_i, [_i]), "tmf_attn_impl_default": (_i, []), "tmf_get_pdl": (_i, []), "tmf_conv3d_supported": (_i, [_i] * 8),
+         "tmf_launch_count": (_i64, []), "tmf_attn_impl_default": (_i, []), "tmf_conv3d_supported": (_i, [_i] * 8),
          "tmf_conv3d_wgrad_workspace_bytes": (_i64, [_i] * 9),
          "tmf_conv3d_umma_plan_info": (_i, [_i] * 8 + [C.POINTER(C.c_int)]),
          "tmf_conv3d_col_plan_info": (_i, [_i] * 7 + [C.POINTER(C.c_int)]),

@@ -43,7 +43,6 @@ __device__ __forceinline__ void emit_pack(const AdamChunk& c, int i, float val) 
 __global__ void __launch_bounds__(256) adam_multi_kernel(const AdamChunk* __restrict__ chunks, const float* __restrict__ lr_dev,
                                                          float b1, float b2, float eps, float wd, float* step_dev,
                                                          unsigned* ticket) {
-  pdl_entry();
   const AdamChunk c = chunks[blockIdx.x];
   const float t = step_dev[0] + 1.f;              // step_dev is only advanced after every block has read it (ticket below)
   const float lr = lr_dev[0];

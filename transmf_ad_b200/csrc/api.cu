@@ -2,7 +2,6 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -20,21 +19,6 @@ void set_error(const char* fmt, ...) {
 
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
 
-// TMF_PDL=1 turns programmatic dependent launch on (read once; tmf_set_pdl() overrides it, e.g. for A/B timing).  Off by
-// default: measured on B200 inside the captured step it is worth 0.6 % (4.679 -> 4.649 ms) and the encoder chain alone got
-// SLOWER (186 -> 194 us per encoder): graph replays already start dependent kernels within ~1 us.
-static std::atomic<int> g_pdl{-1};
-bool pdl_enabled() {
-  int v = g_pdl.load(std::memory_order_relaxed);
-  if (v < 0) {
-    const char* e = getenv("TMF_PDL");
-    v = (e != nullptr && atoi(e) != 0) ? 1 : 0;
-    g_pdl.store(v, std::memory_order_relaxed);
-  }
-  return v != 0;
-}
-void set_pdl(int on) { g_pdl.store(on ? 1 : 0, std::memory_order_relaxed); }
-
 }  // namespace tmf
 
 extern "C" {
@@ -44,10 +28,6 @@ const char* tmf_last_error(void) { return tmf::g_err; }
 int tmf_version(void) { return 200; }
 
 int tmf_stat_rows(void) { return TMF_STAT_ROWS; }
-
-int tmf_set_pdl(int on) { tmf::set_pdl(on); return 0; }
-
-int tmf_get_pdl(void) { return tmf::pdl_enabled() ? 1 : 0; }
 
 int64_t tmf_launch_count(void) { return tmf::g_launches.load(std::memory_order_relaxed); }
 

@@ -64,7 +64,6 @@ __device__ __forceinline__ void stage_rows_t(float* dst, const float* src, int64
 // ---------------------------------------------------------------------------------------------------------------
 template <int NPL>
 __global__ void __launch_bounds__(TA_THREADS) attn_tiled_fwd_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   constexpr int Np = 32 * NPL;
   const int dh = p.dh, ld = dh + 1, inner = p.heads * dh;
@@ -146,7 +145,6 @@ __global__ void __launch_bounds__(TA_THREADS) attn_tiled_fwd_kernel(AttnArgs p) 
 // ---------------------------------------------------------------------------------------------------------------
 template <int NPL>
 __global__ void __launch_bounds__(TA_THREADS) attn_tiled_dq_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   constexpr int Np = 32 * NPL;
   const int dh = p.dh, ld = dh + 1, inner = p.heads * dh;
@@ -227,7 +225,6 @@ __global__ void __launch_bounds__(TA_THREADS) attn_tiled_dq_kernel(AttnArgs p) {
 // ---------------------------------------------------------------------------------------------------------------
 template <int NPL>
 __global__ void __launch_bounds__(TA_THREADS) attn_tiled_dkv_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   constexpr int Np = 32 * NPL;
   const int dh = p.dh, ld = dh + 1, inner = p.heads * dh;

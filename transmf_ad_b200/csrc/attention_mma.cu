@@ -173,7 +173,6 @@ __device__ __forceinline__ float quad_sum(float v) {
 // =====================================================================================================================
 template <int DH>
 __global__ void __launch_bounds__(AM_THREADS) attn_mma_fwd_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) uint8_t smraw[];
   using L = Lay<DH>;
   uint8_t* Kh = smraw;
@@ -260,7 +259,6 @@ __global__ void __launch_bounds__(AM_THREADS) attn_mma_fwd_kernel(AttnArgs p) {
 // =====================================================================================================================
 template <int DH>
 __global__ void __launch_bounds__(AM_THREADS) attn_mma_bwd_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) uint8_t smraw[];
   using L = Lay<DH>;
   const int inner = p.heads * DH;
@@ -446,7 +444,6 @@ struct ScoreArgs {
 
 template <int DH>
 __global__ void __launch_bounds__(AM_THREADS) attn_scores_kernel(ScoreArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) uint8_t smraw[];
   using L = Lay<DH>;
   const int inner = p.heads * DH;
@@ -521,7 +518,6 @@ constexpr int RV_COLS = 32, RV_SLICES = 8;
 __global__ void __launch_bounds__(RV_COLS * RV_SLICES) attn_relevance_kernel(const float* __restrict__ attn,
                                                                            const float* __restrict__ dattn, float* M, float* r,
                                                                            int heads, int Nq, int Nk, int accumulate) {
-  pdl_entry();
   __shared__ float part[RV_SLICES][RV_COLS];
   const int b = blockIdx.y, cx = threadIdx.x % RV_COLS, sl = threadIdx.x / RV_COLS;
   const int j = blockIdx.x * RV_COLS + cx;

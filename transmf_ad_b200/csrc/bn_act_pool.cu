@@ -46,7 +46,6 @@ __global__ void __launch_bounds__(32 * FIN_WARPS) bn_finalize_kernel(GroupPtr<co
                                    GroupPtr<const float> beta, GroupPtr<float> rmean, GroupPtr<float> rvar,
                                    GroupPtr<int64_t> nbt, GroupPtr<float> coef, int C, double count, float momentum,
                                    float eps, int training) {
-  pdl_entry();
   const int g = blockIdx.z;
   double t1, t2;
   sum_stat_rows(stats.p[g], C, training != 0, t1, t2);
@@ -81,7 +80,6 @@ __global__ void __launch_bounds__(32 * FIN_WARPS) bn_finalize_kernel(GroupPtr<co
 __global__ void __launch_bounds__(32 * FIN_WARPS) bn_bwd_finalize_kernel(GroupPtr<const double> sums, GroupPtr<const float> coef, GroupPtr<float> dgamma,
                                        GroupPtr<float> dbeta, GroupPtr<float> dbias, GroupPtr<float> bcoef, int C,
                                        double count, int training) {
-  pdl_entry();
   const int g = blockIdx.z;
   double s1, s2;
   sum_stat_rows(sums.p[g], C, true, s1, s2);
@@ -146,7 +144,6 @@ __device__ __forceinline__ void store8f(void* base, int64_t elem_off, int fp32, 
 // DUAL: also store the fp32 value o in out32 (same layout as out); out (bf16) and ymax are the same bits as without it.
 template <bool KEEP, bool DUAL = false>
 __global__ void __launch_bounds__(256, DUAL ? 2 : (KEEP ? 3 : 4)) bn_act_pool_fwd_kernel(ActPoolArgs p) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int CQ = p.C >> 3;
   const __nv_bfloat16* yg = p.y.p[g];
@@ -258,7 +255,6 @@ __device__ __forceinline__ void block_channel_sums(float* red, double* rows, int
 //    A = scale*(m2*invstd*mean - m1),  Bc = -scale*m2*invstd.
 template <bool APPLY, int POOL>
 __global__ void __launch_bounds__(256, (POOL == TMF_POOL_NONE) ? 3 : 2) bn_act_pool_bwd_kernel(ActPoolArgs p) {
-  pdl_entry();
   const int g = blockIdx.z;
   extern __shared__ float red[];  // [16][256] (REDUCE only)
   const int CQ = p.C >> 3;
@@ -395,7 +391,6 @@ __global__ void __launch_bounds__(256, (POOL == TMF_POOL_NONE) ? 3 : 2) bn_act_p
 constexpr int RK_U = 4;
 template <bool FP32>
 __global__ void __launch_bounds__(256, 2) bn_maxpool_bwd_reduce_kept_kernel(ActPoolArgs p, int npos) {
-  pdl_entry();
   const int g = blockIdx.z;
   extern __shared__ float red[];  // [16][256]
   const int CQ = p.C >> 3;
@@ -473,7 +468,6 @@ __device__ __forceinline__ uint32_t u4_get(const uint4& v, int i) { return i == 
 
 template <bool FP32>
 __global__ void __launch_bounds__(256, 2) bn_maxpool_bwd_apply_kernel(ActPoolArgs p) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int CQ = p.C >> 3;
   const __nv_bfloat16* yg = p.y.p[g];

@@ -69,14 +69,8 @@ static inline bool load_group(GroupPtr<T>& g, T* const* host, int ng, bool requi
 
 static inline int ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
-// Programmatic dependent launch (sm_90+): every kernel of the train step begins with pdl_entry() -- wait until the kernels
-// before it in the stream have completed and their writes are visible, then let the NEXT kernel's blocks be scheduled as
-// soon as SM resources free up -- and is launched through launch_k() with the programmatic-serialisation attribute, so the
-// launch latency, block scheduling and grid ramp-up of kernel i+1 overlap kernel i (the step is ~280 short launches).
-// Nothing is read or written before the wait, so the ordering guarantees are those of a plain in-order stream; in a
-// captured CUDA graph the edges become programmatic dependencies.  OFF by default (TMF_PDL=1 / tmf_set_pdl(1) turn it on):
-// measured gain inside the captured step 0.6 %, see api.cu; without the attribute the wait is a no-op.
-bool pdl_enabled();
+// The single launch helper of the library: a plain cudaLaunchKernelEx with the arguments converted to the kernel's
+// parameter types.
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                                    Args&&... args) {
@@ -85,16 +79,7 @@ static inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 blo
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-__device__ __forceinline__ void pdl_entry() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 }
 
 // Zero one `bytes`-sized buffer per group; adjacent buffers (callers that carve the towers' buffers out of one

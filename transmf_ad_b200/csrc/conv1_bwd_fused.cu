@@ -50,7 +50,6 @@ struct alignas(64) C1BParams {
 // fp32 image (B*D*H rows of W) -> six bf16 rows of pitch P per image row: x6[row][hl*3+kw][k] = hl-part of x[k+kw-1]
 // (zero outside [0,W)); hl = 0: bf16(x), hl = 1: bf16(x - bf16(x)).
 __global__ void conv1_split_x_kernel(GroupPtr<const float> x, GroupPtr<__nv_bfloat16> x6, int rows, int W, int P) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int chunks = P >> 3;
   const unsigned total = (unsigned)rows * (unsigned)chunks;
@@ -75,7 +74,6 @@ __global__ void conv1_split_x_kernel(GroupPtr<const float> x, GroupPtr<__nv_bflo
 }
 
 __global__ void __launch_bounds__(C1B_THREADS, 1) conv1_bwd_fused_kernel(const __grid_constant__ C1BParams p) {
-  pdl_entry();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -314,7 +312,6 @@ __global__ void __launch_bounds__(C1B_THREADS, 1) conv1_bwd_fused_kernel(const _
 
 // dw[co][tap] = sum over CTAs of part[cta][co*27+tap], fixed order
 __global__ void conv1_bwd_reduce_kernel(GroupPtr<const float> part, GroupPtr<float> dw, int ncta) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 32 * 27) return;
@@ -348,7 +345,7 @@ struct C1BPlan {
 static C1BPlan c1b_plan(int ng, int B, int D, int H, int W, int cout) {
   C1BPlan pl{};
   pl.ok = false;
-  if (getenv("TMF_DISABLE_UMMA") != nullptr || getenv("TMF_DISABLE_CONV1_BWD_FUSED") != nullptr) return pl;
+  if (getenv("TMF_DISABLE_UMMA") != nullptr) return pl;
   if (cout != 32 || ng < 1 || ng > TMF_MAX_GROUPS) return pl;
   if (D < 2 || H < 2 || W < 2 || W > 240) return pl;
   if ((long long)B * D * H * ((W + 15) / 8) >= (1ll << 31)) return pl;
@@ -390,10 +387,6 @@ static C1BPlan c1b_plan(int ng, int B, int D, int H, int W, int cout) {
 
 using namespace tmf;
 
-static int conv1_bwd_fused_impl(int ng, const void* const* dout, const void* const* y, const float* const* coef,
-                               const float* const* bcoef, const float* const* x, float* const* dw, int B, int D, int H, int W,
-                               int cout, float slope, void* ws, size_t ws_bytes, void* stream, int mode);
-
 extern "C" {
 
 int64_t tmf_conv1_bwd_fused_workspace_bytes(int ng, int B, int D, int H, int W, int cout) {
@@ -404,29 +397,6 @@ int64_t tmf_conv1_bwd_fused_workspace_bytes(int ng, int B, int D, int H, int W, 
 int tmf_conv1_bwd_fused(int ng, const void* const* dout, const void* const* y, const float* const* coef,
                         const float* const* bcoef, const float* const* x, float* const* dw, int B, int D, int H, int W,
                         int cout, float slope, void* ws, size_t ws_bytes, void* stream) {
-  return conv1_bwd_fused_impl(ng, dout, y, coef, bcoef, x, dw, B, D, H, W, cout, slope, ws, ws_bytes, stream, 0);
-}
-
-// The bf16 hi/lo split of the input image (145 MB written per step at B = 8, 42 us) depends on x alone: callers that know x
-// early (the forward pass) run it ahead of time on another stream with tmf_conv1_bwd_split_x() and then call
-// tmf_conv1_bwd_fused_presplit() with the SAME workspace, which skips the split.
-int tmf_conv1_bwd_split_x(int ng, const float* const* x, int B, int D, int H, int W, int cout, void* ws, size_t ws_bytes,
-                          void* stream) {
-  return conv1_bwd_fused_impl(ng, nullptr, nullptr, nullptr, nullptr, x, nullptr, B, D, H, W, cout, 0.f, ws, ws_bytes, stream, 1);
-}
-
-int tmf_conv1_bwd_fused_presplit(int ng, const void* const* dout, const void* const* y, const float* const* coef,
-                                 const float* const* bcoef, float* const* dw, int B, int D, int H, int W, int cout,
-                                 float slope, void* ws, size_t ws_bytes, void* stream) {
-  return conv1_bwd_fused_impl(ng, dout, y, coef, bcoef, nullptr, dw, B, D, H, W, cout, slope, ws, ws_bytes, stream, 2);
-}
-
-}  // extern "C"
-
-// mode 0: split + fused pass, 1: split only, 2: fused pass on an already split image
-static int conv1_bwd_fused_impl(int ng, const void* const* dout, const void* const* y, const float* const* coef,
-                               const float* const* bcoef, const float* const* x, float* const* dw, int B, int D, int H, int W,
-                               int cout, float slope, void* ws, size_t ws_bytes, void* stream, int mode) {
   TMF_CHECK_NG(ng);
   const C1BPlan pl = c1b_plan(ng, B, D, H, W, cout);
   TMF_REQUIRE(pl.ok, "conv1_bwd_fused: unsupported problem (Cout=%d, %dx%dx%d); use bn_act_pool_bwd_apply + conv1_wgrad",
@@ -452,13 +422,12 @@ static int conv1_bwd_fused_impl(int ng, const void* const* dout, const void* con
   GroupPtr<__nv_bfloat16> gx6;
   GroupPtr<const float> gpart;
   GroupPtr<float> gdw;
-  if (!load_group(gx, x, ng, mode != 2, "x") || !load_group(gdw, dw, ng, mode != 1, "dw")) return 1;
+  if (!load_group(gx, x, ng, true, "x") || !load_group(gdw, dw, ng, true, "dw")) return 1;
   const int Do = D / 2, Ho = H / 2, Wo = W / 2;
   for (int g = 0; g < TMF_MAX_GROUPS; ++g) gx6.p[g] = nullptr;
   for (int g = 0; g < ng; ++g) {
     uint8_t* base = (uint8_t*)ws + (size_t)g * (xbytes + pbytes);
     gx6.p[g] = (__nv_bfloat16*)base;
-    if (mode == 1) continue;
     TMF_REQUIRE(dout[g] && y[g] && coef[g] && bcoef[g], "conv1_bwd_fused: NULL device pointer");
     TMF_REQUIRE(((uintptr_t)dout[g] & 15) == 0 && ((uintptr_t)y[g] & 15) == 0, "conv1_bwd_fused: tensors must be 16-byte aligned");
     p.part[g] = (float*)(base + xbytes);
@@ -495,16 +464,12 @@ static int conv1_bwd_fused_impl(int ng, const void* const* dout, const void* con
       TMF_REQUIRE(r == CUDA_SUCCESS, "conv1_bwd_fused: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
     }
   }
-  if (mode != 2) {
-    const int rows = B * D * H;
-    const long long total = (long long)rows * (pl.P / 8);
-    // at most ~4 blocks (1024 threads) per SM in all: run ahead of time on a side stream (mode 1) the kernel must leave thread
-    // slots to the kernels of the main stream
-    dim3 grid((unsigned)min((long long)(148 * 4 / ng), (total + 255) / 256), 1, ng);
-    launch_k(conv1_split_x_kernel, grid, 256, 0, st, gx, gx6, rows, W, pl.P);
-    TMF_LAUNCH_CHECK();
-  }
-  if (mode == 1) return 0;
+  const int rows = B * D * H;
+  const long long total = (long long)rows * (pl.P / 8);
+  // grid-stride loop over at most ~4 blocks (1024 threads) per SM, shared by the towers
+  dim3 grid((unsigned)min((long long)(148 * 4 / ng), (total + 255) / 256), 1, ng);
+  launch_k(conv1_split_x_kernel, grid, 256, 0, st, gx, gx6, rows, W, pl.P);
+  TMF_LAUNCH_CHECK();
   static bool attr_done = false;
   if (!attr_done) {
     TMF_CUDA(cudaFuncSetAttribute(conv1_bwd_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -516,3 +481,5 @@ static int conv1_bwd_fused_impl(int ng, const void* const* dout, const void* con
   TMF_LAUNCH_CHECK();
   return 0;
 }
+
+}  // extern "C"

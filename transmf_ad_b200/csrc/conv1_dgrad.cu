@@ -74,7 +74,6 @@ __device__ __forceinline__ uint32_t c1d_get(const uint4& v, int i) { return i ==
 // front (s = a1 * c1 / stab(z) at each window's first maximum of y, zero elsewhere) and an epilogue that writes x * (W^T s).
 template <bool LRP>
 __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const __grid_constant__ C1DParams p) {
-  pdl_entry();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (sbase - smem_u32(smem_raw));
@@ -374,7 +373,6 @@ __global__ void __launch_bounds__(C1D_THREADS, 1) conv1_dgrad_umma_kernel(const 
 // (fp32 weights, fixed summation order).  Serves TMF_CONV_DIRECT and the problems the tcgen05 kernel refuses.
 __global__ void __launch_bounds__(256) conv1_dgrad_direct_kernel(GroupPtr<const __nv_bfloat16> dy, GroupPtr<const float> w,
                                                                  GroupPtr<float> dx, int B, int D, int H, int W, int cout) {
-  pdl_entry();
   __shared__ float ws[27 * 64];
   const int g = blockIdx.z;
   for (int i = threadIdx.x; i < 27 * cout; i += blockDim.x) ws[(i % 27) * cout + i / 27] = w.p[g][i];   // [tap][co]

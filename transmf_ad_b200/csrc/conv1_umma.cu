@@ -67,7 +67,6 @@ __device__ __forceinline__ void split_bf16(float v, float& hi, float& lo) {
 // !STAGED keeps the direct loads for images whose base address is not 16-byte aligned or whose rows are too wide.
 template <int NCH, bool STAGED>
 __global__ void __launch_bounds__(C1U_THREADS, 1) conv1_umma_fwd_kernel(const __grid_constant__ C1UParams p) {
-  pdl_entry();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -459,7 +458,6 @@ struct alignas(64) C1WParams {
 };
 
 __global__ void __launch_bounds__(C1W_U_THREADS, 1) conv1_umma_wgrad_kernel(const __grid_constant__ C1WParams p) {
-  pdl_entry();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -610,7 +608,6 @@ __global__ void __launch_bounds__(C1W_U_THREADS, 1) conv1_umma_wgrad_kernel(cons
 }
 
 __global__ void conv1_wgrad_reduce_kernel(GroupPtr<const float> part, GroupPtr<float> dw, int ncta, int n) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -624,7 +621,7 @@ __global__ void conv1_wgrad_reduce_kernel(GroupPtr<const float> part, GroupPtr<f
 using namespace tmf;
 
 bool tmf_conv1_fwd_umma_supported(int cout) {
-  if (getenv("TMF_DISABLE_UMMA") != nullptr || getenv("TMF_DISABLE_UMMA_CONV1") != nullptr) return false;
+  if (getenv("TMF_DISABLE_UMMA") != nullptr) return false;
   return cout == 32 || cout == 64;
 }
 
@@ -685,7 +682,7 @@ int tmf_conv1_fwd_umma(int ng, const float* const* x, const float* const* w, con
 
 
 bool tmf_conv1_wgrad_umma_supported(int W, int cout) {
-  if (getenv("TMF_DISABLE_UMMA") != nullptr || getenv("TMF_DISABLE_UMMA_CONV1") != nullptr) return false;
+  if (getenv("TMF_DISABLE_UMMA") != nullptr) return false;
   return cout == 32 && W + 2 <= 256;
 }
 

@@ -27,7 +27,7 @@ using namespace umma;
 constexpr int UC_TILE_M = 128;
 constexpr int UC_MAX_BSTAGES = 27 * 4;
 constexpr int UC_MAX_ASTAGES = 4;
-constexpr int UC_TMA_LANES = 4;  // producer lanes issuing TMA boxes round-robin (TMF_UMMA_TMA_LANES=1..8: bring-up switch)
+constexpr int UC_TMA_LANES = 4;  // producer lanes issuing TMA boxes round-robin
 constexpr uint32_t UC_SMEM_BUDGET = 227 * 1024;
 
 struct alignas(64) UmmaConvParams {
@@ -45,7 +45,6 @@ struct alignas(64) UmmaConvParams {
   uint32_t a_stage_bytes, b_stage_bytes, a_tx_bytes, b_tx_bytes;
   uint32_t idesc;
   uint32_t tmem_cols;
-  int bo_mode;                    // how the descriptor base-offset field is derived (bring-up switch)
   int tma_lanes;                  // producer lanes that issue TMA boxes round-robin
   int mt;                         // 128-row M tiles per weight pass ("super-tile" = 128*mt consecutive positions)
   int nbuf;                       // accumulator sets in TMEM: 2 = epilogue overlaps the next super-tile, 1 = it does not
@@ -61,18 +60,11 @@ struct alignas(64) UmmaConvParams {
   int kwf;
 };
 
-__device__ __forceinline__ uint32_t desc_base_offset(uint32_t saddr, int mode) {
-  if (mode == 1) return (saddr >> 7) & 7u;
-  if (mode == 2) return (saddr >> 7) & 3u;
-  return 0u;
-}
-
 // NISS = 2 (streamed weights, 4*Cout <= 512 TMEM columns): a narrow-N tcgen05.mma (N = 64: ~54 tensor-pipe cycles) is
 // bound by the ~100 cycles its issuing thread needs, so two issuer warps take alternate taps of the weight ring (ring
 // stage s always belongs to issuer s % 2: SB is even), each into its own TMEM accumulator; the epilogue adds the two.
 template <int KSTEPS, int KS, bool RES, int NISS>
 __global__ void __launch_bounds__(32 * (5 + NISS), 1) conv3d_umma_kernel(const __grid_constant__ UmmaConvParams p) {
-  pdl_entry();
   static_assert(NISS == 1 || !RES, "two issuers only with the streamed weight ring");
   constexpr int NTHREADS = 32 * (5 + NISS);
   constexpr int EPI0 = 32 * (1 + NISS);             // first epilogue thread
@@ -392,15 +384,6 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-static int umma_issuers() {
-  static int n = -1;
-  if (n < 0) {
-    const char* e = getenv("TMF_UMMA_ISSUERS");      // bring-up switch: 1 = single issuer warp everywhere
-    n = e ? atoi(e) : 2;
-  }
-  return n;
-}
-
 struct UmmaPlan {
   bool ok;
   int Wp, NH, QT, nchunk, chunk, row_bytes, SA, SB, b_resident, niss, mt, nbuf;
@@ -463,20 +446,18 @@ static UmmaPlan make_plan(int D, int H, int W, int cin, int cout, int ks, int B 
     //   a CTA walks whole super-tiles, so the total is ceil(B*D*QT / CTAs per tower) rounds of (cost per plane / QT):
     //   big super-tiles lose to wave quantisation on the small layers (conv4.0 fwd: 88 super-tiles on 74 CTAs).
     pl.b_resident = 0;
-    const int force_mt = umma_env_int("TMF_UMMA_MT", 0);             // bring-up switches
     const int want_kwf = umma_env_int("TMF_UMMA_KWF", -1);           // kw-fused weight boxes: 0 = never, 1 = whenever possible
     const int max_kwf = (ks == 3 && want_kwf != 0 && ((uint32_t)cout * pl.row_bytes) % 1024u == 0) ? 1 : 0;
-    const int max_iss = (ks == 3) ? umma_issuers() : 1;
+    const int max_iss = (ks == 3) ? 2 : 1;
     double best = 1e30;
     UmmaPlan bp = pl;
     bool found = false;
     for (int mt = 1; mt <= 4; ++mt) {
-      if (force_mt > 0 && mt != force_mt) continue;
       if (ks != 3 && mt > 1) break;
       // kw-fused boxes on per-plane tiles only on request: measured on B200 (conv3.3 dgrad, B = 8) the plan they allow
       // (mt = 2, two issuers, 24 KB stages) runs 128.9 us against 121.3 us for mt = 3 with single-tap stages
       for (int kwf = 0; kwf <= (want_kwf == 1 ? max_kwf : 0); ++kwf)
-      for (int niss = 1; niss <= (max_iss >= 2 ? 2 : 1); ++niss)
+      for (int niss = 1; niss <= max_iss; ++niss)
         for (int nbuf = 2; nbuf >= 1; --nbuf) {
           if (nbuf * niss * mt * cout > 512) continue;
           UmmaPlan c = pl;
@@ -510,9 +491,9 @@ static UmmaPlan make_plan(int D, int H, int W, int cin, int cout, int ks, int B 
     // Plane-stack candidates (see UmmaConvParams): tiles of 128 consecutive positions of the whole sample, one box of NP
     // padded planes per (kd, chunk); same cost model per tile, rounds = ceil(B * tiles per sample / CTAs per tower).
     const int want_stack = umma_env_int("TMF_UMMA_STACK", -1);       // bring-up switch: 0 = never, 1 = whenever possible
-    if (ks == 3 && want_stack != 0 && force_mt == 0) {
+    if (ks == 3 && want_stack != 0) {
       for (int kwf = 0; kwf <= max_kwf; ++kwf)
-      for (int niss = 1; niss <= (max_iss >= 2 ? 2 : 1); ++niss)
+      for (int niss = 1; niss <= max_iss; ++niss)
         for (int nbuf = 2; nbuf >= 1; --nbuf) {
           if (nbuf * niss * cout > 512) continue;
           UmmaPlan c = pl;
@@ -560,26 +541,6 @@ static UmmaPlan make_plan(int D, int H, int W, int cin, int cout, int ks, int B 
   return pl;
 }
 
-static int umma_bo_mode() {
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("TMF_UMMA_BO");
-    mode = e ? atoi(e) : 0;   // hardware swizzles on absolute smem address bits: verified on B200 (scripts/umma_bringup.py)
-  }
-  return mode;
-}
-
-static int umma_tma_lanes() {
-  static int lanes = -1;
-  if (lanes < 0) {
-    const char* e = getenv("TMF_UMMA_TMA_LANES");
-    lanes = e ? atoi(e) : UC_TMA_LANES;
-    if (lanes < 1) lanes = 1;
-    if (lanes > 8) lanes = 8;
-  }
-  return lanes;
-}
-
 }  // namespace tmf
 
 using namespace tmf;
@@ -620,8 +581,7 @@ int tmf_conv3d_fwd_umma(int ng, const void* const* a, const void* const* wf, con
   p.a_stage_bytes = pl.a_stage_bytes; p.b_stage_bytes = pl.b_stage_bytes; p.a_tx_bytes = pl.a_tx; p.b_tx_bytes = pl.b_tx;
   p.idesc = make_idesc_bf16(UC_TILE_M, cout, 0, 0);
   p.tmem_cols = pl.tmem_cols;
-  p.bo_mode = umma_bo_mode();
-  p.tma_lanes = umma_tma_lanes();
+  p.tma_lanes = UC_TMA_LANES;
   p.mt = pl.mt;
   p.nbuf = pl.nbuf;
   const int taps = ksize * ksize * ksize;

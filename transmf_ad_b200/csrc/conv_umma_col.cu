@@ -95,7 +95,6 @@ template <bool NS> struct ColRoles {
 };
 template <int KSTEPS, bool NS>
 __global__ void __launch_bounds__(ColRoles<NS>::THREADS, 1) conv3d_umma_col_kernel(const __grid_constant__ ColConvParams p) {
-  pdl_entry();
   constexpr int MMA_WARPS = ColRoles<NS>::MMA_WARPS, FIRST_EPI = ColRoles<NS>::FIRST_EPI;
   constexpr uint32_t PITCH = KSTEPS * 32u;          // bytes per smem row (= Cin * 2)
   constexpr uint32_t ROW_UNITS = PITCH >> 4;
@@ -567,7 +566,7 @@ extern "C" int tmf_conv3d_col_plan_info(int ng, int D, int H, int W, int cin, in
 }
 
 bool tmf_conv3d_fwd_col_supported(int ng, int D, int H, int W, int cin, int cout, int ksize) {
-  if (getenv("TMF_DISABLE_UMMA") != nullptr || getenv("TMF_DISABLE_COL") != nullptr) return false;
+  if (getenv("TMF_DISABLE_UMMA") != nullptr) return false;
   return make_col_plan(ng, D, H, W, cin, cout, ksize).ok;
 }
 

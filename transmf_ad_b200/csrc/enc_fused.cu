@@ -428,7 +428,6 @@ struct PackArgs {
   __nv_bfloat16* pack;
 };
 __global__ void __launch_bounds__(256) enc_pack_kernel(PackArgs p) {
-  pdl_entry();
   const int m = blockIdx.y;
   const float4* src = reinterpret_cast<const float4*>(p.w[m]);
   uint2* hi = reinterpret_cast<uint2*>(p.pack + p.off[m]);
@@ -558,7 +557,6 @@ struct ProjFwdArgs {
 };
 
 __global__ void __launch_bounds__(THREADS) enc_proj_fwd_kernel(ProjFwdArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   float* P0 = sm;                           // [16][132] input panel
   float* P1 = P0 + PR * LD128;              // [16][260] output panel
@@ -599,7 +597,6 @@ struct ChainFwdArgs {
 
 template <int MLP>
 __global__ void __launch_bounds__(THREADS) enc_chain_fwd_kernel(ChainFwdArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   constexpr int ldf = MLP + 4;
   float* P0 = sm;                           // o, later g
@@ -678,7 +675,6 @@ struct ChainBwdArgs {
 
 template <int MLP>
 __global__ void __launch_bounds__(THREADS) enc_chain_bwd_kernel(ChainBwdArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   constexpr int ldf = MLP + 4;
   float* P0 = sm;
@@ -753,7 +749,6 @@ struct ProjBwdArgs {
 };
 
 __global__ void __launch_bounds__(THREADS) enc_proj_bwd_kernel(ProjBwdArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   float* P0 = sm;                           // [16][260]
   float* P1 = P0 + PR * 260;                // [16][132]
@@ -821,7 +816,6 @@ struct WgradArgs {
 };
 
 __global__ void __launch_bounds__(THREADS) enc_wgrad_kernel(WgradArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float sm[];
   float* At = sm;                           // [32][WG_LDA]: dY^T chunk
   float* wst = At + 32 * WG_LDA;

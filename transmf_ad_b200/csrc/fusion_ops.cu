@@ -47,7 +47,6 @@ __device__ __forceinline__ float gelu_exact(float x) { return 0.5f * x * (1.f + 
 // These GEMMs are tiny (M = B*150 rows, K, N <= 512): what matters is latency, so the global loads of tile k+1 are
 // issued before the FMAs of tile k (register double buffering), and long-K problems are split over blockIdx.z.
 __global__ void __launch_bounds__(256) gemm_kernel(GemmArgs p) {
-  pdl_entry();
   __shared__ __align__(16) float As[G_TK][G_TM + G_PAD];
   __shared__ __align__(16) float Bs[G_TK][G_TN + G_PAD];
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
@@ -123,7 +122,6 @@ __global__ void __launch_bounds__(256) gemm_kernel(GemmArgs p) {
 // block of a column group adds them in index order (deterministic; no atomics, nothing to zero).
 __global__ void colsum_kernel(const float* __restrict__ x, float* __restrict__ out, int M, int N, int rows_per_block,
                               float* __restrict__ partbuf, unsigned* __restrict__ tickets) {
-  pdl_entry();
   __shared__ float part[8][33];
   const int n = blockIdx.x * 32 + (threadIdx.x & 31);
   const int r = threadIdx.x >> 5;
@@ -158,7 +156,6 @@ __global__ void __launch_bounds__(256)
 layernorm_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
                      const float* __restrict__ residual, float* __restrict__ y, float* __restrict__ mean_out,
                      float* __restrict__ rstd_out, int rows, int dim, float eps) {
-  pdl_entry();
   const int lane = threadIdx.x & 31;
   const int nv = dim >> 2;
   for (int row = blockIdx.x * 8 + (threadIdx.x >> 5); row < rows; row += gridDim.x * 8) {
@@ -207,7 +204,6 @@ layernorm_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, 
                      const float* __restrict__ mean, const float* __restrict__ rstd, float* __restrict__ dx,
                      float* __restrict__ dgamma, float* __restrict__ dbeta, int rows, int dim, int accumulate,
                      float* __restrict__ partbuf, unsigned* __restrict__ ticket) {
-  pdl_entry();
   extern __shared__ float sm[];  // [2][dim]
   for (int i = threadIdx.x; i < 2 * dim; i += blockDim.x) sm[i] = 0.f;
   __syncthreads();
@@ -283,7 +279,6 @@ layernorm_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x, 
 // ------------------------------------------------------------------------------------------------------------
 __global__ void gelu_bwd_kernel(const float4* __restrict__ dy, const float4* __restrict__ pre, float4* __restrict__ dx,
                                 int64_t n4) {
-  pdl_entry();
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
     const float4 g = dy[i], x = pre[i];
     float4 o;
@@ -302,7 +297,6 @@ __global__ void gelu_bwd_kernel(const float4* __restrict__ dy, const float4* __r
 
 __global__ void scale_kernel(const float* __restrict__ x, float* __restrict__ y, float alpha,
                              const float* __restrict__ alpha_dev, int64_t n) {
-  pdl_entry();
   if (alpha_dev != nullptr) alpha *= alpha_dev[0];
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     y[i] = alpha * x[i];
@@ -316,7 +310,6 @@ constexpr int AT_ROWS = 32;  // rows per block
 
 // smem: Ks[Nk][dh+1], Vs[Nk][dh+1], sc[AT_WARPS][Nk], qs[AT_WARPS][dh]
 __global__ void __launch_bounds__(AT_WARPS * 32) attn_fwd_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ float sm[];
   const int dh = p.dh, ld = dh + 1, inner = p.heads * dh;
   float* Ks = sm;
@@ -367,7 +360,6 @@ __global__ void __launch_bounds__(AT_WARPS * 32) attn_fwd_kernel(AttnArgs p) {
 
 // dq: same staging as forward.  extra smem: dos[AT_WARPS][dh]
 __global__ void __launch_bounds__(AT_WARPS * 32) attn_bwd_dq_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ float sm[];
   const int dh = p.dh, ld = dh + 1, inner = p.heads * dh;
   float* Ks = sm;
@@ -418,7 +410,6 @@ __global__ void __launch_bounds__(AT_WARPS * 32) attn_bwd_dq_kernel(AttnArgs p) 
 
 // dk, dv: smem Qs[Nq][dh+1], dOs[Nq][dh+1], lses[Nq], Ds[Nq], pw[AT_WARPS][Nq], dsw[AT_WARPS][Nq], ks/vs[AT_WARPS][dh]
 __global__ void __launch_bounds__(AT_WARPS * 32) attn_bwd_dkv_kernel(AttnArgs p) {
-  pdl_entry();
   extern __shared__ float sm[];
   const int dh = p.dh, ld = dh + 1, inner = p.heads * dh;
   float* Qs = sm;
@@ -488,7 +479,6 @@ constexpr int TP_WARPS = 8;
 __global__ void __launch_bounds__(32 * TP_WARPS) token_pool_fwd_kernel(const float* __restrict__ x, float* __restrict__ mean,
                                                                       float* __restrict__ mx, int32_t* __restrict__ amax, int B,
                                                                       int N, int C) {
-  pdl_entry();
   __shared__ float ssum[TP_WARPS][32], sbest[TP_WARPS][32];
   __shared__ int sidx[TP_WARPS][32];
   const int cblocks = (C + 31) / 32;
@@ -527,7 +517,6 @@ __global__ void __launch_bounds__(32 * TP_WARPS) token_pool_fwd_kernel(const flo
 __global__ void token_pool_bwd_kernel(const float* __restrict__ dmean, const float* __restrict__ dmax,
                                       const int32_t* __restrict__ amax, float* __restrict__ dx, int B, int N, int C,
                                       int accumulate) {
-  pdl_entry();
   const int64_t total = (int64_t)B * N * C;
   const float invn = 1.f / N;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -544,22 +533,20 @@ __global__ void token_pool_bwd_kernel(const float* __restrict__ dmean, const flo
 
 
 // ------------------------------------------------------------------------------------------------------------
-// Pipelined variant for the shapes the fusion transformer actually runs (every extent a multiple of 4, 16-byte
-// aligned rows): 32 x 64 output tile, 128 threads (4 x 4 outputs each), K in 32-wide slices moved global -> shared
-// with 16-byte cp.async through a 3-deep ring, so the loads of two slices are in flight while one is multiplied
-// (gemm_kernel exposes one global-load latency per 16-wide slice: ~1 us x K/16, i.e. 8-30 us for these GEMMs whose
-// arithmetic is ~1 us).  Smaller tiles also put M = B*150 = 1200 rows on 76-304 CTAs instead of 38-152.
+// Linear GEMM for the shapes the fusion transformer actually runs (every extent a multiple of 4, 16-byte aligned
+// rows), built for latency.  32 x 32 output tile, 256 threads = 4 K-GROUPS of 64 threads.  A "super-slice" is four
+// 32-wide K slices; it moves global -> shared with 16-byte cp.async into one of two buffers, so the loads of the next
+// super-slice are in flight while one is multiplied (gemm_kernel exposes one global-load latency per 16-wide slice:
+// ~1 us x K/16, i.e. 8-30 us for these GEMMs whose arithmetic is ~1 us).  Group g
+// multiplies slice g of every super-slice into its own 4 x 4 register tiles, and the four partial tiles meet in shared
+// memory at the end.  Per thread a K = 128 GEMM is 512 FMAs instead of 2048 for one thread per 4 x 4 outputs over the
+// whole of K, and M = 1200, N = 128 is 152 CTAs of 8 warps -- these GEMMs are bound by the serial FMA chain of a thread
+// plus one load latency, not by throughput.
 //   AKF / BKF: the operand is contiguous along k in global memory (x and w of the forward pass; dy of dgrad).  It is
-//   kept as [row][k] in shared memory and read four k at a time; rows are interleaved over the threads (row = t +
-//   8*i or t + 16*j) so that the 144-byte row pitch spreads a quarter-warp over all 32 banks.  Otherwise the operand
-//   is contiguous along m / n (w of dgrad, dy and x of wgrad), kept as [k][m|n] and read as one float4 per k.
+//   kept as [row][k] in shared memory and read four k at a time; rows are interleaved over the threads (row = t + 8*i)
+//   so that the 144-byte row pitch spreads a quarter-warp over all 32 banks.  Otherwise the operand is contiguous along
+//   m / n (w of dgrad, dy and x of wgrad), kept as [k][m|n] and read as one float4 per k.
 // ------------------------------------------------------------------------------------------------------------
-constexpr int F_TM = 32, F_TN = 64, F_TK = 32, F_STAGES = 3, F_THREADS = 128;
-constexpr int F_KPITCH = F_TK + 4;                 // [row][k] tiles
-constexpr int F_A_FLOATS = (F_TM * F_KPITCH > F_TK * (F_TM + 4)) ? F_TM * F_KPITCH : F_TK * (F_TM + 4);
-constexpr int F_B_FLOATS = (F_TN * F_KPITCH > F_TK * (F_TN + 4)) ? F_TN * F_KPITCH : F_TK * (F_TN + 4);
-constexpr int F_STAGE_FLOATS = F_A_FLOATS + F_B_FLOATS;
-
 __device__ __forceinline__ void cp_async16(float* smem_dst, const float* gsrc, bool valid) {
   const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
   const int n = valid ? 16 : 0;                    // src-size 0: the 16 bytes are zero-filled, gsrc is not read
@@ -569,144 +556,6 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-template <bool AKF, bool BKF>
-__global__ void __launch_bounds__(F_THREADS) gemm_pipe_kernel(GemmArgs p) {
-  pdl_entry();
-  extern __shared__ __align__(16) float fsm[];
-  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  const int m0 = blockIdx.y * F_TM, n0 = blockIdx.x * F_TN;
-  const int kb = p.kchunk ? blockIdx.z * p.kchunk : 0;
-  const int ke = p.kchunk ? min(p.K, kb + p.kchunk) : p.K;
-  const int nkt = (ke - kb + F_TK - 1) / F_TK;
-  const int64_t lda = AKF ? p.sAm : p.sAk, ldb = BKF ? p.sBn : p.sBk;
-
-  auto load_stage = [&](int kt) {
-    float* As = fsm + (kt % F_STAGES) * F_STAGE_FLOATS;
-    float* Bs = As + F_A_FLOATS;
-    const int k0 = kb + kt * F_TK;
-    if (AKF) {                                     // [m][k]: 32 rows x 8 chunks
-#pragma unroll
-      for (int c = tid; c < F_TM * (F_TK / 4); c += F_THREADS) {
-        const int r = c >> 3, q = c & 7;
-        const int m = m0 + r, k = k0 + 4 * q;
-        const bool ok = m < p.M && k < ke;
-        cp_async16(As + r * F_KPITCH + 4 * q, p.A + (ok ? (int64_t)m * lda + k : 0), ok);
-      }
-    } else {                                       // [k][m]: 32 rows x 8 chunks
-#pragma unroll
-      for (int c = tid; c < F_TK * (F_TM / 4); c += F_THREADS) {
-        const int r = c >> 3, q = c & 7;
-        const int k = k0 + r, m = m0 + 4 * q;
-        const bool ok = m < p.M && k < ke;
-        cp_async16(As + r * (F_TM + 4) + 4 * q, p.A + (ok ? (int64_t)k * lda + m : 0), ok);
-      }
-    }
-    if (BKF) {                                     // [n][k]: 64 rows x 8 chunks
-#pragma unroll
-      for (int c = tid; c < F_TN * (F_TK / 4); c += F_THREADS) {
-        const int r = c >> 3, q = c & 7;
-        const int n = n0 + r, k = k0 + 4 * q;
-        const bool ok = n < p.N && k < ke;
-        cp_async16(Bs + r * F_KPITCH + 4 * q, p.B + (ok ? (int64_t)n * ldb + k : 0), ok);
-      }
-    } else {                                       // [k][n]: 32 rows x 16 chunks
-#pragma unroll
-      for (int c = tid; c < F_TK * (F_TN / 4); c += F_THREADS) {
-        const int r = c >> 4, q = c & 15;
-        const int k = k0 + r, n = n0 + 4 * q;
-        const bool ok = n < p.N && k < ke;
-        cp_async16(Bs + r * (F_TN + 4) + 4 * q, p.B + (ok ? (int64_t)k * ldb + n : 0), ok);
-      }
-    }
-  };
-
-  float acc[4][4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-
-#pragma unroll
-  for (int s = 0; s < F_STAGES - 1; ++s) {
-    if (s < nkt) load_stage(s);
-    cp_async_commit();
-  }
-  for (int kt = 0; kt < nkt; ++kt) {
-    cp_async_wait<F_STAGES - 2>();                 // slice kt has landed (for this thread's copies)
-    __syncthreads();                               // ... and everybody's; slice kt-1's buffer is free again
-    if (kt + F_STAGES - 1 < nkt) load_stage(kt + F_STAGES - 1);
-    cp_async_commit();
-    const float* As = fsm + (kt % F_STAGES) * F_STAGE_FLOATS;
-    const float* Bs = As + F_A_FLOATS;
-#pragma unroll
-    for (int k4 = 0; k4 < F_TK; k4 += 4) {
-      float a[4][4], b[4][4];                      // [k][i], [k][j]
-      if (AKF) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const float4 v = *reinterpret_cast<const float4*>(As + (ty + 8 * i) * F_KPITCH + k4);
-          a[0][i] = v.x; a[1][i] = v.y; a[2][i] = v.z; a[3][i] = v.w;
-        }
-      } else {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const float4 v = *reinterpret_cast<const float4*>(As + (k4 + k) * (F_TM + 4) + ty * 4);
-          a[k][0] = v.x; a[k][1] = v.y; a[k][2] = v.z; a[k][3] = v.w;
-        }
-      }
-      if (BKF) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 v = *reinterpret_cast<const float4*>(Bs + (tx + 16 * j) * F_KPITCH + k4);
-          b[0][j] = v.x; b[1][j] = v.y; b[2][j] = v.z; b[3][j] = v.w;
-        }
-      } else {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const float4 v = *reinterpret_cast<const float4*>(Bs + (k4 + k) * (F_TN + 4) + tx * 4);
-          b[k][0] = v.x; b[k][1] = v.y; b[k][2] = v.z; b[k][3] = v.w;
-        }
-      }
-#pragma unroll
-      for (int k = 0; k < 4; ++k)
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[k][i], b[k][j], acc[i][j]);
-    }
-  }
-  cp_async_wait<0>();
-
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int m = m0 + (AKF ? ty + 8 * i : ty * 4 + i);
-    if (m >= p.M) continue;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int n = n0 + (BKF ? tx + 16 * j : tx * 4 + j);
-      if (n >= p.N) continue;
-      float v = acc[i][j];
-      const int64_t o = (int64_t)m * p.N + n;
-      if (p.kchunk) { p.part[(size_t)blockIdx.z * p.M * p.N + o] = v; continue; }
-      if (p.bias) v += __ldg(p.bias + n);
-      if (p.pre) p.pre[o] = v;
-      if (p.act == 1) v = gelu_exact(v);
-      if (p.residual) v += __ldg(p.residual + o);
-      if (p.accumulate) v += p.C[o];
-      p.C[o] = v;
-    }
-  }
-  if (p.kchunk) splitk_finish(p, m0, n0, F_TM, F_TN);
-}
-
-
-// ------------------------------------------------------------------------------------------------------------
-// Second pipelined variant, for latency: 32 x 32 output tile, 256 threads = 4 K-GROUPS of 64 threads.  A "super-slice"
-// is four 32-wide K slices; group g multiplies slice g of every super-slice into its own 4 x 4 register tiles, and
-// the four partial tiles meet in shared memory at the end.  Per thread a K = 128 GEMM is 512 FMAs instead of 2048,
-// and M = 1200, N = 128 is 152 CTAs of 8 warps instead of 76 CTAs of 4 -- these GEMMs are bound by the serial FMA
-// chain of a thread plus one load latency, not by throughput.  Operand layouts as in gemm_pipe_kernel.
-// ------------------------------------------------------------------------------------------------------------
 constexpr int V_TM = 32, V_TN = 32, V_TK = 32, V_GROUPS = 4, V_THREADS = 64 * V_GROUPS, V_BUFS = 2;
 constexpr int V_PITCH = 36;                                        // both [row][k] (32 + 4) and [k][m|n] (32 + 4) tiles
 constexpr int V_SLICE_FLOATS = 2 * 32 * V_PITCH;                   // A tile + B tile of one K slice
@@ -715,7 +564,6 @@ constexpr int V_RED_PITCH = 36;
 
 template <bool AKF, bool BKF>
 __global__ void __launch_bounds__(V_THREADS) gemm_ksplit_kernel(GemmArgs p) {
-  pdl_entry();
   extern __shared__ __align__(16) float fsm[];
   const int tid = threadIdx.x, grp = tid >> 6, t = tid & 63, tx = t & 7, ty = t >> 3;
   const int m0 = blockIdx.y * V_TM, n0 = blockIdx.x * V_TN;
@@ -843,10 +691,7 @@ __global__ void __launch_bounds__(V_THREADS) gemm_ksplit_kernel(GemmArgs p) {
   if (p.kchunk) splitk_finish(p, m0, n0, V_TM, V_TN);
 }
 
-static bool gemm_pipe_eligible(const GemmArgs& p) {
-  static int off = -1;
-  if (off < 0) off = getenv("TMF_GEMM_IMPL") != nullptr && atoi(getenv("TMF_GEMM_IMPL")) == 0;   // 0: always gemm_kernel
-  if (off) return false;
+static bool gemm_ksplit_eligible(const GemmArgs& p) {
   const bool akf = p.sAk == 1, bkf = p.sBk == 1;
   if (!akf && p.sAm != 1) return false;
   if (!bkf && p.sBn != 1) return false;
@@ -858,17 +703,8 @@ static bool gemm_pipe_eligible(const GemmArgs& p) {
   return true;
 }
 
-static int gemm_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TMF_GEMM_IMPL");       // 0: gemm_kernel, 1: gemm_pipe_kernel, 2 (default): gemm_ksplit_kernel
-    v = e ? atoi(e) : 2;
-  }
-  return v;
-}
-
 static int launch_gemm(GemmArgs& p, cudaStream_t st) {
-  if (gemm_pipe_eligible(p) && gemm_variant() >= 2) {
+  if (gemm_ksplit_eligible(p)) {
     dim3 grid(ceil_div(p.N, V_TN), ceil_div(p.M, V_TM), p.kchunk ? ceil_div(p.K, p.kchunk) : 1);
     const size_t smem = sizeof(float) * V_BUFS * V_SUPER_FLOATS;
     const bool akf = p.sAk == 1, bkf = p.sBk == 1;
@@ -886,27 +722,6 @@ static int launch_gemm(GemmArgs& p, cudaStream_t st) {
     else if (bkf) TMF_LAUNCH_KS(false, true);
     else TMF_LAUNCH_KS(false, false);
 #undef TMF_LAUNCH_KS
-    TMF_LAUNCH_CHECK();
-    return 0;
-  }
-  if (gemm_pipe_eligible(p)) {
-    dim3 grid(ceil_div(p.N, F_TN), ceil_div(p.M, F_TM), p.kchunk ? ceil_div(p.K, p.kchunk) : 1);
-    const size_t smem = sizeof(float) * F_STAGES * F_STAGE_FLOATS;
-    const bool akf = p.sAk == 1, bkf = p.sBk == 1;
-#define TMF_LAUNCH_PIPE(AK, BK)                                                                                      \
-  do {                                                                                                             \
-    static bool attr_done = false;                                                                                 \
-    if (!attr_done) {                                                                                              \
-      TMF_CUDA(cudaFuncSetAttribute(gemm_pipe_kernel<AK, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-      attr_done = true;                                                                                            \
-    }                                                                                                              \
-    launch_k(gemm_pipe_kernel<AK, BK>, grid, F_THREADS, smem, st, p);                                                     \
-  } while (0)
-    if (akf && bkf) TMF_LAUNCH_PIPE(true, true);
-    else if (akf) TMF_LAUNCH_PIPE(true, false);
-    else if (bkf) TMF_LAUNCH_PIPE(false, true);
-    else TMF_LAUNCH_PIPE(false, false);
-#undef TMF_LAUNCH_PIPE
     TMF_LAUNCH_CHECK();
     return 0;
   }
@@ -964,24 +779,15 @@ int tmf_linear_wgrad(const float* dy, const float* x, float* dw, float* dbias, i
   cudaStream_t st = (cudaStream_t)stream;
   if (M > 2 * G_SPLIT_K) {             // long reduction over the tokens: split it, partial sums meet in a zeroed dw
     p.kchunk = G_SPLIT_K;
-    if (gemm_pipe_eligible(p)) {       // enough K slices to put ~one CTA on every SM, in whole 32-wide slices
-      if (gemm_variant() >= 2) {       // whole super-slices (4 x 32 tokens) per CTA
-        const int tiles = ceil_div(N, V_TM) * ceil_div(K, V_TN), ss = V_GROUPS * V_TK;
-        int splits = ceil_div(2 * 148, tiles);
-        if (splits > ceil_div(M, ss)) splits = ceil_div(M, ss);
-        p.kchunk = ceil_div(ceil_div(M, splits), ss) * ss;
-      } else {
-        const int tiles = ceil_div(N, F_TM) * ceil_div(K, F_TN);
-        int splits = ceil_div(148, tiles);
-        if (splits > ceil_div(M, F_TK)) splits = ceil_div(M, F_TK);
-        p.kchunk = ceil_div(ceil_div(M, splits), F_TK) * F_TK;
-      }
+    if (gemm_ksplit_eligible(p)) {     // enough K slices to put ~two CTAs on every SM, in whole super-slices (4 x 32 tokens)
+      const int tiles = ceil_div(N, V_TM) * ceil_div(K, V_TN), ss = V_GROUPS * V_TK;
+      int splits = ceil_div(2 * 148, tiles);
+      if (splits > ceil_div(M, ss)) splits = ceil_div(M, ss);
+      p.kchunk = ceil_div(ceil_div(M, splits), ss) * ss;
     }
     // split-K partial tiles meet in the scratch buffer; the last split of a tile adds them in order (deterministic)
     const int splits = ceil_div(M, p.kchunk);
-    const int tiles = gemm_pipe_eligible(p) ? (gemm_variant() >= 2 ? ceil_div(N, V_TM) * ceil_div(K, V_TN)
-                                                                    : ceil_div(N, F_TM) * ceil_div(K, F_TN))
-                                            : ceil_div(N, G_TM) * ceil_div(K, G_TN);
+    const int tiles = gemm_ksplit_eligible(p) ? ceil_div(N, V_TM) * ceil_div(K, V_TN) : ceil_div(N, G_TM) * ceil_div(K, G_TN);
     if (tiles > 2048 || (size_t)splits * N * K > part_floats) {
       p.kchunk = 0;                      // too large for the scratch buffer: one CTA per tile walks the whole reduction
     } else {

@@ -14,7 +14,6 @@ namespace tmf {
 // ---- bf16 <-> fp32 ---------------------------------------------------------------------------------------------------
 template <bool WIDEN>
 __global__ void __launch_bounds__(256) convert_kernel(GroupPtr<const void> src, GroupPtr<void> dst, int64_t n8) {
-  pdl_entry();
   const int g = blockIdx.z;
   for (int64_t i = blockIdx.x * 256ll + threadIdx.x; i < n8; i += (int64_t)gridDim.x * 256) {
     if (WIDEN) {
@@ -88,7 +87,6 @@ struct CamArgs {
 // Partial column sums of G over one chunk of positions of one sample: thread (k, cq) adds positions k, k+pstep, ... of the
 // chunk for channels 4cq..4cq+3 in double; the block then adds its pstep rows in index order.
 __global__ void __launch_bounds__(CAM_THREADS) cam_alpha_kernel(CamArgs a) {
-  pdl_entry();
   __shared__ double red[CAM_THREADS * 4];
   const int g = blockIdx.z, b = blockIdx.y, chunk = blockIdx.x;
   const int cq = threadIdx.x % a.CQ, k = threadIdx.x / a.CQ;
@@ -125,7 +123,6 @@ __global__ void __launch_bounds__(CAM_THREADS) cam_alpha_kernel(CamArgs a) {
 // the loads are issued together instead of as one dependent chain per channel.
 constexpr int CAM_STAGE = 4096;                                     // doubles per staging pass
 __global__ void __launch_bounds__(CAM_THREADS) cam_alpha_final_kernel(CamArgs a) {
-  pdl_entry();
   extern __shared__ double sm[];                                    // [CAM_STAGE] staging + [C] totals
   double* acc = sm + CAM_STAGE;
   const int g = blockIdx.z, b = blockIdx.y;
@@ -167,7 +164,6 @@ __device__ __forceinline__ void block_minmax(float mn, float mx, float* dst) {
 // stores this block's minimum / maximum.
 template <bool MINMAX>
 __global__ void __launch_bounds__(CAM_THREADS) cam_map_kernel(CamArgs a) {
-  pdl_entry();
   extern __shared__ double alpha[];
   const int g = blockIdx.z, b = blockIdx.y;
   for (int c = threadIdx.x; c < a.C; c += CAM_THREADS) alpha[c] = a.alpha[((int64_t)g * a.B + b) * a.C + c];
@@ -244,7 +240,6 @@ __device__ __forceinline__ float cam_value(const CamArgs& a, const float* lo, in
 // sample's minimum / maximum over all partial rows when `normalize` (min / max are exact: the order does not matter).
 template <bool UPS, bool WRITE>
 __global__ void __launch_bounds__(CAM_THREADS) cam_resample_kernel(CamArgs a, int normalize) {
-  pdl_entry();
   const int g = blockIdx.z, b = blockIdx.y;
   const float* lo = UPS ? a.lo + ((int64_t)g * a.B + b) * a.P : a.out.p[g] + (int64_t)b * a.P;
   float* out = a.out.p[g] + (int64_t)b * a.nout;

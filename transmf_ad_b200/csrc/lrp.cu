@@ -79,7 +79,6 @@ __device__ __forceinline__ float lrp_block_sum(float v, float* red) {
 
 // One thread per cell (pool window, 8 channels).  Voxels outside every complete window (odd extents) get s = 0.
 __global__ void __launch_bounds__(LRP_THREADS) lrp_ratio_kernel(const __grid_constant__ LrpRatioParams p) {
-  pdl_entry();
   __shared__ float red[LRP_THREADS];
   const int g = blockIdx.z, n = blockIdx.y;
   const int win = p.pool == TMF_POOL_NONE ? 1 : 2;
@@ -198,7 +197,6 @@ __global__ void __launch_bounds__(LRP_THREADS) lrp_ratio_kernel(const __grid_con
 // out = x * c (in place on c), plus per-CTA partial sums of out: the relevance map of block 1's CUDA-core path.
 __global__ void __launch_bounds__(LRP_THREADS) lrp_xmul_kernel(GroupPtr<const float> x, GroupPtr<float> c, GroupPtr<float> part,
                                                                int64_t per, int nblk) {
-  pdl_entry();
   __shared__ float red[LRP_THREADS];
   const int g = blockIdx.z, n = blockIdx.y;
   const float* xs = x.p[g] + (int64_t)n * per;
@@ -215,7 +213,6 @@ __global__ void __launch_bounds__(LRP_THREADS) lrp_xmul_kernel(GroupPtr<const fl
 
 // totals[g][n][col + k] = sum over r (in index order, fp64) of part[g][n][r][k]
 __global__ void lrp_sum_rows_kernel(GroupPtr<const float> part, GroupPtr<float> totals, int B, int rows, int K, int col) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * K) return;
@@ -227,7 +224,6 @@ __global__ void lrp_sum_rows_kernel(GroupPtr<const float> part, GroupPtr<float> 
 }
 
 __global__ void __launch_bounds__(1024) lrp_normalize_kernel(GroupPtr<float> map, int64_t per) {
-  pdl_entry();
   __shared__ float red[32];
   const int g = blockIdx.z, n = blockIdx.y;
   float* m = map.p[g] + (int64_t)n * per;

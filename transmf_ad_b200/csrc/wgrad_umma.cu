@@ -58,7 +58,6 @@ struct alignas(64) WgradParams {
 
 template <int KSTEPS>
 __global__ void __launch_bounds__(WG_THREADS, 1) conv3d_wgrad_umma_kernel(const __grid_constant__ WgradParams p) {
-  pdl_entry();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t bars = smem_base + (uint32_t)p.stages * p.stage_bytes;
@@ -198,7 +197,6 @@ __global__ void __launch_bounds__(WG_THREADS, 1) conv3d_wgrad_umma_kernel(const 
 // dw[co][ci][tap] = sum_split ws[split][tap][ci][co]   (fixed order -> deterministic)
 __global__ void wgrad_reduce_kernel(GroupPtr<const float> ws, GroupPtr<float> dw, int nsplit, int taps, int cin,
                                     int cout) {
-  pdl_entry();
   const int g = blockIdx.z;
   const int64_t total = (int64_t)taps * cin * cout;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -388,7 +386,7 @@ int tmf_wgrad_reduce(int ng, float* const* ws, float* const* dw, int nsplit, int
 }
 
 bool tmf_conv3d_wgrad_umma_supported(int D, int H, int W, int cin, int cout, int ksize) {
-  if (getenv("TMF_DISABLE_UMMA") != nullptr || getenv("TMF_DISABLE_UMMA_WGRAD") != nullptr) return false;
+  if (getenv("TMF_DISABLE_UMMA") != nullptr) return false;
   WgradParams p{};
   uint32_t smem;
   CUtensorMapSwizzle a, b;

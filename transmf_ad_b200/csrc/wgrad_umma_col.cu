@@ -43,7 +43,6 @@ struct alignas(64) WgColParams {
 };
 
 __global__ void __launch_bounds__(WC_THREADS, 1) conv3d_wgrad_col_kernel(const __grid_constant__ WgColParams p) {
-  pdl_entry();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t smX = smem_base;
@@ -276,8 +275,7 @@ static WcPlan make_wc_plan(int ng, int D, int H, int W, int cin, int cout, int k
 using namespace tmf;
 
 bool tmf_conv3d_wgrad_col_supported(int ng, int D, int H, int W, int cin, int cout, int ksize) {
-  if (getenv("TMF_DISABLE_UMMA") != nullptr || getenv("TMF_DISABLE_UMMA_WGRAD") != nullptr || getenv("TMF_DISABLE_COL") != nullptr)
-    return false;
+  if (getenv("TMF_DISABLE_UMMA") != nullptr) return false;
   return make_wc_plan(ng, D, H, W, cin, cout, ksize).ok;
 }
 

@@ -242,8 +242,6 @@ class SNetFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, spec, run, buffers, ng, *args):
-        if not isinstance(run, SNetRun):
-            run = SNetRun(bool(run), True)
         training = run.training
         seg = spec if isinstance(spec, SNetSegment) else None
         if seg is not None:
@@ -345,31 +343,6 @@ class SNetFunction(torch.autograd.Function):
                 saved.append((act, y, coef, wd, dims, ymax))
             act = out
             dims = (Do, Ho, Wo)
-        # The fused block-1 backward (conv1_bwd_fused.cu) reads the input image as six bf16 hi/lo planes.  That split depends
-        # on x alone: it is launched HERE, behind the last forward launch of the towers, on a side stream (a parallel branch of a
-        # captured graph), so that it runs beside the fusion transformer / heads / the small deep layers of the backward pass,
-        # which leave most of the GPU idle -- instead of in front of the backward kernel (145 MB written, 42 us at B = 8).
-        # (Launched at the START of the forward pass it ran beside conv1.0 forward and cost that kernel what it saved.)
-        # OFF by default (TMF_C1B_PRESPLIT=1): measured on B200 over 60 graph replays the step is 4.304 ms with the early split
-        # and 4.295 ms without -- the parallel branch costs the kernels it overlaps what it saves the backward pass.
-        ctx.c1split = None
-        cout0, pool0 = spec.layers[0][1], spec.layers[0][3]
-        if (need_wgrad and l0 == 0 and pool0 == L.POOL_MAX and impl != L.CONV_DIRECT and len(spec.layers) > 1
-                and os.environ.get("TMF_C1B_PRESPLIT", "0") != "0"):
-            nws0 = int(L.load().tmf_conv1_bwd_fused_workspace_bytes(ng, B, D, H, W, cout0))
-            if nws0 > 0:
-                ws0 = torch.empty(nws0, dtype=torch.uint8, device=dev)
-                cur = torch.cuda.current_stream(dev)
-                side = _side_stream(dev)
-                side.wait_stream(cur)
-                with torch.cuda.stream(side):
-                    L.call("tmf_conv1_bwd_split_x", ng, L.ptrs(xs), B, D, H, W, cout0, L.ptr(ws0), nws0)
-                    ev = torch.cuda.Event()
-                    ev.record(side)
-                ws0.record_stream(side)
-                for x in xs:
-                    x.record_stream(side)
-                ctx.c1split = (ws0, nws0, ev)
         ctx.spec, ctx.training, ctx.ng, ctx.saved, ctx.B = spec, training, ng, saved, B
         ctx.hyper = run.hyper
         ctx.sync_group, ctx.sync_world = run.sync_group, sync_world
@@ -525,16 +498,9 @@ class SNetFunction(torch.autograd.Function):
                 fused_ws = int(L.load().tmf_conv1_bwd_fused_workspace_bytes(ng, B, Dl, Hl, Wl, cout))
             if fused_ws > 0:
                 # block 1: BN/LeakyReLU/MaxPool backward "apply" + conv1.0 weight gradient in one pass; dy stays on chip
-                if ctx.c1split is not None and ctx.c1split[1] == fused_ws:
-                    ws, _, ev = ctx.c1split
-                    torch.cuda.current_stream(dev).wait_event(ev)        # the image split launched by the forward pass
-                    L.call("tmf_conv1_bwd_fused_presplit", ng, L.ptrs(dout), L.ptrs(y), L.ptrs(coef), L.ptrs(bcoef),
-                           L.ptrs(dw), B, Dl, Hl, Wl, cout, slope, L.ptr(ws), fused_ws, tag="tmf_conv1_bwd_fused")
-                    ctx.c1split = None
-                else:
-                    ws = torch.empty(fused_ws, dtype=torch.uint8, device=dev)
-                    L.call("tmf_conv1_bwd_fused", ng, L.ptrs(dout), L.ptrs(y), L.ptrs(coef), L.ptrs(bcoef), L.ptrs(act),
-                           L.ptrs(dw), B, Dl, Hl, Wl, cout, slope, L.ptr(ws), fused_ws)
+                ws = torch.empty(fused_ws, dtype=torch.uint8, device=dev)
+                L.call("tmf_conv1_bwd_fused", ng, L.ptrs(dout), L.ptrs(y), L.ptrs(coef), L.ptrs(bcoef), L.ptrs(act),
+                       L.ptrs(dw), B, Dl, Hl, Wl, cout, slope, L.ptr(ws), fused_ws)
                 SNetFunction._layer_grads(ctx, pgrads, l, dw, dbias, dgamma, dbeta)
                 saved[l - l0] = None
                 continue
@@ -964,23 +930,20 @@ class EncoderFunction(torch.autograd.Function):
             # out of the input-gradient kernels anyway
             return (dx.reshape(x3.shape), dctx.reshape(c3.shape)) + (None,) * 22
         table = (ctypes_ptr_array([dq, h1, d_wq, dkv, c3, d_wkv, da, o, d_wo, d_bo, dp, h2, d_w1, d_b1, dg]))
-        if os.environ.get("TMF_ENC_SIDE", "1") != "0":
-            # all five weight gradients feed nothing downstream in this backward pass: off the critical path
-            cur = torch.cuda.current_stream(dev)
-            side = _side_stream(dev)
-            side.wait_stream(cur)
-            with torch.cuda.stream(side):
-                ws2, nws2 = L.scratch(dev)                   # the side stream's own scratch buffer
-                L.call("tmf_encoder_wgrad", table, L.ptr(f), L.ptr(d_w2), L.ptr(d_b2), Mx, Mc, mlp, L.ptr(ws2), nws2)
-                ev = torch.cuda.Event()
-                ev.record(side)
-            for t in (dq, h1, dkv, c3, da, o, dp, h2, dg, f, d_wq, d_wkv, d_wo, d_bo, d_w1, d_b1, d_w2, d_b2):
-                t.record_stream(side)
-            if not _SIDE_PENDING:
-                torch.autograd.Variable._execution_engine.queue_callback(join_side_streams)
-            _SIDE_PENDING.append(ev)
-        else:
-            L.call("tmf_encoder_wgrad", table, L.ptr(f), L.ptr(d_w2), L.ptr(d_b2), Mx, Mc, mlp, L.ptr(ws), nws)
+        # all five weight gradients feed nothing downstream in this backward pass: off the critical path
+        cur = torch.cuda.current_stream(dev)
+        side = _side_stream(dev)
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            ws2, nws2 = L.scratch(dev)                       # the side stream's own scratch buffer
+            L.call("tmf_encoder_wgrad", table, L.ptr(f), L.ptr(d_w2), L.ptr(d_b2), Mx, Mc, mlp, L.ptr(ws2), nws2)
+            ev = torch.cuda.Event()
+            ev.record(side)
+        for t in (dq, h1, dkv, c3, da, o, dp, h2, dg, f, d_wq, d_wkv, d_wo, d_bo, d_w1, d_b1, d_w2, d_b2):
+            t.record_stream(side)
+        if not _SIDE_PENDING:
+            torch.autograd.Variable._execution_engine.queue_callback(join_side_streams)
+        _SIDE_PENDING.append(ev)
         return (dx.reshape(x3.shape), dctx.reshape(c3.shape), None, None, None, None, None, None, None, None,
                 d_ln1_w, d_ln1_b, d_wq, d_wkv, d_wo, d_bo, d_ln2_w, d_ln2_b, d_w1, d_b1, d_w2, d_b2, d_lnf_w, d_lnf_b)
 
