@@ -340,6 +340,27 @@ int tmf_lrp_conv1(int ng, const void* const* a1, const void* const* c1, const vo
                   int W, int cout, float eps, int impl, void* ws, size_t ws_bytes, void* stream);
 int tmf_lrp_normalize(int ng, float* const* map, int B, int64_t per, void* stream);
 
+/* ---- integrated gradients through the sNet towers, block 1 factored out of the path integral (DESIGN section 3.10) -----
+ * Zero baseline, path points alpha_k > 0.  umax: bf16 [B][Do][Ho][Wo][C] per tower, the bias-free folded conv1.0 output u'
+ * at the first maximum of each 2x2x2 window (tmf_bn_act_pool_fwd_keepmax's ymax with identity coefficients and slope 1);
+ * bias: the folded conv1.0 bias b', fp32 [C]; alpha / w: device fp32 tables of the chunk's n path points and weights; per =
+ * Do*Ho*Wo*C elements per sample; z_k = fmaf(alpha_k, umax, b') in both kernels; slope >= 0; C a multiple of 8; 16-byte
+ * aligned tensors.  Every element is written once, no atomics (bitwise reproducible; a tower's bits do not depend on ng).
+ * tmf_ig_expand: a1[k*B + b] = LeakyReLU(z_k), step-major [n*B][Do][Ho][Wo][C], bf16 (round to nearest) and its fp32 twin
+ * a1_32 (the value whose rounding is a1, as the dual-output passes write it).
+ * tmf_ig_combine: G[b] += w_k * grad[k*B + b] * LeakyReLU'(z_k) (1 where z_k > 0, else slope), k = 0 .. n-1 in order onto
+ * the loaded G, so any split of the path into chunks gives the same bits.  grad: fp32 [n*B][Do][Ho][Wo][C] step-major (the
+ * gradients at the block-1 output); G fp32 [B][Do][Ho][Wo][C], updated in place.
+ * tmf_ig_attribute: dx[g][b] *= x[g][b] in place (per elements per sample, fp32) and sums[g] fp32 [B][8], column 0 = the
+ * per-sample sum of the products (per-CTA partial rows added in index order); ws of tmf_ig_attribute_workspace_bytes. */
+int tmf_ig_expand(int ng, const void* const* umax, const float* const* bias, const float* alpha, int n, void* const* a1,
+                  float* const* a1_32, int B, int64_t per, int C, float slope, void* stream);
+int tmf_ig_combine(int ng, const float* const* grad, const void* const* umax, const float* const* bias, const float* alpha,
+                   const float* w, int n, float* const* G, int B, int64_t per, int C, float slope, void* stream);
+int64_t tmf_ig_attribute_workspace_bytes(int ng, int B, int64_t per);
+int tmf_ig_attribute(int ng, const float* const* x, float* const* dx, float* const* sums, int B, int64_t per, void* ws,
+                     size_t ws_bytes, void* stream);
+
 /* ---- attention maps of the fusion transformer (DESIGN section 3.8) ------------------------------------------------------
  * tmf_attn_scores: per-head product of the attention core's operands (q / kv as for tmf_attn_fwd; dh in {16, 32, 64}, any
  * Nq, Nk), written out as fp32 [B, heads, Nq, Nk]:

@@ -43,6 +43,9 @@ SIGNATURES = {
     "tmf_lrp_ratio": [_i, _pp, _pp, _i, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp, C.c_size_t, _vp],
     "tmf_lrp_conv1": [_i, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _i, _vp, C.c_size_t, _vp],
     "tmf_lrp_normalize": [_i, _pp, _i, _i64, _vp],
+    "tmf_ig_expand": [_i, _pp, _pp, _vp, _i, _pp, _pp, _i, _i64, _i, _f, _vp],
+    "tmf_ig_combine": [_i, _pp, _pp, _pp, _vp, _vp, _i, _pp, _i, _i64, _i, _f, _vp],
+    "tmf_ig_attribute": [_i, _pp, _pp, _pp, _i, _i64, _vp, C.c_size_t, _vp],
     "tmf_attn_scores": [_i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp],
     "tmf_attn_relevance": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "tmf_bn_maxpool_bwd_reduce_kept": [_i, _pp, _i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp],
@@ -91,7 +94,8 @@ PLAIN = {"tmf_last_error": (C.c_char_p, []), "tmf_version": (_i, []), "tmf_check
          "tmf_conv1_bwd_fused_workspace_bytes": (_i64, [_i] * 6), "tmf_conv1_dgrad_fused_workspace_bytes": (_i64, [_i] * 7),
          "tmf_conv1_wgrad_workspace_bytes": (_i64, [_i] * 4), "tmf_gradcam_workspace_bytes": (_i64, [_i] * 11), "tmf_map_resample_workspace_bytes": (_i64, [_i] * 9),
          "tmf_lrp_ratio_workspace_bytes": (_i64, [_i] * 7), "tmf_lrp_conv1_workspace_bytes": (_i64, [_i] * 7),
-         "tmf_lrp_conv1_impl": (_i, [_i] * 7), "tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
+         "tmf_lrp_conv1_impl": (_i, [_i] * 7), "tmf_ig_attribute_workspace_bytes": (_i64, [_i, _i, _i64]),
+         "tmf_line_conv_wgrad_workspace_bytes": (_i64, [_i, _i]), "tmf_adam_chunk_bytes": (_i, [])}
 
 _lib = None
 _device_checked = False

@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtmf_sm100a.so")
-SOURCES = ["api.cu", "conv_direct.cu", "conv_umma.cu", "conv_umma_col.cu", "wgrad_umma.cu", "wgrad_umma_col.cu", "conv1_umma.cu", "conv1_bwd_fused.cu", "conv1_dgrad.cu", "gradcam.cu", "lrp.cu", "bn_act_pool.cu", "fusion_ops.cu", "attention.cu", "attention_mma.cu", "enc_fused.cu", "eval_ops.cu", "augment.cu", "mnet_ops.cu", "adam.cu"]
+SOURCES = ["api.cu", "conv_direct.cu", "conv_umma.cu", "conv_umma_col.cu", "wgrad_umma.cu", "wgrad_umma_col.cu", "conv1_umma.cu", "conv1_bwd_fused.cu", "conv1_dgrad.cu", "gradcam.cu", "lrp.cu", "ig.cu", "bn_act_pool.cu", "fusion_ops.cu", "attention.cu", "attention_mma.cu", "enc_fused.cu", "eval_ops.cu", "augment.cu", "mnet_ops.cu", "adam.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-DTMF_BUILD", "-Xptxas", "-v"]
 

@@ -185,6 +185,19 @@ class EvalFold:
         return sig != self.sig, sig
 
 
+def refresh_eval_folds(folds, l, tensors, bn_eps):
+    """Rebuild the ``EvalFold`` of layer l of one or two towers where it is stale (one ``tmf_fold_bn_pack`` launch for the
+    group).  tensors[t] = (conv.weight, conv.bias, bn.weight, bn.bias, running_mean, running_var) of tower t."""
+    state = [fo.stale(l, list(ts)) for fo, ts in zip(folds, tensors)]
+    if any(st for st, _ in state):
+        w = tensors[0][0]
+        L.call("tmf_fold_bn_pack", len(folds), *[L.ptrs([ts[i] for ts in tensors]) for i in range(6)],
+               L.ptrs([fo.wf for fo in folds]), L.ptrs([fo.w32 for fo in folds]), L.ptrs([fo.bias for fo in folds]),
+               w.shape[0], w.shape[1], w.shape[2], float(bn_eps))
+        for fo, (_, sig) in zip(folds, state):
+            fo.sig = sig
+
+
 class SNetRun:
     """Per-call settings of the conv stack: train / eval, whether autograd is recording (``torch.is_grad_enabled()`` at
     the call site: inside ``Function.forward`` grad mode is always off), and the hyper-parameters read from the
@@ -377,16 +390,8 @@ class SNetFunction(torch.autograd.Function):
             Dl, Hl, Wl = dims
             bn_eps, _, slope = run.hyper[l]
             folds = [run.folds[t][l] for t in range(ng)]
-            state = [fo.stale(l, [P(t, l, 0), P(t, l, 1), P(t, l, 2), P(t, l, 3), buffers[t][l][0], buffers[t][l][1]])
-                     for t, fo in enumerate(folds)]
-            if any(st for st, _ in state):
-                L.call("tmf_fold_bn_pack", ng, L.ptrs([P(t, l, 0) for t in range(ng)]), L.ptrs([P(t, l, 1) for t in range(ng)]),
-                       L.ptrs([P(t, l, 2) for t in range(ng)]), L.ptrs([P(t, l, 3) for t in range(ng)]),
-                       L.ptrs([buffers[t][l][0] for t in range(ng)]), L.ptrs([buffers[t][l][1] for t in range(ng)]),
-                       L.ptrs([fo.wf for fo in folds]), L.ptrs([fo.w32 for fo in folds]), L.ptrs([fo.bias for fo in folds]),
-                       cout, cin, ks, float(bn_eps))
-                for fo, (_, sig) in zip(folds, state):
-                    fo.sig = sig
+            refresh_eval_folds(folds, l, [(P(t, l, 0), P(t, l, 1), P(t, l, 2), P(t, l, 3), buffers[t][l][0], buffers[t][l][1])
+                                          for t in range(ng)], bn_eps)
             y = [torch.empty((B, Dl, Hl, Wl, cout), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
             for t, kept in enumerate(run.keep or ()):
                 if kept is not None:
@@ -1162,3 +1167,79 @@ def lrp_normalize(maps):
         B = grp[0].shape[0]
         L.call("tmf_lrp_normalize", len(grp), L.ptrs(grp), B, grp[0].numel() // B)
     return maps
+
+
+# ==============================================================================================================
+# Integrated gradients   (csrc/ig.cu; DESIGN section 3.10)
+# ==============================================================================================================
+def ig_block1(xs, folds, tensors, bn_eps):
+    """Block 1 of one or two towers, once for a whole integrated-gradients path: the layer-0 ``EvalFold`` brought up to date
+    (``tensors`` as for ``refresh_eval_folds``), u' = W' * x without bias (bf16 [B,D,H,W,C]) and umax = u' at the first
+    maximum of each 2x2x2 window (bf16 [B,D/2,H/2,W/2,C]).  xs: fp32 contiguous (B,1,D,H,W) volumes."""
+    refresh_eval_folds(folds, 0, tensors, bn_eps)
+    ng = len(xs)
+    B, _, D, H, W = xs[0].shape
+    C = folds[0].bias.shape[0]
+    dev = xs[0].device
+    u = [torch.empty((B, D, H, W, C), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
+    zero = torch.zeros(C, dtype=torch.float32, device=dev)
+    L.call("tmf_conv1_fwd", ng, L.ptrs(xs), L.ptrs([f.w32 for f in folds]), L.ptrs([zero] * ng), L.ptrs(u), L.ptrs(None),
+           B, D, H, W, C, conv_impl())
+    umax = [torch.empty((B, D // 2, H // 2, W // 2, C), dtype=torch.bfloat16, device=dev) for _ in range(ng)]
+    pooled = [torch.empty_like(m) for m in umax]
+    # identity coefficients and slope 1: the pass pools u' itself, and ymax is u' at the first maximum
+    L.call("tmf_bn_act_pool_fwd_keepmax", ng, L.ptrs(u), L.ptrs([f.ident for f in folds]), L.ptrs(pooled), L.ptrs(umax), 0,
+           B, D, H, W, C, 1.0)
+    return u, umax
+
+
+def ig_expand(umax, bias, alpha, slope):
+    """The block-1 outputs at the path points ``alpha`` (fp32 device table of n): per tower (bf16 twin, fp32 value), both
+    [n*B, D/2, H/2, W/2, C] step-major."""
+    ng, n = len(umax), alpha.numel()
+    B, C = umax[0].shape[0], umax[0].shape[-1]
+    shape = (n * B,) + tuple(umax[0].shape[1:])
+    a16 = [torch.empty(shape, dtype=torch.bfloat16, device=umax[0].device) for _ in range(ng)]
+    a32 = [torch.empty(shape, dtype=torch.float32, device=umax[0].device) for _ in range(ng)]
+    L.call("tmf_ig_expand", ng, L.ptrs(umax), L.ptrs(bias), L.ptr(alpha), n, L.ptrs(a16), L.ptrs(a32), B,
+           umax[0].numel() // B, C, float(slope))
+    return a16, a32
+
+
+def ig_combine(grads, umax, bias, alpha, w, G, slope):
+    """G[t] += sum_k w_k * grads[t][k*B + b] * LeakyReLU'(alpha_k * umax + b'), k in order (``tmf_ig_combine``); grads: fp32
+    [n*B, D/2, H/2, W/2, C] contiguous, step-major."""
+    ng, n = len(umax), alpha.numel()
+    B, C = umax[0].shape[0], umax[0].shape[-1]
+    L.call("tmf_ig_combine", ng, L.ptrs(grads), L.ptrs(umax), L.ptrs(bias), L.ptr(alpha), L.ptr(w), n, L.ptrs(G), B,
+           umax[0].numel() // B, C, float(slope))
+
+
+def ig_input_grad(G, u, folds, impl=None):
+    """W'^T route(G): the block-1 input-gradient kernel with identity coefficients, zero bcoef and slope 1, fed bf16(G) and
+    u' -- its dz is then G at the first maximum of u' in every window.  Returns fp32 (B,1,D,H,W) per tower."""
+    ng = len(G)
+    B, D, H, W, C = u[0].shape
+    dev = G[0].device
+    g16 = [torch.empty(g.shape, dtype=torch.bfloat16, device=dev) for g in G]
+    L.call("tmf_narrow_f32", ng, L.ptrs(G), L.ptrs(g16), G[0].numel())
+    bcoef = [torch.zeros(2 * C, dtype=torch.float32, device=dev)] * ng
+    dx = [torch.empty((B, 1, D, H, W), dtype=torch.float32, device=dev) for _ in range(ng)]
+    impl = conv_impl() if impl is None else impl
+    nws = int(L.load().tmf_conv1_dgrad_fused_workspace_bytes(ng, impl, B, D, H, W, C))
+    ws = torch.empty(nws, dtype=torch.uint8, device=dev) if nws > 0 else None
+    L.call("tmf_conv1_dgrad_fused", ng, L.ptrs(g16), L.ptrs(u), L.ptrs([f.ident for f in folds]), L.ptrs(bcoef),
+           L.ptrs([f.w32 for f in folds]), L.ptrs(dx), B, D, H, W, C, 1.0, impl, L.ptr(ws), nws)
+    return dx
+
+
+def ig_attribute(xs, dx):
+    """dx[t] *= xs[t] in place (fp32 (B,1,D,H,W)); returns per tower the (B,) per-sample sums of the products."""
+    ng = len(xs)
+    B = xs[0].shape[0]
+    per = xs[0].numel() // B
+    sums = torch.empty((ng, B, 8), dtype=torch.float32, device=xs[0].device)
+    nws = int(L.load().tmf_ig_attribute_workspace_bytes(ng, B, per))
+    ws = torch.empty(nws, dtype=torch.uint8, device=xs[0].device)
+    L.call("tmf_ig_attribute", ng, L.ptrs(xs), L.ptrs(dx), L.ptrs(list(sums.unbind(0))), B, per, L.ptr(ws), nws)
+    return list(sums[:, :, 0].unbind(0))

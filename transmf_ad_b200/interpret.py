@@ -1,6 +1,6 @@
 """Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, layer-wise relevance
-propagation (Bach et al., 2015) through the towers, and head-averaged or gradient-weighted (Chefer et al., 2021)
-cross-modal attention maps of the fusion transformer.
+propagation (Bach et al., 2015) and integrated gradients (Sundararajan et al., 2017) through the towers, and head-averaged
+or gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the fusion transformer.
 
 Input gradients (saliency maps) need nothing from here: ``mri.requires_grad_(True)`` and plain autograd work on every model
 (INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c), and so do
@@ -13,7 +13,7 @@ from collections import namedtuple
 import torch
 
 from . import functional as TF
-from .models.networks import BLOCKS, CrossTransformer, CrossTransformer_MOD_AVG, sNet
+from .models.networks import BLOCKS, CrossTransformer, CrossTransformer_MOD_AVG, _has_backward_hooks, sNet
 
 
 def _target_index(target, B, device, who="grad_cam"):
@@ -255,3 +255,135 @@ def lrp(model, inputs, target, rule="epsilon", eps=1e-6, normalize=False):
     if normalize:
         TF.lrp_normalize(maps)
     return LRP(maps, totals)
+
+
+IG = namedtuple("IG", ["maps", "delta"])
+IG_METHODS = ("gausslegendre", "riemann_middle")
+
+
+def ig_path(n_steps, method="gausslegendre"):
+    """Path points and weights (alpha, w) of integrated gradients on [0, 1], float64 numpy arrays of ``n_steps``, as captum
+    places them: ``"gausslegendre"`` maps numpy's ``leggauss`` nodes t to alpha = (1 + t) / 2 with w = w_t / 2;
+    ``"riemann_middle"`` has alpha = (k + 1/2) / n and w = 1 / n.  Both put every alpha in (0, 1) and sum w to 1."""
+    import numpy as np
+    if method == "gausslegendre":
+        t, wt = np.polynomial.legendre.leggauss(n_steps)
+        return (1.0 + t) / 2.0, wt / 2.0
+    k = np.arange(n_steps, dtype=np.float64)
+    return (k + 0.5) / n_steps, np.full(n_steps, 1.0 / n_steps)
+
+
+def _is_count(v):
+    return isinstance(v, int) and not isinstance(v, bool) and v >= 1
+
+
+def integrated_gradients(model, inputs, target, n_steps=50, method="gausslegendre", internal_batch_size=None):
+    """Integrated gradients (Sundararajan et al., 2017) through every sNet tower of ``model`` (eval mode) with the zero
+    baseline, for the objective f = ``logits[b, target_b]`` of the model's first output: IG = x * sum_k w_k df/dx(alpha_k x),
+    with the path points of ``method`` (``ig_path``: ``"gausslegendre"``, captum's default, or ``"riemann_middle"``).
+    ``inputs`` and ``target`` as for ``grad_cam``; tower t takes ``inputs[t]``.  ``internal_batch_size`` counts volumes per
+    pass as captum does: max(1, internal_batch_size // B) path points go through the model together (``None``: all).
+
+    Returns ``IG(maps, delta)``: per tower, in tower order (``model.modules()``), an fp32 (B,1,D,H,W) attribution map, and
+    the fp32 (B,) convergence delta sum_towers sum_voxels maps - (f(x) - f(0)), with f(x) and f(0) from two eval forwards.
+
+    Block 1 is factored out of the path integral (DESIGN section 3.10): for alpha > 0 its output at alpha x is
+    LeakyReLU(alpha * umax + b') with the max-pool winners of u' = W' * x fixed, so conv1.0 runs once, the path points
+    start at layer 1, and the block-1 input gradient runs once on the weighted sum of the path's gradients.  That is exact
+    only for the zero baseline and alpha > 0: methods with a point at alpha = 0 (left / trapezoid Riemann sums) are
+    refused, and so are non-zero baselines -- their winners move with alpha.  For those, captum's ``IntegratedGradients``
+    works on these modules through plain autograd (INTEGRATION.md section 3b).
+
+    No parameter receives a ``.grad``, no weight-gradient kernel runs, BatchNorm buffers and the module mode are untouched
+    and ``requires_grad`` flags are restored."""
+    who = "integrated_gradients"
+    if method not in IG_METHODS:
+        raise ValueError(f"{who}: method must be one of {IG_METHODS}; got {method!r} (left / trapezoid Riemann sums put a "
+                         f"path point at alpha = 0, where every pooling window ties and block 1 cannot be factored out)")
+    if not _is_count(n_steps):
+        raise ValueError(f"{who}: n_steps must be an integer >= 1; got {n_steps!r}")
+    if internal_batch_size is not None and not _is_count(internal_batch_size):
+        raise ValueError(f"{who}: internal_batch_size must be None or an integer >= 1; got {internal_batch_size!r}")
+    towers = [m for m in model.modules() if isinstance(m, sNet)]
+    if not towers:
+        raise ValueError(f"{who}: the model has no sNet tower")
+    if any(m.training for m in model.modules()):
+        raise ValueError(f"{who}: BatchNorm is folded with its running statistics; call model.eval() first")
+    inputs = tuple(inputs) if isinstance(inputs, (tuple, list)) else (inputs,)
+    if (len(inputs) != len(towers) or not all(torch.is_tensor(x) and x.dim() == 5 and x.shape[1] == 1 for x in inputs)
+            or any(x.shape != inputs[0].shape for x in inputs)):
+        raise ValueError(f"{who}: inputs must be {len(towers)} (B,1,D,H,W) volume(s) of one shape, one per tower")
+    for t in towers:
+        if t._forward_hooks or t._forward_pre_hooks or _has_backward_hooks(t) or t.conv1._forward_hooks \
+                or t.conv1._forward_pre_hooks:
+            raise ValueError(f"{who}: hooks on an sNet tower or its conv1 block would observe volumes that are never formed "
+                             f"(the path points start at layer 1); remove them")
+        if t._hyper()[0][2] < 0:
+            raise ValueError(f"{who}: block 1's LeakyReLU slope must be >= 0 (the pooling winners must not move with alpha)")
+    B = inputs[0].shape[0]
+    idx = _target_index(target, B, inputs[0].device, who)
+    if not all(x.is_cuda for x in inputs):
+        raise ValueError(f"{who}: inputs must be CUDA tensors")
+    alpha64, w64 = ig_path(n_steps, method)
+    dev = inputs[0].device
+    alpha = torch.tensor(alpha64, dtype=torch.float32, device=dev)
+    weight = torch.tensor(w64, dtype=torch.float32, device=dev)
+    chunk = n_steps if internal_batch_size is None else max(1, internal_batch_size // B)
+    xs = [TF._f32c(x.detach()) for x in inputs]
+
+    def objective(outs, rows):
+        logits = outs[0] if isinstance(outs, (tuple, list)) else outs
+        return logits.gather(1, rows.view(-1, 1)).view(-1)
+
+    with torch.no_grad():
+        f_x = objective(model(*xs), idx)
+        f_0 = objective(model(*[torch.zeros_like(x) for x in xs]), idx)
+    groups, i = [], 0
+    while i < len(towers):
+        grp = [i]
+        if i + 1 < len(towers) and towers[i + 1]._spec.dim == towers[i]._spec.dim and towers[i + 1]._hyper() == towers[i]._hyper():
+            grp.append(i + 1)
+        groups.append(grp)
+        i += len(grp)
+    state = []
+    for grp in groups:
+        folds = [towers[t]._folds[0] for t in grp]
+        units = [towers[t]._units()[0] for t in grp]
+        tensors = [(c.weight, c.bias, bn.weight, bn.bias, bn.running_mean, bn.running_var) for c, bn in units]
+        u, umax = TF.ig_block1([xs[t] for t in grp], folds, tensors, towers[grp[0]]._hyper()[0][0])
+        G = [torch.zeros(m.shape, dtype=torch.float32, device=dev) for m in umax]
+        state.append((folds, [f.bias for f in folds], u, umax, G, towers[grp[0]]._hyper()[0][2]))
+    flags = [(p, p.requires_grad) for p in model.parameters()]
+    try:
+        for p, _ in flags:
+            p.requires_grad_(False)
+        for k0 in range(0, n_steps, chunk):
+            m = min(chunk, n_steps - k0)
+            a_k, w_k = alpha[k0:k0 + m], weight[k0:k0 + m]
+            leaves = [None] * len(towers)
+            for grp, (_, bias, _, umax, _, slope) in zip(groups, state):
+                a16, a32 = TF.ig_expand(umax, bias, a_k, slope)
+                for t, h, v in zip(grp, a16, a32):
+                    leaves[t] = v.permute(0, 4, 1, 2, 3).detach().requires_grad_(True)
+                    towers[t]._ig_src = (leaves[t], h)
+            # zero-stride stand-ins of batch m*B: the towers start from the supplied block-1 outputs and never read them
+            stand_ins = [x.as_strided((m * B,) + tuple(x.shape[1:]), (0,) * 5) for x in xs]
+            with torch.enable_grad():
+                obj = objective(model(*stand_ins), idx.repeat(m)).sum()
+                grads = torch.autograd.grad(obj, leaves, allow_unused=True)
+            for grp, (_, bias, _, umax, G, slope) in zip(groups, state):
+                g = [TF._f32c((torch.zeros_like(leaves[t]) if grads[t] is None else grads[t]).permute(0, 2, 3, 4, 1))
+                     for t in grp]
+                TF.ig_combine(g, umax, bias, a_k, w_k, G, slope)
+    finally:
+        for p, f in flags:
+            p.requires_grad_(f)
+        for t in towers:
+            t._ig_src = None
+    maps, total = [None] * len(towers), torch.zeros_like(f_x)
+    for grp, (folds, _, u, _, G, _) in zip(groups, state):
+        dx = TF.ig_input_grad(G, u, folds)
+        for t, m, s in zip(grp, dx, TF.ig_attribute([xs[t] for t in grp], dx)):
+            maps[t] = m
+            total = total + s
+    return IG(maps, total - (f_x - f_0))

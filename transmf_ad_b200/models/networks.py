@@ -50,6 +50,7 @@ class sNet(nn.Module):
         self._cam_act = None
         self._lrp_keep = None          # transmf_ad_b200.interpret.lrp: a list the folded eval forward appends (a, y) to
         self._lrp_folds = {}           # LRP rule -> 7 TF.LrpFold
+        self._ig_src = None            # transmf_ad_b200.interpret.integrated_gradients: block 1's output (fp32 leaf, bf16 twin)
 
     def _units(self):
         """[(conv, bn)] in execution order."""
@@ -184,6 +185,8 @@ def _tapped_boundaries(nets):
     for net in nets:
         if net._cam_tap is not None:
             taps.add(net._cam_tap)
+        if net._ig_src is not None:
+            taps.add(0)
         for k, name in enumerate(BLOCKS):
             blk = getattr(net, name)
             if _has_backward_hooks(blk):
@@ -220,10 +223,23 @@ def _segmented_forward(nets, xs, params, bufs, taps):
         run_nograd.grad_enabled = False
     cuts = [l1 for _, l1 in segment_plan(taps)]
     bound = {-1: list(xs)}
-    for t, net in enumerate(nets):
-        if net.conv1._forward_pre_hooks:
-            _fire_pre_hooks(net.conv1, xs[t], block=True)
-    cur, src, l0 = list(xs), None, 0
+    supplied = [net._ig_src for net in nets]
+    if any(s is not None for s in supplied):
+        # integrated gradients supplies block 1's output for every path point: the towers start at layer 1 and the
+        # volumes xs are never read
+        if any(s is None for s in supplied):
+            raise RuntimeError("a block-1 output was supplied for only one tower of a pair")
+        cur, src, l0 = [s[0] for s in supplied], [s[1] for s in supplied], BLOCK_END[0] + 1
+        bound[0] = cur
+        cuts = cuts[1:]
+        for t, net in enumerate(nets):
+            if net.conv2._forward_pre_hooks:
+                _fire_pre_hooks(net.conv2, cur[t], block=True)
+    else:
+        for t, net in enumerate(nets):
+            if net.conv1._forward_pre_hooks:
+                _fire_pre_hooks(net.conv1, xs[t], block=True)
+        cur, src, l0 = list(xs), None, 0
     for l1 in cuts:
         upstream = cam is not None and l1 <= BLOCK_END[cam] + 1
         with torch.no_grad() if upstream else contextlib.nullcontext():
