@@ -361,6 +361,26 @@ int64_t tmf_ig_attribute_workspace_bytes(int ng, int B, int64_t per);
 int tmf_ig_attribute(int ng, const float* const* x, float* const* dx, float* const* sums, int B, int64_t per, void* ws,
                      size_t ws_bytes, void* stream);
 
+/* ---- occlusion sensitivity through the sNet towers, recomputing only what each window changes (DESIGN section 3.11) ------
+ * m windows per pass, window-major rows n*B + b.  tab: device int32 [m][3][4], per window and axis (D, H, W) {crop origin, lo,
+ * hi of the changed region, origin of the previous layer's recomputed output}, in the global coordinates of the layer's input
+ * (functional.OccPlan); the planner guarantees every index it implies lies inside its tensor.  Every element written once, no
+ * atomics, 64-bit offsets.
+ * tmf_occ_input: out[g] fp32 [m*B][Dc][Hc][Wc] = x[g][b] (fp32 [B][D][H][W]) at crop origin + (x, y, z), or baseline where that
+ * voxel lies in [lo, hi) on all three axes (the window).
+ * tmf_occ_compose: out[g] [m*B][Dc][Hc][Wc][C] (bf16, or fp32 with fp32 != 0; C a multiple of 8, 16-byte aligned tensors): at
+ * global g = crop origin + (x, y, z), crop[g][n*B + b] at g - (previous output origin) (extent Dp, Hp, Wp) where g lies in
+ * [lo, hi) on all three axes, else base[g][b] at g (base [B][D][H][W][C]).  crop[g] == NULL replicates the base.
+ * tmf_occ_map: map[g] fp32 [B][D][H][W] = the mean of scores[g][b] (fp32 [B][nD][nH][nW]) over the windows i*s <= x < i*s + w
+ * (per axis, w = wD.., s = sD..) that contain the voxel, added in window order; 0 where none does. */
+int tmf_occ_input(int ng, const float* const* x, const int* tab, int m, float baseline, float* const* out, int B, int D,
+                  int H, int W, int Dc, int Hc, int Wc, void* stream);
+int tmf_occ_compose(int ng, const void* const* base, const void* const* crop, const int* tab, int m, void* const* out,
+                    int B, int D, int H, int W, int Dc, int Hc, int Wc, int Dp, int Hp, int Wp, int C, int fp32,
+                    void* stream);
+int tmf_occ_map(int ng, const float* const* scores, float* const* map, int B, int D, int H, int W, int nD, int nH, int nW,
+                int wD, int wH, int wW, int sD, int sH, int sW, void* stream);
+
 /* ---- attention maps of the fusion transformer (DESIGN section 3.8) ------------------------------------------------------
  * tmf_attn_scores: per-head product of the attention core's operands (q / kv as for tmf_attn_fwd; dh in {16, 32, 64}, any
  * Nq, Nk), written out as fp32 [B, heads, Nq, Nk]:

@@ -1243,3 +1243,196 @@ def ig_attribute(xs, dx):
     ws = torch.empty(nws, dtype=torch.uint8, device=xs[0].device)
     L.call("tmf_ig_attribute", ng, L.ptrs(xs), L.ptrs(dx), L.ptrs(list(sums.unbind(0))), B, per, L.ptr(ws), nws)
     return list(sums[:, :, 0].unbind(0))
+
+
+# ==============================================================================================================
+# Occlusion sensitivity with incremental recomputation   (csrc/occlusion.cu; DESIGN section 3.11)
+# ==============================================================================================================
+def occ_positions(E, w, s):
+    """Window starts along an axis of extent E: i*s for i = 0 .. (E - w) // s (captum's ``Occlusion``)."""
+    return list(range(0, E - w + 1, s))
+
+
+class OccPlan:
+    """Crop geometry of incremental occlusion through one sNet (host only, per axis; a window's geometry is the product of its
+    three axes' entries).
+
+    For layer l (0 .. 6) and every window: the changed region of the layer's input (layer 0: the window itself, then the
+    recomputed output of layer l-1), the recompute region R of the layer's conv output (the changed outputs -- the changed input
+    grown by the conv halo -- widened to whole 2x2x2 pooling windows at pooled layers) and the input crop, of one extent per layer
+    for all windows: it covers R plus the halo, is shifted inward at the volume faces and starts on an even index at pooled
+    layers, so that the crop's pooling grid is the global one.  Entry 7 is the tower output (the whole extent).
+
+    ``crop[l]``: (Dc, Hc, Wc) of layer l's input crop (7: the output extent); ``full[l]``: the layer's full input extent;
+    ``tab[l]``: int32 numpy [nwin, 3, 4], per window and axis (origin of the crop, lo, hi of the changed input region -- global
+    coordinates of layer l's input --, origin of layer l-1's recomputed output in those coordinates); window n = (i*nH + j)*nW + k.
+    """
+
+    def __init__(self, dims, window, stride, layers):
+        import numpy as np
+        self.dims, self.window, self.stride = tuple(dims), tuple(window), tuple(stride)
+        self.grid = tuple(len(occ_positions(E, w, s)) for E, w, s in zip(dims, window, stride))
+        axes = [self._axis(E, w, s, layers) for E, w, s in zip(dims, window, stride)]
+        self.crop = [tuple(ax[0][l] for ax in axes) for l in range(len(layers) + 1)]
+        self.full = [tuple(ax[1][l] for ax in axes) for l in range(len(layers) + 1)]
+        nD, nH, nW = self.grid
+        self.tab = []
+        for l in range(len(layers) + 1):
+            t = np.empty((nD, nH, nW, 3, 4), dtype=np.int32)
+            t[:, :, :, 0] = axes[0][2][:, l].reshape(nD, 1, 1, 4)
+            t[:, :, :, 1] = axes[1][2][:, l].reshape(1, nH, 1, 4)
+            t[:, :, :, 2] = axes[2][2][:, l].reshape(1, 1, nW, 4)
+            self.tab.append(t.reshape(nD * nH * nW, 3, 4))
+
+    @property
+    def nwin(self):
+        return self.grid[0] * self.grid[1] * self.grid[2]
+
+    @staticmethod
+    def _axis(E, w, s, layers):
+        """One axis: crop extents, full extents and the [n, 8, 4] table (crop origin, lo, hi, previous output origin)."""
+        import numpy as np
+        starts = occ_positions(E, w, s)
+        nl = len(layers)
+        ext = [E]
+        for ks, pool in layers:
+            ext.append(ext[-1] // 2 if pool != L.POOL_NONE else ext[-1])
+        # pass 1: per window and layer the changed input [a, b), the recompute region [ra, rb) and the needed input [na, nb)
+        geo = []
+        for a0 in starts:
+            a, b, rows = a0, a0 + w, []
+            for l, (ks, pool) in enumerate(layers):
+                e, h = ext[l], ks // 2
+                oa, ob = max(a - h, 0), min(b + h, e)                     # conv outputs that change
+                if pool != L.POOL_NONE:
+                    ra, rb = oa - oa % 2, min(ob + ob % 2, e - e % 2)     # whole pooling windows (floor mode drops e-1)
+                else:
+                    ra, rb = oa, ob
+                rows.append((a, b, ra, rb, max(ra - h, 0), min(rb + h, e)))
+                a, b = (ra // 2, rb // 2) if pool != L.POOL_NONE else (ra, rb)
+            rows.append((a, b))
+            geo.append(rows)
+        crop = []
+        for l, (ks, pool) in enumerate(layers):
+            e, even = ext[l], pool != L.POOL_NONE
+            c = max(r[l][5] - (r[l][4] - r[l][4] % 2 if even else r[l][4]) for r in geo)
+            if even and c < e and (e - c) % 2:
+                c += 1                           # the inward shift at the far face must keep an even origin
+            crop.append(min(c, e))
+        crop.append(ext[nl])
+        tab = np.zeros((len(starts), nl + 1, 4), dtype=np.int32)
+        for n, rows in enumerate(geo):
+            prev = 0
+            for l, (ks, pool) in enumerate(layers):
+                e, h, c = ext[l], ks // 2, crop[l]
+                a, b, ra, rb, na, nb = rows[l]
+                c0 = min(na - na % 2 if pool != L.POOL_NONE else na, e - c)
+                assert c0 >= 0 and (pool == L.POOL_NONE or c0 % 2 == 0), (l, c0)
+                assert c0 <= na and nb <= c0 + c and c0 <= a and b <= c0 + c, (l, c0, c, rows[l])
+                # a crop output within h of a crop face that is not a volume face saw zero padding instead of data
+                lo_ok, hi_ok = c0 + (h if c0 > 0 else 0), c0 + c - (h if c0 + c < e else 0)
+                assert lo_ok <= ra and rb <= hi_ok, (l, c0, c, ra, rb)
+                tab[n, l] = (c0, a, b, prev)
+                prev = c0 // 2 if pool != L.POOL_NONE else c0
+            a, b = rows[nl]
+            tab[n, nl] = (0, a, b, prev)
+            # the changed input of every layer lies inside the previous layer's recomputed output
+            for l in range(1, nl + 1):
+                ks, pool = layers[l - 1]
+                pc = crop[l - 1] // 2 if pool != L.POOL_NONE else crop[l - 1]
+                assert tab[n, l, 3] <= tab[n, l, 1] and tab[n, l, 2] <= tab[n, l, 3] + pc, (l, tab[n, l])
+        return crop, ext, tab
+
+    def out_extent(self, l, pool):
+        """Extent of layer l's recomputed (pooled) crop output."""
+        return tuple(c // 2 for c in self.crop[l]) if pool != L.POOL_NONE else self.crop[l]
+
+
+def occ_pass_limit(plan, spec, B, ng):
+    """Most windows one pass may take (rows m*B) while every crop launch stays inside its kernel's 32-bit index limits:
+    tmf_conv1_fwd rows*D*H*W < 2^31, tmf_bn_act_pool_fwd rows*D*H*W*C/8 < 2^31 and the column conv rows*NC*D < 2^30 (NC from
+    its launch plan, counted wherever the plan exists)."""
+    import ctypes
+    per = []
+    for l, (cin, cout, ks, pool) in enumerate(spec.layers):
+        Dc, Hc, Wc = plan.crop[l]
+        vox = B * Dc * Hc * Wc
+        per.append((vox * (cout // 8), 1 << 31))
+        if l == 0:
+            per.append((vox, 1 << 31))
+        else:
+            info = (ctypes.c_int * 6)()
+            if L.load().tmf_conv3d_col_plan_info(ng, Dc, Hc, Wc, cin, cout, ks, info) == 0:
+                per.append((B * info[3] * Dc, 1 << 30))
+    return max(1, min((lim - 1) // c for c, lim in per))
+
+
+def occ_input(xs, tab, m, baseline, extent):
+    """fp32 (m*B, 1, Dc, Hc, Wc) layer-0 crops per tower (``tmf_occ_input``); xs: fp32 contiguous (B,1,D,H,W)."""
+    B, _, D, H, W = xs[0].shape
+    out = [torch.empty((m * B, 1) + tuple(extent), dtype=torch.float32, device=xs[0].device) for _ in xs]
+    L.call("tmf_occ_input", len(xs), L.ptrs(xs), L.ptr(tab), m, float(baseline), L.ptrs(out), B, D, H, W, *extent)
+    return out
+
+
+def occ_compose(base, crops, tab, m, extent, out=None, tag=None):
+    """Input crops (m*B, Dc, Hc, Wc, C) per tower (``tmf_occ_compose``): base (B, D, H, W, C) contiguous, bf16 or fp32; crops:
+    the previous layer's recomputed outputs (m*B, Dp, Hp, Wp, C), or None to replicate the base; ``out``: optional contiguous
+    destinations."""
+    B, D, H, W, C = base[0].shape
+    if out is None:
+        out = [torch.empty((m * B,) + tuple(extent) + (C,), dtype=base[0].dtype, device=base[0].device) for _ in base]
+    Dp, Hp, Wp = crops[0].shape[1:4] if crops is not None else (0, 0, 0)
+    L.call("tmf_occ_compose", len(base), L.ptrs(base), L.ptrs(crops), L.ptr(tab), m, L.ptrs(out), B, D, H, W, *extent,
+           Dp, Hp, Wp, C, int(base[0].dtype == torch.float32), tag=tag)
+    return out
+
+
+def occ_layer(l, spec, hyper, folds, act, extent, impl):
+    """Layer l of the folded eval sNet on a batch of crops, as ``SNetFunction._eval_forward`` runs it: the conv on the folded
+    operands, then LeakyReLU and the pool with the identity coefficients.  act: fp32 (R,1,D,H,W) crops at layer 0, else bf16
+    (R,D,H,W,Cin); returns (R, pooled extent, Cout), fp32 at the last layer."""
+    cin, cout, ks, pool = spec.layers[l]
+    slope = hyper[l][2]
+    R = act[0].shape[0]
+    dev = act[0].device
+    y = [torch.empty((R,) + tuple(extent) + (cout,), dtype=torch.bfloat16, device=dev) for _ in act]
+    bias = [fo.bias for fo in folds]
+    if l == 0:
+        L.call("tmf_conv1_fwd", len(act), L.ptrs(act), L.ptrs([fo.w32 for fo in folds]), L.ptrs(bias), L.ptrs(y), L.ptrs(None),
+               R, *extent, cout, impl, tag="tmf_conv1_fwd@occ")
+    else:
+        L.call("tmf_conv3d_fwd", len(act), L.ptrs(act), L.ptrs([fo.wf for fo in folds]), L.ptrs(bias), L.ptrs(y), L.ptrs(None),
+               R, *extent, cin, cout, ks, impl, tag=f"tmf_conv3d_fwd@occL{l}")
+    last = l == len(spec.layers) - 1
+    Do, Ho, Wo = _pooled(*extent, pool)
+    out = [torch.empty((R, Do, Ho, Wo, cout), dtype=torch.float32 if last else torch.bfloat16, device=dev) for _ in act]
+    L.call("tmf_bn_act_pool_fwd", len(act), L.ptrs(y), L.ptrs([fo.ident for fo in folds]), L.ptrs(out), int(last), R, *extent,
+           cout, pool, slope, tag=f"tmf_bn_act_pool_fwd@occL{l}")
+    return out
+
+
+def occ_towers(spec, hyper, folds, xs, kept, base_out, plan, tabs, m, baseline, out):
+    """One pass of m windows through one or two towers of the same shape: the layer-0 crops, then per layer the conv on the
+    crops and the composition of the next layer's input crops from the recomputed region and the kept base activations;
+    the final composition writes the (m*B, d, h, w, C) fp32 tower outputs into ``out``.  folds[t]: the tower's 7 ``EvalFold``
+    (current: the base forward refreshed them); kept[t]: its 7 (input activation, y) pairs; base_out[t]: its fp32 (B,d,h,w,C)
+    output; tabs: the pass's device tables (``OccPlan.tab`` rows), one per layer and the output."""
+    impl = conv_impl()
+    act = occ_input(xs, tabs[0], m, baseline, plan.crop[0])
+    for l in range(len(spec.layers)):
+        if l > 0:
+            act = occ_compose([k[l][0] for k in kept], act, tabs[l], m, plan.crop[l], tag=f"tmf_occ_compose@L{l}")
+        act = occ_layer(l, spec, hyper, [f[l] for f in folds], act, plan.crop[l], impl)
+    return occ_compose(base_out, act, tabs[-1], m, plan.crop[-1], out=out, tag="tmf_occ_compose@out")
+
+
+def occ_map(scores, plan):
+    """Per tower, the fp32 (B,1,D,H,W) map: each voxel's mean score over the windows containing it (``tmf_occ_map``).
+    scores: fp32 contiguous (B, nD, nH, nW) per tower."""
+    B = scores[0].shape[0]
+    maps = [torch.empty((B, 1) + plan.dims, dtype=torch.float32, device=scores[0].device) for _ in scores]
+    for i in range(0, len(scores), 2):
+        L.call("tmf_occ_map", len(scores[i:i + 2]), L.ptrs(scores[i:i + 2]), L.ptrs(maps[i:i + 2]), B, *plan.dims, *plan.grid,
+               *plan.window, *plan.stride)
+    return maps

@@ -1,6 +1,7 @@
 """Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, layer-wise relevance
-propagation (Bach et al., 2015) and integrated gradients (Sundararajan et al., 2017) through the towers, and head-averaged
-or gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the fusion transformer.
+propagation (Bach et al., 2015), integrated gradients (Sundararajan et al., 2017) and occlusion sensitivity (Zeiler & Fergus,
+2014) through the towers, and head-averaged or gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the
+fusion transformer.
 
 Input gradients (saliency maps) need nothing from here: ``mri.requires_grad_(True)`` and plain autograd work on every model
 (INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c), and so do
@@ -387,3 +388,138 @@ def integrated_gradients(model, inputs, target, n_steps=50, method="gausslegendr
             maps[t] = m
             total = total + s
     return IG(maps, total - (f_x - f_0))
+
+
+Occlusion = namedtuple("Occlusion", ["maps", "scores"])
+
+
+def _triple(v, who, name):
+    v = (v,) * 3 if isinstance(v, int) and not isinstance(v, bool) else v
+    if not (isinstance(v, (tuple, list)) and len(v) == 3 and all(_is_count(e) for e in v)):
+        raise ValueError(f"{who}: {name} must be an integer >= 1 or a 3-tuple of them; got {v!r}")
+    return tuple(v)
+
+
+def occlusion(model, inputs, target, window=16, stride=8, baseline=0.0, internal_batch_size=None):
+    """Occlusion sensitivity (Zeiler & Fergus, 2014) through every sNet tower of ``model`` (eval mode), for the objective
+    f = ``logits[b, target_b]`` of the model's first output.  A box of ``window`` voxels set to ``baseline`` (a finite Python
+    scalar) slides over tower t's input ``inputs[t]`` with ``stride``, the other inputs unchanged; along an axis of extent E,
+    window i covers [i*s, i*s + w) for i = 0 .. (E - w) // s, as captum's ``Occlusion`` places them.  ``window`` and ``stride``:
+    an int or a 3-tuple.  ``inputs`` and ``target`` as for ``integrated_gradients``.  ``internal_batch_size`` counts volumes per
+    pass: max(1, internal_batch_size // B) windows of every tower go through the model together (``None``: all of them, split
+    only where a kernel's 32-bit index limit requires it).
+
+    Returns ``Occlusion(maps, scores)``, per tower in tower order (``model.modules()``): ``scores`` fp32 (B, nD, nH, nW),
+    f(x) - f(x with window (i, j, k) of that tower's input set to the baseline); ``maps`` fp32 (B,1,D,H,W), each voxel's mean
+    score over the windows that contain it (0 where none does).
+
+    The occluded towers are not run in full (DESIGN section 3.11): one eval forward keeps every layer's input activation,
+    and per window only the region the window changes is recomputed, layer by layer, on fixed-extent crops batched over the
+    windows; the composed tower outputs then go through the model's own fusion stack and heads.  No parameter receives a
+    ``.grad``, no weight-gradient kernel runs, BatchNorm buffers and the module mode are untouched and ``requires_grad``
+    flags are restored."""
+    import math
+    who = "occlusion"
+    window, stride = _triple(window, who, "window"), _triple(stride, who, "stride")
+    if isinstance(baseline, bool) or not isinstance(baseline, (int, float)) or not math.isfinite(baseline):
+        raise ValueError(f"{who}: baseline must be a finite Python scalar; got {baseline!r}")
+    if internal_batch_size is not None and not _is_count(internal_batch_size):
+        raise ValueError(f"{who}: internal_batch_size must be None or an integer >= 1; got {internal_batch_size!r}")
+    towers = [m for m in model.modules() if isinstance(m, sNet)]
+    if not towers:
+        raise ValueError(f"{who}: the model has no sNet tower")
+    if any(m.training for m in model.modules()):
+        raise ValueError(f"{who}: BatchNorm is folded with its running statistics; call model.eval() first")
+    inputs = tuple(inputs) if isinstance(inputs, (tuple, list)) else (inputs,)
+    if (len(inputs) != len(towers) or not all(torch.is_tensor(x) and x.dim() == 5 and x.shape[1] == 1 for x in inputs)
+            or any(x.shape != inputs[0].shape for x in inputs)):
+        raise ValueError(f"{who}: inputs must be {len(towers)} (B,1,D,H,W) volume(s) of one shape, one per tower")
+    for t in towers:
+        for mod in [t] + [getattr(t, name) for name in BLOCKS]:
+            if mod._forward_hooks or mod._forward_pre_hooks or _has_backward_hooks(mod):
+                raise ValueError(f"{who}: hooks on an sNet tower or its blocks would observe tensors that are never formed "
+                                 f"(the occluded towers run on crops); remove them")
+    B, dims = inputs[0].shape[0], tuple(inputs[0].shape[2:])
+    if any(w > E for w, E in zip(window, dims)):
+        raise ValueError(f"{who}: window {window} is larger than the volume {dims}")
+    idx = _target_index(target, B, inputs[0].device, who)
+    if not all(x.is_cuda for x in inputs):
+        raise ValueError(f"{who}: inputs must be CUDA tensors")
+    dev = inputs[0].device
+    xs = [TF._f32c(x.detach()) for x in inputs]
+    spec = towers[0]._spec
+    plan = TF.OccPlan(dims, window, stride, [(ks, pool) for _, _, ks, pool in spec.layers])
+    groups, i = [], 0
+    while i < len(towers):
+        grp = [i]
+        if i + 1 < len(towers) and towers[i + 1]._spec.dim == towers[i]._spec.dim and towers[i + 1]._hyper() == towers[i]._hyper():
+            grp.append(i + 1)
+        groups.append(grp)
+        i += len(grp)
+    nt, nwin = len(towers), plan.nwin
+    chunk = nwin if internal_batch_size is None else max(1, internal_batch_size // B)
+    chunk = min([chunk] + [TF.occ_pass_limit(plan, towers[g[0]]._spec, B, len(g)) for g in groups])
+
+    def objective(outs, rows):
+        logits = outs[0] if isinstance(outs, (tuple, list)) else outs
+        return logits.gather(1, rows.view(-1, 1)).view(-1)
+
+    outs = {}
+
+    def keep_out(module, args, out):
+        outs[module] = out
+
+    flags = [(p, p.requires_grad) for p in model.parameters()]
+    handles = []
+    try:
+        for p, _ in flags:
+            p.requires_grad_(False)
+        for t in towers:
+            t._lrp_keep = []
+            handles.append(t.register_forward_hook(keep_out))
+        with torch.no_grad():
+            f_x = objective(model(*xs), idx)
+        for h in handles:
+            h.remove()
+        handles = []
+        kept = [t._lrp_keep for t in towers]
+        if any(t not in outs for t in towers):
+            raise RuntimeError(f"{who}: a tower of the model did not run in its forward pass")
+        if any(len(k) != len(t._spec.layers) for k, t in zip(kept, towers)):
+            raise RuntimeError(f"{who}: the towers did not run the folded eval path (TMF_EVAL_FOLD=0?)")
+        base = [TF._f32c(outs[t].permute(0, 2, 3, 4, 1)) for t in towers]
+        tabs = [torch.from_numpy(tb).to(dev) for tb in plan.tab]          # ordinary host-to-device copies
+        scores = torch.empty((nt, nwin, B), dtype=torch.float32, device=dev)
+        for n0 in range(0, nwin, chunk):
+            m = min(chunk, nwin - n0)
+            rows = nt * m * B
+            # rows [u*m*B, (u+1)*m*B) occlude tower u's input: tower u's output there is composed, the others' replicated
+            bufs = [torch.empty((rows,) + plan.crop[-1] + (b.shape[-1],), dtype=torch.float32, device=dev) for b in base]
+            tab = [tb[n0:n0 + m] for tb in tabs]
+            for grp in groups:
+                TF.occ_towers(towers[grp[0]]._spec, towers[grp[0]]._hyper(), [towers[t]._folds for t in grp],
+                              [xs[t] for t in grp], [kept[t] for t in grp], [base[t] for t in grp], plan, tab, m, baseline,
+                              [bufs[t][t * m * B:(t + 1) * m * B] for t in grp])
+            reps = [(t, u) for t in range(nt) for u in range(nt) if u != t]
+            while reps:
+                pair = reps[:2] if len(reps) > 1 and base[reps[0][0]].shape == base[reps[1][0]].shape else reps[:1]
+                TF.occ_compose([base[t] for t, _ in pair], None, tab[-1], m, plan.crop[-1],
+                               out=[bufs[t][u * m * B:(u + 1) * m * B] for t, u in pair], tag="tmf_occ_compose@base")
+                reps = reps[len(pair):]
+            for t, buf in zip(towers, bufs):
+                t._occ_out = buf.permute(0, 4, 1, 2, 3)
+            # zero-stride stand-ins of batch rows: the towers return their composed outputs and never read them
+            stand_ins = [x.as_strided((rows,) + tuple(x.shape[1:]), (0,) * 5) for x in xs]
+            with torch.no_grad():
+                f_occ = objective(model(*stand_ins), idx.repeat(nt * m)).view(nt, m, B)
+            scores[:, n0:n0 + m] = f_x.view(1, 1, B) - f_occ
+    finally:
+        for h in handles:
+            h.remove()
+        for p, f in flags:
+            p.requires_grad_(f)
+        for t in towers:
+            t._lrp_keep = None
+            t._occ_out = None
+    per = [s.t().reshape((B,) + plan.grid).contiguous() for s in scores.unbind(0)]
+    return Occlusion(TF.occ_map(per, plan), per)

@@ -51,6 +51,7 @@ class sNet(nn.Module):
         self._lrp_keep = None          # transmf_ad_b200.interpret.lrp: a list the folded eval forward appends (a, y) to
         self._lrp_folds = {}           # LRP rule -> 7 TF.LrpFold
         self._ig_src = None            # transmf_ad_b200.interpret.integrated_gradients: block 1's output (fp32 leaf, bf16 twin)
+        self._occ_out = None           # transmf_ad_b200.interpret.occlusion: the composed tower output, returned as is
 
     def _units(self):
         """[(conv, bn)] in execution order."""
@@ -109,6 +110,8 @@ class sNet(nn.Module):
         return params, bufs
 
     def forward(self, mri):
+        if self._occ_out is not None:
+            return self._occ_out
         params, bufs = self._params_and_buffers()
         taps = _tapped_boundaries([self])
         if taps:
@@ -119,7 +122,8 @@ class sNet(nn.Module):
 def snet_pair_forward(net_a: sNet, net_b: sNet, xa, xb):
     """Run two towers of identical shape as one grouped launch sequence (grid.z = tower).  Forward pre-hooks and forward
     hooks of the towers fire as ``nn.Module.__call__`` would fire them; towers with backward hooks go through it."""
-    if (net_a._spec.dim != net_b._spec.dim or net_a.training != net_b.training or tuple(xa.shape) != tuple(xb.shape)
+    if (net_a._occ_out is not None or net_b._occ_out is not None
+            or net_a._spec.dim != net_b._spec.dim or net_a.training != net_b.training or tuple(xa.shape) != tuple(xb.shape)
             or net_a._hyper() != net_b._hyper() or _has_backward_hooks(net_a) or _has_backward_hooks(net_b)):
         return net_a(xa), net_b(xb)
     xa, xb = _fire_pre_hooks(net_a, xa), _fire_pre_hooks(net_b, xb)
