@@ -381,6 +381,21 @@ int tmf_occ_compose(int ng, const void* const* base, const void* const* crop, co
 int tmf_occ_map(int ng, const float* const* scores, float* const* map, int B, int D, int H, int W, int nD, int nH, int nW,
                 int wD, int wH, int wW, int sD, int sH, int sW, void* stream);
 
+/* ---- feature ablation over the regions of a mask through the sNet towers (DESIGN section 3.12) -----------------------------
+ * The crops and tables of occlusion (tab as for tmf_occ_input, from functional.BoxPlan: one row per box, rows n*B + b); mask:
+ * int32 [1|B][D][H][W] (mask_per_sample != 0: one volume per sample).  Every element written once, no atomics, 64-bit offsets.
+ * tmf_abl_input: out[g] fp32 [m*B][Dc][Hc][Wc] = x[g][b] at crop origin + (x, y, z), or the baseline where that voxel lies in
+ * [lo, hi) on all three axes and its mask id equals ids[n] (device int32 [m]).  The baseline of tower g: bvol[g] (fp32
+ * [1|B][D][H][W], one volume per sample where bit g of bvol_per_sample is set), or the scalar bval[g] (host array) where bvol
+ * or bvol[g] is NULL.
+ * tmf_abl_map: map[g] fp32 [B][D][H][W] = scores[g][b][id] (fp32 [B][F]) for the voxel's mask id, 0 for an id outside
+ * [0, F). */
+int tmf_abl_input(int ng, const float* const* x, const int* mask, int mask_per_sample, const float* const* bvol,
+                  const float* bval, int bvol_per_sample, const int* tab, const int* ids, int m, float* const* out, int B,
+                  int D, int H, int W, int Dc, int Hc, int Wc, void* stream);
+int tmf_abl_map(int ng, const float* const* scores, const int* mask, int mask_per_sample, int F, float* const* map, int B,
+                int D, int H, int W, void* stream);
+
 /* ---- attention maps of the fusion transformer (DESIGN section 3.8) ------------------------------------------------------
  * tmf_attn_scores: per-head product of the attention core's operands (q / kv as for tmf_attn_fwd; dh in {16, 32, 64}, any
  * Nq, Nk), written out as fp32 [B, heads, Nq, Nk]:

@@ -1272,7 +1272,7 @@ class OccPlan:
         import numpy as np
         self.dims, self.window, self.stride = tuple(dims), tuple(window), tuple(stride)
         self.grid = tuple(len(occ_positions(E, w, s)) for E, w, s in zip(dims, window, stride))
-        axes = [self._axis(E, w, s, layers) for E, w, s in zip(dims, window, stride)]
+        axes = [self._axis(E, [(a, a + w) for a in occ_positions(E, w, s)], layers) for E, w, s in zip(dims, window, stride)]
         self.crop = [tuple(ax[0][l] for ax in axes) for l in range(len(layers) + 1)]
         self.full = [tuple(ax[1][l] for ax in axes) for l in range(len(layers) + 1)]
         nD, nH, nW = self.grid
@@ -1289,18 +1289,18 @@ class OccPlan:
         return self.grid[0] * self.grid[1] * self.grid[2]
 
     @staticmethod
-    def _axis(E, w, s, layers):
-        """One axis: crop extents, full extents and the [n, 8, 4] table (crop origin, lo, hi, previous output origin)."""
+    def _axis(E, spans, layers):
+        """One axis for the intervals ``spans`` [(a, b)] of the input changed, one per window or box: crop extents (one per
+        layer for all of them), full extents and the [n, 8, 4] table (crop origin, lo, hi, previous output origin)."""
         import numpy as np
-        starts = occ_positions(E, w, s)
         nl = len(layers)
         ext = [E]
         for ks, pool in layers:
             ext.append(ext[-1] // 2 if pool != L.POOL_NONE else ext[-1])
         # pass 1: per window and layer the changed input [a, b), the recompute region [ra, rb) and the needed input [na, nb)
         geo = []
-        for a0 in starts:
-            a, b, rows = a0, a0 + w, []
+        for a, b in spans:
+            rows = []
             for l, (ks, pool) in enumerate(layers):
                 e, h = ext[l], ks // 2
                 oa, ob = max(a - h, 0), min(b + h, e)                     # conv outputs that change
@@ -1320,7 +1320,7 @@ class OccPlan:
                 c += 1                           # the inward shift at the far face must keep an even origin
             crop.append(min(c, e))
         crop.append(ext[nl])
-        tab = np.zeros((len(starts), nl + 1, 4), dtype=np.int32)
+        tab = np.zeros((len(spans), nl + 1, 4), dtype=np.int32)
         for n, rows in enumerate(geo):
             prev = 0
             for l, (ks, pool) in enumerate(layers):
@@ -1418,8 +1418,13 @@ def occ_towers(spec, hyper, folds, xs, kept, base_out, plan, tabs, m, baseline, 
     the final composition writes the (m*B, d, h, w, C) fp32 tower outputs into ``out``.  folds[t]: the tower's 7 ``EvalFold``
     (current: the base forward refreshed them); kept[t]: its 7 (input activation, y) pairs; base_out[t]: its fp32 (B,d,h,w,C)
     output; tabs: the pass's device tables (``OccPlan.tab`` rows), one per layer and the output."""
+    return occ_crops(spec, hyper, folds, occ_input(xs, tabs[0], m, baseline, plan.crop[0]), kept, base_out, plan, tabs, m, out)
+
+
+def occ_crops(spec, hyper, folds, act, kept, base_out, plan, tabs, m, out):
+    """``occ_towers`` from given fp32 (m*B, 1, Dc, Hc, Wc) layer-0 crops ``act`` (one per tower): layers 0 .. 6 and the
+    composition of the tower outputs into ``out``.  ``plan``: an ``OccPlan`` or a ``BoxPlan``."""
     impl = conv_impl()
-    act = occ_input(xs, tabs[0], m, baseline, plan.crop[0])
     for l in range(len(spec.layers)):
         if l > 0:
             act = occ_compose([k[l][0] for k in kept], act, tabs[l], m, plan.crop[l], tag=f"tmf_occ_compose@L{l}")
@@ -1435,4 +1440,94 @@ def occ_map(scores, plan):
     for i in range(0, len(scores), 2):
         L.call("tmf_occ_map", len(scores[i:i + 2]), L.ptrs(scores[i:i + 2]), L.ptrs(maps[i:i + 2]), B, *plan.dims, *plan.grid,
                *plan.window, *plan.stride)
+    return maps
+
+
+# ==============================================================================================================
+# Feature ablation over regions of a mask, with incremental recomputation   (csrc/ablation.cu; DESIGN section 3.12)
+# ==============================================================================================================
+# Extent classes: per axis, a feature's box extent rounds up to the first rung that is at least as large (the full extent past
+# the last rung).  The features of one class share crop extents, the largest over the class.  Coarse rungs: fewer, fuller
+# passes through the fusion stack outweigh the padding (finer ladders measured slower, DESIGN section 3.12).
+ABL_LADDER = (24, 48, 96)
+
+
+class BoxPlan:
+    """Crop geometry of incremental recomputation for a list of boxes ``[((a0, b0), (a1, b1), (a2, b2))]`` of the input, one
+    per feature of an extent class (host only).  Each axis goes through ``OccPlan._axis`` with the boxes' intervals, so the
+    crop extents are one per layer for all the boxes; ``crop`` and ``full`` as for ``OccPlan``; ``tab[l]``: int32 numpy
+    [n, 3, 4], per box and axis, the same layout; ``ids``: int32 numpy [n], the boxes' feature ids."""
+
+    def __init__(self, dims, boxes, layers, ids):
+        import numpy as np
+        self.dims = tuple(dims)
+        axes = [OccPlan._axis(E, [bx[a] for bx in boxes], layers) for a, E in enumerate(self.dims)]
+        self.crop = [tuple(ax[0][l] for ax in axes) for l in range(len(layers) + 1)]
+        self.full = [tuple(ax[1][l] for ax in axes) for l in range(len(layers) + 1)]
+        self.tab = [np.ascontiguousarray(np.stack([ax[2][:, l] for ax in axes], axis=1)) for l in range(len(layers) + 1)]
+        self.ids = np.asarray(ids, dtype=np.int32)
+
+    @property
+    def n(self):
+        return len(self.ids)
+
+
+def abl_boxes(mask, F):
+    """Bounding box of every id 0 .. F-1 of an integer mask (1|B, 1, D, H, W), over all its samples (torch ops on the mask's
+    device, then one device-to-host copy): int64 numpy [F, 6] (lo_D, lo_H, lo_W, hi_D, hi_H, hi_W), hi exclusive; an absent
+    id has lo = extent and hi = 0."""
+    dims = mask.shape[2:]
+    ids = mask.reshape(-1).long()
+    cols = []
+    for a, E in enumerate(dims):
+        shape = [1] * 5
+        shape[2 + a] = E
+        c = torch.arange(E, device=mask.device).view(shape).expand(mask.shape).reshape(-1)
+        cols.append((torch.full((F,), E, dtype=torch.long, device=mask.device).scatter_reduce_(0, ids, c, "amin"),
+                     torch.full((F,), -1, dtype=torch.long, device=mask.device).scatter_reduce_(0, ids, c, "amax") + 1))
+    return torch.stack([lo for lo, _ in cols] + [hi for _, hi in cols], 1).cpu().numpy()
+
+
+def abl_classes(boxes, dims):
+    """The present features of ``abl_boxes`` grouped by extent class (``ABL_LADDER``): [(class key, [ids ascending])] in key
+    order.  The grouping depends on the mask alone, so a feature's crop extents do not depend on how the passes are cut."""
+    classes = {}
+    for f in range(len(boxes)):
+        ext = [int(boxes[f, 3 + a] - boxes[f, a]) for a in range(3)]
+        if ext[0] <= 0:
+            continue
+        key = tuple(next((r for r in ABL_LADDER if e <= r < E), E) for e, E in zip(ext, dims))
+        classes.setdefault(key, []).append(f)
+    return sorted(classes.items())
+
+
+def abl_plan(boxes, ids, dims, layers):
+    """The ``BoxPlan`` of one extent class: the features ``ids`` with their boxes from ``abl_boxes``."""
+    return BoxPlan(dims, [tuple((int(boxes[f, a]), int(boxes[f, 3 + a])) for a in range(3)) for f in ids], layers, ids)
+
+
+def abl_input(xs, mask, baselines, tab, ids, m, extent):
+    """fp32 (m*B, 1, Dc, Hc, Wc) layer-0 crops per tower (``tmf_abl_input``): x, with the baseline where the mask holds the
+    row's feature id.  xs: fp32 contiguous (B,1,D,H,W); mask: int32 contiguous (1|B,1,D,H,W); baselines: per tower a float or
+    an fp32 contiguous (1|B,1,D,H,W) tensor; tab: a pass's layer-0 rows of ``BoxPlan.tab``; ids: int32 [m], their features."""
+    import ctypes
+    B, _, D, H, W = xs[0].shape
+    out = [torch.empty((m * B, 1) + tuple(extent), dtype=torch.float32, device=xs[0].device) for _ in xs]
+    vols = [b if torch.is_tensor(b) else None for b in baselines]
+    vals = (ctypes.c_float * len(xs))(*[0.0 if torch.is_tensor(b) else float(b) for b in baselines])
+    per = sum(1 << g for g, v in enumerate(vols) if v is not None and v.shape[0] > 1)
+    L.call("tmf_abl_input", len(xs), L.ptrs(xs), L.ptr(mask), int(mask.shape[0] > 1), L.ptrs(vols), vals, per, L.ptr(tab),
+           L.ptr(ids), m, L.ptrs(out), B, D, H, W, *extent)
+    return out
+
+
+def abl_map(scores, mask):
+    """Per tower, the fp32 (B,1,D,H,W) map with each voxel holding its feature's score, map[b, v] = scores[b, mask[b|0, v]]
+    (``tmf_abl_map``).  scores: fp32 contiguous (B, F) per tower; mask: int32 contiguous (1|B,1,D,H,W), ids < F."""
+    B, F = scores[0].shape
+    dims = tuple(mask.shape[2:])
+    maps = [torch.empty((B, 1) + dims, dtype=torch.float32, device=scores[0].device) for _ in scores]
+    for i in range(0, len(scores), 2):
+        L.call("tmf_abl_map", len(scores[i:i + 2]), L.ptrs(scores[i:i + 2]), L.ptr(mask), int(mask.shape[0] > 1), F,
+               L.ptrs(maps[i:i + 2]), B, *dims)
     return maps

@@ -1,7 +1,7 @@
 """Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, layer-wise relevance
-propagation (Bach et al., 2015), integrated gradients (Sundararajan et al., 2017) and occlusion sensitivity (Zeiler & Fergus,
-2014) through the towers, and head-averaged or gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the
-fusion transformer.
+propagation (Bach et al., 2015), integrated gradients (Sundararajan et al., 2017), occlusion sensitivity (Zeiler & Fergus,
+2014) and feature ablation over the regions of a mask through the towers, and head-averaged or gradient-weighted (Chefer
+et al., 2021) cross-modal attention maps of the fusion transformer.
 
 Input gradients (saliency maps) need nothing from here: ``mri.requires_grad_(True)`` and plain autograd work on every model
 (INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c), and so do
@@ -393,6 +393,76 @@ def integrated_gradients(model, inputs, target, n_steps=50, method="gausslegendr
 Occlusion = namedtuple("Occlusion", ["maps", "scores"])
 
 
+def _refuse_tower_hooks(towers, who, what):
+    for t in towers:
+        for mod in [t] + [getattr(t, name) for name in BLOCKS]:
+            if mod._forward_hooks or mod._forward_pre_hooks or _has_backward_hooks(mod):
+                raise ValueError(f"{who}: hooks on an sNet tower or its blocks would observe tensors that are never formed "
+                                 f"(the {what} towers run on crops); remove them")
+
+
+def _tower_groups(towers):
+    """Runs of at most two consecutive towers of one shape, which go through the crop launches as one group."""
+    groups, i = [], 0
+    while i < len(towers):
+        grp = [i]
+        if i + 1 < len(towers) and towers[i + 1]._spec.dim == towers[i]._spec.dim and towers[i + 1]._hyper() == towers[i]._hyper():
+            grp.append(i + 1)
+        groups.append(grp)
+        i += len(grp)
+    return groups
+
+
+def _objective(outs, rows):
+    logits = outs[0] if isinstance(outs, (tuple, list)) else outs
+    return logits.gather(1, rows.view(-1, 1)).view(-1)
+
+
+def _base_forward(model, towers, xs, idx, who):
+    """The unchanged eval forward that incremental recomputation starts from: f(x), every tower's kept (input activation, y)
+    pairs and its fp32 (B, d, h, w, C) output.  Sets ``_lrp_keep`` on the towers; the caller clears it."""
+    outs = {}
+
+    def keep_out(module, args, out):
+        outs[module] = out
+
+    handles = []
+    try:
+        for t in towers:
+            t._lrp_keep = []
+            handles.append(t.register_forward_hook(keep_out))
+        with torch.no_grad():
+            f_x = _objective(model(*xs), idx)
+    finally:
+        for h in handles:
+            h.remove()
+    kept = [t._lrp_keep for t in towers]
+    if any(t not in outs for t in towers):
+        raise RuntimeError(f"{who}: a tower of the model did not run in its forward pass")
+    if any(len(k) != len(t._spec.layers) for k, t in zip(kept, towers)):
+        raise RuntimeError(f"{who}: the towers did not run the folded eval path (TMF_EVAL_FOLD=0?)")
+    return f_x, kept, [TF._f32c(outs[t].permute(0, 2, 3, 4, 1)) for t in towers]
+
+
+def _through_fusion(model, towers, xs, base, bufs, tab_out, m, extent, idx, blocks):
+    """The end of a pass whose tower outputs are composed into ``bufs`` (per tower, fp32 rows blocks*m*B): with blocks > 1,
+    row block u changed tower u only, and the other towers' outputs there are replicated from their base outputs; then the
+    model's own fusion stack and heads.  Returns the objective on the rows, (blocks, m, B)."""
+    nt, B = len(towers), xs[0].shape[0]
+    reps = [(t, u) for t in range(nt) for u in range(nt) if u != t] if blocks > 1 else []
+    while reps:
+        pair = reps[:2] if len(reps) > 1 and base[reps[0][0]].shape == base[reps[1][0]].shape else reps[:1]
+        TF.occ_compose([base[t] for t, _ in pair], None, tab_out, m, extent,
+                       out=[bufs[t][u * m * B:(u + 1) * m * B] for t, u in pair], tag="tmf_occ_compose@base")
+        reps = reps[len(pair):]
+    for t, buf in zip(towers, bufs):
+        t._occ_out = buf.permute(0, 4, 1, 2, 3)
+    # zero-stride stand-ins of batch rows: the towers return their composed outputs and never read them
+    stand_ins = [x.as_strided((blocks * m * B,) + tuple(x.shape[1:]), (0,) * 5) for x in xs]
+    with torch.no_grad():
+        return _objective(model(*stand_ins), idx.repeat(blocks * m)).view(blocks, m, B)
+
+
 def _triple(v, who, name):
     v = (v,) * 3 if isinstance(v, int) and not isinstance(v, bool) else v
     if not (isinstance(v, (tuple, list)) and len(v) == 3 and all(_is_count(e) for e in v)):
@@ -434,11 +504,7 @@ def occlusion(model, inputs, target, window=16, stride=8, baseline=0.0, internal
     if (len(inputs) != len(towers) or not all(torch.is_tensor(x) and x.dim() == 5 and x.shape[1] == 1 for x in inputs)
             or any(x.shape != inputs[0].shape for x in inputs)):
         raise ValueError(f"{who}: inputs must be {len(towers)} (B,1,D,H,W) volume(s) of one shape, one per tower")
-    for t in towers:
-        for mod in [t] + [getattr(t, name) for name in BLOCKS]:
-            if mod._forward_hooks or mod._forward_pre_hooks or _has_backward_hooks(mod):
-                raise ValueError(f"{who}: hooks on an sNet tower or its blocks would observe tensors that are never formed "
-                                 f"(the occluded towers run on crops); remove them")
+    _refuse_tower_hooks(towers, who, "occluded")
     B, dims = inputs[0].shape[0], tuple(inputs[0].shape[2:])
     if any(w > E for w, E in zip(window, dims)):
         raise ValueError(f"{who}: window {window} is larger than the volume {dims}")
@@ -449,45 +515,16 @@ def occlusion(model, inputs, target, window=16, stride=8, baseline=0.0, internal
     xs = [TF._f32c(x.detach()) for x in inputs]
     spec = towers[0]._spec
     plan = TF.OccPlan(dims, window, stride, [(ks, pool) for _, _, ks, pool in spec.layers])
-    groups, i = [], 0
-    while i < len(towers):
-        grp = [i]
-        if i + 1 < len(towers) and towers[i + 1]._spec.dim == towers[i]._spec.dim and towers[i + 1]._hyper() == towers[i]._hyper():
-            grp.append(i + 1)
-        groups.append(grp)
-        i += len(grp)
+    groups = _tower_groups(towers)
     nt, nwin = len(towers), plan.nwin
     chunk = nwin if internal_batch_size is None else max(1, internal_batch_size // B)
     chunk = min([chunk] + [TF.occ_pass_limit(plan, towers[g[0]]._spec, B, len(g)) for g in groups])
 
-    def objective(outs, rows):
-        logits = outs[0] if isinstance(outs, (tuple, list)) else outs
-        return logits.gather(1, rows.view(-1, 1)).view(-1)
-
-    outs = {}
-
-    def keep_out(module, args, out):
-        outs[module] = out
-
     flags = [(p, p.requires_grad) for p in model.parameters()]
-    handles = []
     try:
         for p, _ in flags:
             p.requires_grad_(False)
-        for t in towers:
-            t._lrp_keep = []
-            handles.append(t.register_forward_hook(keep_out))
-        with torch.no_grad():
-            f_x = objective(model(*xs), idx)
-        for h in handles:
-            h.remove()
-        handles = []
-        kept = [t._lrp_keep for t in towers]
-        if any(t not in outs for t in towers):
-            raise RuntimeError(f"{who}: a tower of the model did not run in its forward pass")
-        if any(len(k) != len(t._spec.layers) for k, t in zip(kept, towers)):
-            raise RuntimeError(f"{who}: the towers did not run the folded eval path (TMF_EVAL_FOLD=0?)")
-        base = [TF._f32c(outs[t].permute(0, 2, 3, 4, 1)) for t in towers]
+        f_x, kept, base = _base_forward(model, towers, xs, idx, who)
         tabs = [torch.from_numpy(tb).to(dev) for tb in plan.tab]          # ordinary host-to-device copies
         scores = torch.empty((nt, nwin, B), dtype=torch.float32, device=dev)
         for n0 in range(0, nwin, chunk):
@@ -500,22 +537,9 @@ def occlusion(model, inputs, target, window=16, stride=8, baseline=0.0, internal
                 TF.occ_towers(towers[grp[0]]._spec, towers[grp[0]]._hyper(), [towers[t]._folds for t in grp],
                               [xs[t] for t in grp], [kept[t] for t in grp], [base[t] for t in grp], plan, tab, m, baseline,
                               [bufs[t][t * m * B:(t + 1) * m * B] for t in grp])
-            reps = [(t, u) for t in range(nt) for u in range(nt) if u != t]
-            while reps:
-                pair = reps[:2] if len(reps) > 1 and base[reps[0][0]].shape == base[reps[1][0]].shape else reps[:1]
-                TF.occ_compose([base[t] for t, _ in pair], None, tab[-1], m, plan.crop[-1],
-                               out=[bufs[t][u * m * B:(u + 1) * m * B] for t, u in pair], tag="tmf_occ_compose@base")
-                reps = reps[len(pair):]
-            for t, buf in zip(towers, bufs):
-                t._occ_out = buf.permute(0, 4, 1, 2, 3)
-            # zero-stride stand-ins of batch rows: the towers return their composed outputs and never read them
-            stand_ins = [x.as_strided((rows,) + tuple(x.shape[1:]), (0,) * 5) for x in xs]
-            with torch.no_grad():
-                f_occ = objective(model(*stand_ins), idx.repeat(nt * m)).view(nt, m, B)
+            f_occ = _through_fusion(model, towers, xs, base, bufs, tab[-1], m, plan.crop[-1], idx, nt)
             scores[:, n0:n0 + m] = f_x.view(1, 1, B) - f_occ
     finally:
-        for h in handles:
-            h.remove()
         for p, f in flags:
             p.requires_grad_(f)
         for t in towers:
@@ -523,3 +547,134 @@ def occlusion(model, inputs, target, window=16, stride=8, baseline=0.0, internal
             t._occ_out = None
     per = [s.t().reshape((B,) + plan.grid).contiguous() for s in scores.unbind(0)]
     return Occlusion(TF.occ_map(per, plan), per)
+
+
+FeatureAblation = namedtuple("FeatureAblation", ["maps", "scores"])
+
+
+def _ablation_baselines(baselines, nt, shape, device, who):
+    """Per tower a float or an fp32 contiguous (1|B,1,D,H,W) tensor, from a scalar or a tuple of one entry per tower."""
+    import math
+
+    def scalar(b):
+        return isinstance(b, (int, float)) and not isinstance(b, bool) and math.isfinite(b)
+
+    if not isinstance(baselines, (tuple, list)):
+        if not scalar(baselines):
+            raise ValueError(f"{who}: baselines must be a finite Python scalar or a tuple of {nt} entries, one per tower; "
+                             f"got {baselines!r}")
+        return [float(baselines)] * nt
+    if len(baselines) != nt:
+        raise ValueError(f"{who}: baselines must be a scalar or a tuple of {nt} entries, one per tower; got {len(baselines)}")
+    out = []
+    for b in baselines:
+        if scalar(b):
+            out.append(float(b))
+        elif (torch.is_tensor(b) and b.dtype == torch.float32 and b.device == device and b.dim() == 5
+              and b.shape[0] in (1, shape[0]) and tuple(b.shape[1:]) == tuple(shape[1:])):
+            out.append(b.detach().contiguous())
+        else:
+            raise ValueError(f"{who}: each baseline must be a finite Python scalar or an fp32 tensor of shape "
+                             f"(1|{shape[0]}, 1, {', '.join(map(str, shape[2:]))}) on {device}; got {b!r}")
+    return out
+
+
+def feature_ablation(model, inputs, target, feature_mask, baselines=0.0, joint=False, internal_batch_size=None):
+    """Feature ablation over the regions of ``feature_mask`` through every sNet tower of ``model`` (eval mode), for the
+    objective f = ``logits[b, target_b]`` of the model's first output (captum's ``FeatureAblation`` with a feature mask).
+
+    ``feature_mask``: an integer tensor (1|B, 1, D, H, W) on the inputs' device; every id present, 0 included, is one feature,
+    and ids must be >= 0.  It applies to every tower's input (the modalities are co-registered); a per-sample mask ablates
+    each sample's own region.  ``baselines``: a finite Python scalar, or a tuple of one entry per tower, each a finite scalar
+    or an fp32 CUDA tensor (1|B, 1, D, H, W); inside the feature the voxels take the baseline's value.  ``joint``: False
+    ablates a feature in one tower's input at a time; True ablates it in every tower's input at once (captum's
+    ``enable_cross_tensor_attribution``).  ``inputs``, ``target`` and ``internal_batch_size`` (volumes per pass) as for
+    ``occlusion``.
+
+    Returns ``FeatureAblation(maps, scores)``, per tower in tower order: ``scores`` fp32 (B, F), F = max id + 1, f(x) - f(x
+    with feature j ablated) (0 for an id absent from the mask; with ``joint`` every tower has the same scores); ``maps`` fp32
+    (B,1,D,H,W), each voxel holding its feature's score.
+
+    The ablated towers are not run in full (DESIGN section 3.12): as in ``occlusion``, each feature recomputes only what its
+    bounding box changes, on crops of one extent per extent class of features, and the composed tower outputs go through
+    the model's own fusion stack and heads.  No parameter receives a ``.grad``, no weight-gradient kernel runs, BatchNorm
+    buffers and the module mode are untouched and ``requires_grad`` flags are restored."""
+    who = "feature_ablation"
+    if not isinstance(joint, bool):
+        raise ValueError(f"{who}: joint must be True or False; got {joint!r}")
+    if internal_batch_size is not None and not _is_count(internal_batch_size):
+        raise ValueError(f"{who}: internal_batch_size must be None or an integer >= 1; got {internal_batch_size!r}")
+    towers = [m for m in model.modules() if isinstance(m, sNet)]
+    if not towers:
+        raise ValueError(f"{who}: the model has no sNet tower")
+    if any(m.training for m in model.modules()):
+        raise ValueError(f"{who}: BatchNorm is folded with its running statistics; call model.eval() first")
+    inputs = tuple(inputs) if isinstance(inputs, (tuple, list)) else (inputs,)
+    if (len(inputs) != len(towers) or not all(torch.is_tensor(x) and x.dim() == 5 and x.shape[1] == 1 for x in inputs)
+            or any(x.shape != inputs[0].shape for x in inputs)):
+        raise ValueError(f"{who}: inputs must be {len(towers)} (B,1,D,H,W) volume(s) of one shape, one per tower")
+    _refuse_tower_hooks(towers, who, "ablated")
+    shape = tuple(inputs[0].shape)
+    B, dims, dev = shape[0], shape[2:], inputs[0].device
+    mask = feature_mask
+    if (not torch.is_tensor(mask) or mask.is_floating_point() or mask.is_complex() or mask.dtype == torch.bool
+            or mask.dim() != 5 or mask.shape[0] not in (1, B) or tuple(mask.shape[1:]) != shape[1:] or mask.device != dev):
+        got = f"{mask.dtype} {tuple(mask.shape)} on {mask.device}" if torch.is_tensor(mask) else repr(mask)
+        raise ValueError(f"{who}: feature_mask must be an integer tensor of shape (1|{B}, 1, {', '.join(map(str, dims))}) on "
+                         f"{dev}; got {got}")
+    bls = _ablation_baselines(baselines, len(towers), shape, dev, who)
+    idx = _target_index(target, B, dev, who)
+    if not all(x.is_cuda for x in inputs):
+        raise ValueError(f"{who}: inputs must be CUDA tensors")
+    lo, hi = (int(v) for v in torch.stack(mask.aminmax()).tolist())           # one device-to-host copy of the id range
+    if lo < 0:
+        raise ValueError(f"{who}: feature_mask ids must be >= 0; found {lo}")
+    if hi >= 2 ** 31 - 1:
+        raise ValueError(f"{who}: feature_mask ids must be below 2^31 - 1; found {hi}")
+    F = hi + 1
+    mask = mask.to(torch.int32).contiguous()
+    xs = [TF._f32c(x.detach()) for x in inputs]
+    spec = towers[0]._spec
+    layers = [(ks, pool) for _, _, ks, pool in spec.layers]
+    boxes = TF.abl_boxes(mask, F)
+    plans = [TF.abl_plan(boxes, ids, dims, layers) for _, ids in TF.abl_classes(boxes, dims)]
+    groups = _tower_groups(towers)
+    nt = len(towers)
+    blocks = 1 if joint else nt
+
+    flags = [(p, p.requires_grad) for p in model.parameters()]
+    try:
+        for p, _ in flags:
+            p.requires_grad_(False)
+        f_x, kept, base = _base_forward(model, towers, xs, idx, who)
+        scores = torch.zeros((blocks, F, B), dtype=torch.float32, device=dev)
+        for plan in plans:
+            tabs = [torch.from_numpy(tb).to(dev) for tb in plan.tab]      # ordinary host-to-device copies
+            fids = torch.from_numpy(plan.ids).to(dev)
+            chunk = plan.n if internal_batch_size is None else max(1, internal_batch_size // B)
+            chunk = min([chunk] + [TF.occ_pass_limit(plan, towers[g[0]]._spec, B, len(g)) for g in groups])
+            for n0 in range(0, plan.n, chunk):
+                m = min(chunk, plan.n - n0)
+                # joint: every tower's rows 0 .. m*B are composed from its own crops; else rows [u*m*B, (u+1)*m*B) ablate
+                # tower u, and the other towers' outputs there are replicated from their base outputs
+                bufs = [torch.empty((blocks * m * B,) + plan.crop[-1] + (b.shape[-1],), dtype=torch.float32, device=dev)
+                        for b in base]
+                tab = [tb[n0:n0 + m] for tb in tabs]
+                for grp in groups:
+                    act = TF.abl_input([xs[t] for t in grp], mask, [bls[t] for t in grp], tab[0], fids[n0:n0 + m], m,
+                                       plan.crop[0])
+                    TF.occ_crops(towers[grp[0]]._spec, towers[grp[0]]._hyper(), [towers[t]._folds for t in grp], act,
+                                 [kept[t] for t in grp], [base[t] for t in grp], plan, tab, m,
+                                 [bufs[t][(0 if joint else t) * m * B:((0 if joint else t) + 1) * m * B] for t in grp])
+                f_abl = _through_fusion(model, towers, xs, base, bufs, tab[-1], m, plan.crop[-1], idx, blocks)
+                scores[:, plan.ids[n0:n0 + m].tolist()] = f_x.view(1, 1, B) - f_abl
+    finally:
+        for p, f in flags:
+            p.requires_grad_(f)
+        for t in towers:
+            t._lrp_keep = None
+            t._occ_out = None
+    per = [s.t().contiguous() for s in scores.unbind(0)]
+    if joint:
+        per += [per[0].clone() for _ in range(nt - 1)]
+    return FeatureAblation(TF.abl_map(per, mask), per)

@@ -37,6 +37,24 @@ def make_volumes(batch, shape=PRIMARY_SHAPE, seed=1, labels=None, device="cpu"):
     return vol.contiguous().to(device)
 
 
+def make_atlas(shape=PRIMARY_SHAPE, cells=96, seed=0, radius=0.42):
+    """-> int64 (1,1,D,H,W) synthetic parcellation: ``cells`` Voronoi cells (ids 1 .. cells) of seeded centres inside an
+    ellipsoid of semi-axes ``radius`` times the extent, background 0 outside it (a stand-in for an anatomical atlas)."""
+    g = torch.Generator().manual_seed(int(seed))
+    D, H, W = shape
+    grid = torch.stack(torch.meshgrid(torch.arange(D), torch.arange(H), torch.arange(W), indexing="ij"), -1).reshape(-1, 3)
+    grid = grid.double()
+    centre = torch.tensor([(D - 1) / 2, (H - 1) / 2, (W - 1) / 2], dtype=torch.float64)
+    semi = radius * torch.tensor([D, H, W], dtype=torch.float64)
+    inside = (((grid - centre) / semi) ** 2).sum(1) <= 1
+    pts = grid[inside]
+    seeds = pts[torch.randperm(len(pts), generator=g)[:cells]]
+    lab = torch.zeros(D * H * W, dtype=torch.int64)
+    cell = torch.cat([torch.cdist(pts[i:i + 65536], seeds).argmin(1) for i in range(0, len(pts), 65536)])
+    lab[inside] = cell + 1
+    return lab.view(1, 1, D, H, W)
+
+
 def make_labels(batch, device="cpu"):
     return (torch.arange(batch) % 2).to(torch.int64).to(device)
 
