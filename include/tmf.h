@@ -156,8 +156,11 @@ int tmf_bn_act_pool_fwd(int ng, const void* const* y, const float* const* coef, 
                         int B, int D, int H, int W, int C, int pool, float slope, void* stream);
 
 /* tmf_bn_act_pool_fwd for a MAX pool that also keeps ymax[B,D/2,H/2,W/2,C] (bf16): the stored pre-BN value behind each
- * window's maximum activation (first maximum in (d,h,w) scan order).  The backward reduction of the layer then runs on
- * ymax + dout at pooled resolution (tmf_bn_maxpool_bwd_reduce_kept) instead of re-reading y.  networks.py:23-25. */
+ * window's maximum activation, at the position every max-pool backward kernel routes to: the first in (d,h,w) scan order
+ * that maximises sign(scale)*y (position 0 where scale = 0).  It holds the maximum activation because the map is
+ * non-decreasing, which needs slope >= 0 (refused otherwise, like every max-pool entry point below).  The backward
+ * reduction of the layer then runs on ymax + dout at pooled resolution (tmf_bn_maxpool_bwd_reduce_kept) instead of
+ * re-reading y.  networks.py:23-25. */
 int tmf_bn_act_pool_fwd_keepmax(int ng, const void* const* y, const float* const* coef, void* const* out,
                                 void* const* ymax, int out_fp32, int B, int D, int H, int W, int C, float slope,
                                 void* stream);

@@ -3,7 +3,7 @@
 //   on NDHWC bf16 tensors, 16-byte vectorised (8 channels per thread), per-channel reductions in double.
 // Reference semantics: models/networks.py:23-25, 29-34, 38-43, 47-52 (nn.BatchNorm3d eps 1e-5 momentum 0.1, biased
 // variance for normalisation / unbiased into running_var; nn.LeakyReLU() slope 0.01; floor-mode pools; max-pool
-// gradient to the first maximum in (d,h,w) scan order).
+// gradient to the first maximum in (d,h,w) scan order, found on sign(scale)*y by every kernel: bn_act_pool_bwd_kernel).
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -137,10 +137,31 @@ __device__ __forceinline__ void store8f(void* base, int64_t elem_off, int fp32, 
   }
 }
 
-// KEEP (max pool only): also store ymax[B,Do,Ho,Wo,C] = the stored pre-BN value y whose activation is the window's
-// maximum (first maximum in (d,h,w) scan order, torch's rule).  The backward reduction of a max-pool layer needs y
-// only there (dz is zero elsewhere), so it can run on ymax + dout at pooled resolution instead of re-reading all of y:
-// block 1 re-read 925 MB per step for two per-channel sums.
+__device__ __forceinline__ uint32_t bf2_max(uint32_t a, uint32_t b) {
+  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
+  return *reinterpret_cast<uint32_t*>(&r);
+}
+__device__ __forceinline__ uint32_t u4_get(const uint4& v, int i) { return i == 0 ? v.x : (i == 1 ? v.y : (i == 2 ? v.z : v.w)); }
+
+// per 8-channel chunk: the sign bits of its 8 scales at the bf16 sign positions of 4 packed pairs (y ^ flip is
+// sign(scale)*y as a bf16 key), and 0xFFFF in the halves whose scale is zero
+__device__ __forceinline__ void scale_sign_pairs(const float* sc, uint32_t* flip, uint32_t* zero) {
+#pragma unroll
+  for (int j2 = 0; j2 < 4; ++j2) {
+    flip[j2] = ((__float_as_uint(sc[2 * j2]) >> 16) & 0x8000u) | (__float_as_uint(sc[2 * j2 + 1]) & 0x80000000u);
+    zero[j2] = (sc[2 * j2] == 0.f ? 0x0000FFFFu : 0u) | (sc[2 * j2 + 1] == 0.f ? 0xFFFF0000u : 0u);
+  }
+}
+
+// KEEP (max pool only): also store ymax[B,Do,Ho,Wo,C] = the stored pre-BN value y of the window's arg-max, chosen by the
+// backward kernels' rule: the first position in (d,h,w) scan order that maximises sign(scale)*y, position 0 when the
+// scale is 0.  Equal keys are equal y, so ymax is the maximum of the bf16 keys y ^ flip (HMNMX2 on packed pairs, one
+// instruction per two channels and position: per-element fp32 compares made this pass instruction-bound, 346 us instead
+// of 248 us at block 1, two towers of batch 8 on a B200 at 1000 W).  BatchNorm's affine map and a LeakyReLU with slope >= 0 are non-decreasing, so that position
+// holds the window's maximum activation (torch's first maximum wherever the activations are distinct); where fp32
+// rounding makes distinct y give equal activations, ymax still names the voxel the backward kernels route dz to.  The
+// backward reduction of a max-pool layer needs y only there (dz is zero elsewhere), so it can run on ymax + dout at
+// pooled resolution instead of re-reading all of y: block 1 re-read 925 MB per step for two per-channel sums.
 // DUAL: also store the fp32 value o in out32 (same layout as out); out (bf16) and ymax are the same bits as without it.
 template <bool KEEP, bool DUAL = false>
 __global__ void __launch_bounds__(256, DUAL ? 2 : (KEEP ? 3 : 4)) bn_act_pool_fwd_kernel(ActPoolArgs p) {
@@ -156,6 +177,8 @@ __global__ void __launch_bounds__(256, DUAL ? 2 : (KEEP ? 3 : 4)) bn_act_pool_fw
   float sc[8], sh[8];
 #pragma unroll
   for (int j = 0; j < 8; ++j) { sc[j] = p.coef.p[g][c0 + j]; sh[j] = p.coef.p[g][p.C + c0 + j]; }
+  uint32_t flip[4], zero[4];
+  if (KEEP) scale_sign_pairs(sc, flip, zero);
   const int nunits = p.B * p.Do * p.nch;
   for (int unit = blockIdx.x; unit < nunits; unit += gridDim.x) {
     const int hc = unit % p.nch;
@@ -178,29 +201,41 @@ __global__ void __launch_bounds__(256, DUAL ? 2 : (KEEP ? 3 : 4)) bn_act_pool_fw
     } else {
 #pragma unroll
       for (int j = 0; j < 8; ++j) o[j] = (p.pool == TMF_POOL_MAX) ? -INFINITY : 0.f;
-      float yb[8];
-      if (KEEP) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) yb[j] = 0.f;
-      }
+      uint32_t km[4], y0[4];                       // KEEP: window maximum of the bf16 keys y ^ flip; position 0's y
 #pragma unroll
       for (int q = 0; q < 8; ++q) {
         const int di = 2 * dd + (q >> 2), hi = 2 * ho + ((q >> 1) & 1), wi = 2 * wo + (q & 1);
+        const uint4 raw = *reinterpret_cast<const uint4*>(yg + ((((int64_t)n * p.D + di) * p.H + hi) * p.W + wi) * p.C + c0);
         float f[8];
-        unpack8(*reinterpret_cast<const uint4*>(yg + ((((int64_t)n * p.D + di) * p.H + hi) * p.W + wi) * p.C + c0), f);
+        unpack8(raw, f);
+        if (KEEP) {
+#pragma unroll
+          for (int j2 = 0; j2 < 4; ++j2) {
+            const uint32_t key = u4_get(raw, j2) ^ flip[j2];
+            if (q == 0) { km[j2] = key; y0[j2] = u4_get(raw, j2); }
+            else km[j2] = bf2_max(km[j2], key);
+          }
+        }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const float z = fmaf(f[j], sc[j], sh[j]);
           const float a = z > 0.f ? z : z * p.slope;
           if (KEEP) {
-            if (a > o[j]) { o[j] = a; yb[j] = f[j]; }          // strict: the first maximum wins
+            if (a > o[j]) o[j] = a;                // strict: the first maximum's bits, as without KEEP
           } else {
             o[j] = (p.pool == TMF_POOL_MAX) ? fmaxf(o[j], a) : o[j] + a;
           }
         }
       }
-      if (KEEP)
-        *reinterpret_cast<uint4*>(p.ymax.p[g] + ((((int64_t)n * p.Do + dd) * p.Ho + ho) * p.Wo + wo) * p.C + c0) = pack8(yb);
+      if (KEEP) {
+        // y of the maximum key (equal keys are equal y), position 0's y where the scale is zero
+        uint4 ym;
+        ym.x = ((km[0] ^ flip[0]) & ~zero[0]) | (y0[0] & zero[0]);
+        ym.y = ((km[1] ^ flip[1]) & ~zero[1]) | (y0[1] & zero[1]);
+        ym.z = ((km[2] ^ flip[2]) & ~zero[2]) | (y0[2] & zero[2]);
+        ym.w = ((km[3] ^ flip[3]) & ~zero[3]) | (y0[3] & zero[3]);
+        *reinterpret_cast<uint4*>(p.ymax.p[g] + ((((int64_t)n * p.Do + dd) * p.Ho + ho) * p.Wo + wo) * p.C + c0) = ym;
+      }
       if (p.pool == TMF_POOL_AVG) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) o[j] *= 0.125f;
@@ -248,8 +283,11 @@ __device__ __forceinline__ void block_channel_sums(float* red, double* rows, int
 // APPLY: write dy = scale * (dz - m1 - xhat*m2) for every existing input voxel (incl. those dropped by floor pooling).
 //
 // ALU diet (these passes are instruction-bound, not HBM-bound, if written naively):
-//  * LeakyReLU and the BatchNorm affine map are monotonic, so the max-pool arg-max is found on the raw y values
-//    (times sign(scale)), first maximum in (d,h,w) scan order with a strict compare exactly like torch;
+//  * LeakyReLU (slope >= 0) and the BatchNorm affine map are non-decreasing, so the max-pool arg-max is found on the raw
+//    y values times sign(scale) (sign(0) = 0: position 0), first maximum in (d,h,w) scan order with a strict compare.
+//    That position holds the window's maximum activation; it is torch's first maximum wherever the activations are
+//    distinct, and where fp32 rounding makes distinct y give equal activations every kernel that routes max-pool
+//    gradients (the forward's kept ymax, conv1_bwd_fused.cu, conv1_dgrad.cu) picks the same one by the same rule;
 //  * only the arg-max position carries dz for a max pool, so REDUCE touches one position per channel;
 //  * APPLY folds the constant part into one FMA per element:  dy = A + Bc*y (+ scale*dz at the arg-max),
 //    A = scale*(m2*invstd*mean - m1),  Bc = -scale*m2*invstd.
@@ -456,15 +494,10 @@ __global__ void __launch_bounds__(256, 2) bn_maxpool_bwd_reduce_kept_kernel(ActP
 // HMNMX2, first position equal to it with HSET2 (1.0 / 0.0 per half) and two logic ops; the output is
 //   dy = fma(sel, scale*dz, fma(Bc, y, A))      on packed fp32 pairs (FFMA2),  sel in {0, 1}
 // -- the same values as the generic kernel (it stays the reference in the op tests).
-__device__ __forceinline__ uint32_t bf2_max(uint32_t a, uint32_t b) {
-  __nv_bfloat162 r = __hmax2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
-  return *reinterpret_cast<uint32_t*>(&r);
-}
 __device__ __forceinline__ uint32_t bf2_eq(uint32_t a, uint32_t b) {       // 0x3F80 (1.0) per half where equal, else 0
   __nv_bfloat162 r = __heq2(*reinterpret_cast<__nv_bfloat162*>(&a), *reinterpret_cast<__nv_bfloat162*>(&b));
   return *reinterpret_cast<uint32_t*>(&r);
 }
-__device__ __forceinline__ uint32_t u4_get(const uint4& v, int i) { return i == 0 ? v.x : (i == 1 ? v.y : (i == 2 ? v.z : v.w)); }
 
 template <bool FP32>
 __global__ void __launch_bounds__(256, 2) bn_maxpool_bwd_apply_kernel(ActPoolArgs p) {
@@ -649,6 +682,8 @@ int tmf_bn_act_pool_fwd_keepmax(int ng, const void* const* y, const float* const
                                 void* stream) {
   TMF_CHECK_NG(ng);
   ActPoolArgs p{};
+  TMF_REQUIRE(slope >= 0.f, "%s: a max pool routes gradients by y, which needs a LeakyReLU slope >= 0 (got %g)", __func__,
+              (double)slope);
   if (fill_args(p, B, D, H, W, C, TMF_POOL_MAX, slope, out_fp32)) return 1;
   if (!load_group(p.y, (const __nv_bfloat16* const*)y, ng, true, "y") || !load_group(p.coef, coef, ng, true, "coef") ||
       !load_group(p.out, (void* const*)out, ng, true, "out") ||
@@ -679,6 +714,8 @@ int tmf_bn_act_pool_fwd_keepmax_dual(int ng, const void* const* y, const float* 
                                      void* stream) {
   TMF_CHECK_NG(ng);
   ActPoolArgs p{};
+  TMF_REQUIRE(slope >= 0.f, "%s: a max pool routes gradients by y, which needs a LeakyReLU slope >= 0 (got %g)", __func__,
+              (double)slope);
   if (fill_args(p, B, D, H, W, C, TMF_POOL_MAX, slope, 0)) return 1;
   if (!load_group(p.y, (const __nv_bfloat16* const*)y, ng, true, "y") || !load_group(p.coef, coef, ng, true, "coef") ||
       !load_group(p.out, (void* const*)out, ng, true, "out") || !load_group(p.out32, out32, ng, true, "out32") ||
@@ -694,6 +731,8 @@ int tmf_bn_maxpool_bwd_reduce_kept(int ng, const void* const* dout, int dout_fp3
                                    const float* const* coef, double* const* sums, int B, int Do, int Ho, int Wo, int C,
                                    float slope, void* stream) {
   TMF_CHECK_NG(ng);
+  TMF_REQUIRE(slope >= 0.f, "%s: a max pool routes gradients by y, which needs a LeakyReLU slope >= 0 (got %g)", __func__,
+              (double)slope);
   TMF_REQUIRE(C % 8 == 0 && C >= 8 && C <= 1024, "bn_maxpool_bwd_reduce_kept: C must be a multiple of 8 in [8,1024]");
   const int64_t npos = (int64_t)B * Do * Ho * Wo;
   TMF_REQUIRE(npos > 0 && npos * (C / 8) < (1ll << 31), "bn_maxpool_bwd_reduce_kept: bad extent");
@@ -719,6 +758,8 @@ int tmf_bn_act_pool_bwd_reduce(int ng, const void* const* dout, int dout_fp32, c
                                int pool, float slope, void* stream) {
   TMF_CHECK_NG(ng);
   ActPoolArgs p{};
+  TMF_REQUIRE(pool != TMF_POOL_MAX || slope >= 0.f,
+              "%s: a max pool routes gradients by y, which needs a LeakyReLU slope >= 0 (got %g)", __func__, (double)slope);
   if (fill_args(p, B, D, H, W, C, pool, slope, dout_fp32)) return 1;
   if (!load_group(p.y, (const __nv_bfloat16* const*)y, ng, true, "y") || !load_group(p.coef, coef, ng, true, "coef") ||
       !load_group(p.dout, (const void* const*)dout, ng, true, "dout") || !load_group(p.sums, sums, ng, true, "sums"))
@@ -768,6 +809,8 @@ int tmf_bn_act_pool_bwd_apply(int ng, const void* const* dout, int dout_fp32, co
                               int H, int W, int C, int pool, float slope, void* stream) {
   TMF_CHECK_NG(ng);
   ActPoolArgs p{};
+  TMF_REQUIRE(pool != TMF_POOL_MAX || slope >= 0.f,
+              "%s: a max pool routes gradients by y, which needs a LeakyReLU slope >= 0 (got %g)", __func__, (double)slope);
   if (fill_args(p, B, D, H, W, C, pool, slope, dout_fp32)) return 1;
   if (!load_group(p.y, (const __nv_bfloat16* const*)y, ng, true, "y") || !load_group(p.coef, coef, ng, true, "coef") ||
       !load_group(p.bcoef, bcoef, ng, true, "bcoef") ||

@@ -319,7 +319,7 @@ def integrated_gradients(model, inputs, target, n_steps=50, method="gausslegendr
                 or t.conv1._forward_pre_hooks:
             raise ValueError(f"{who}: hooks on an sNet tower or its conv1 block would observe volumes that are never formed "
                              f"(the path points start at layer 1); remove them")
-        if t._hyper()[0][2] < 0:
+        if not t.conv1[2].negative_slope >= 0:          # before sNet._hyper, which refuses any negative slope
             raise ValueError(f"{who}: block 1's LeakyReLU slope must be >= 0 (the pooling winners must not move with alpha)")
     B = inputs[0].shape[0]
     idx = _target_index(target, B, inputs[0].device, who)

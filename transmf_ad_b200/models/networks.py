@@ -69,6 +69,9 @@ class sNet(nn.Module):
             if bn.momentum is None or not bn.track_running_stats or not bn.affine:
                 raise NotImplementedError("sNet on the B200 kernels needs affine BatchNorm3d with running statistics and "
                                           "a numeric momentum (the reference's nn.BatchNorm3d defaults)")
+            if not act.negative_slope >= 0:
+                raise NotImplementedError("sNet on the B200 kernels needs LeakyReLU slopes >= 0: the max pools route gradients "
+                                          f"by the pre-BatchNorm value, which a negative slope reorders (got {act.negative_slope})")
             out.append((float(bn.eps), float(bn.momentum), float(act.negative_slope)))
         return out
 
