@@ -215,7 +215,9 @@ int tmf_linear_dgrad(const float* dy, const float* w, float* dx, int M, int K, i
 /* Scratch buffer of the entry points below that take `ws`: caller-owned, 256-byte aligned, tmf_scratch_bytes() bytes,
  * ZERO-INITIALISED ONCE (its first 16 KB hold "last block" tickets that every kernel leaves zero again); one buffer per
  * stream may be shared by all calls.  It carries split-K / per-block partial sums that the last block to finish adds
- * in index order: the weight gradients of the fusion transformer are bitwise reproducible (no float atomics). */
+ * in index order: the weight gradients of the fusion transformer are bitwise reproducible (no float atomics).  Each kernel
+ * family owns its own ticket words (LayerNorm, split-K GEMM tiles, column sums, encoder; csrc/common.cuh): the column sums
+ * are capped below the encoder's range, so tmf_linear_wgrad with a bias takes N <= 26496. */
 int64_t tmf_scratch_bytes(void);
 /* dw[N,K] = dy^T . x ; dbias[N] = column sums of dy (dbias may be NULL); both overwritten */
 int tmf_linear_wgrad(const float* dy, const float* x, float* dw, float* dbias, int M, int K, int N, void* ws,

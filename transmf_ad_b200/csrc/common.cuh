@@ -127,8 +127,15 @@ __device__ __forceinline__ bool last_block_arrives(unsigned* ticket, unsigned nb
 
 // Layout of the caller-owned scratch buffer (`ws`) of the fusion-transformer entry points: tickets first (zero before the
 // first use, left zero by every kernel), then partial results.  tmf_scratch_bytes() is the size callers allocate.
-constexpr size_t TMF_WS_TICKET_BYTES = 16384;                 // 4096 tickets: [0,1024) LayerNorm, [1024,3072) GEMM tiles, [3072,4096) column sums
+constexpr size_t TMF_WS_TICKET_BYTES = 16384;                 // 4096 tickets
 constexpr size_t TMF_WS_BYTES = (size_t)16 << 20;
+// Ticket words [first, first + count) of each user.  The ranges are disjoint, so no two kernels ever share a ticket even if
+// calls on one buffer were not stream-ordered (tests/test_fusion_exact_host.py checks it): the column sums of
+// tmf_linear_wgrad are capped at TK_COLSUM_N column blocks (N <= 32 * 828) so that the encoder keeps the top words.
+constexpr unsigned TK_LN = 0, TK_LN_N = 1024;                 // tmf_layernorm_bwd (uses word 0)
+constexpr unsigned TK_GEMM = 1024, TK_GEMM_N = 2048;          // split-K GEMM tiles of tmf_linear_wgrad
+constexpr unsigned TK_COLSUM = 3072, TK_COLSUM_N = 828;       // column blocks of tmf_linear_wgrad's bias sums
+constexpr unsigned TK_ENC = 3900, TK_ENC_N = 3 * 64;          // encoder: chain_bwd, proj_bwd (one word each), wgrad (64 tiles)
 
 // Packed fp32 pairs in one 64-bit register (sm_100: FADD2 / FFMA2 issue two fp32 operations per slot).
 __device__ __forceinline__ uint64_t pair_u32(uint32_t lo, uint32_t hi) {

@@ -903,9 +903,9 @@ static int enc_check_ws(const char* who, void* ws, size_t ws_bytes) {
               "%s: needs the 256-byte aligned scratch buffer of tmf_scratch_bytes() bytes (tickets zero-initialised)", who);
   return 0;
 }
-// ticket slots of the encoder kernels inside the scratch buffer's ticket area (fusion_ops.cu uses [0, 4096) x 4 bytes of
-// the 16 KB; here: the upper words)
-static unsigned* enc_tickets(void* ws, int which) { return reinterpret_cast<unsigned*>(ws) + 3900 + which * 64; }
+// ticket slots of the encoder kernels inside the scratch buffer's ticket area: [TK_ENC, TK_ENC + TK_ENC_N) (common.cuh), 64
+// words per kernel
+static unsigned* enc_tickets(void* ws, int which) { return reinterpret_cast<unsigned*>(ws) + TK_ENC + which * 64; }
 static float* enc_partials(void* ws) { return reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + TMF_WS_TICKET_BYTES); }
 
 extern "C" {
@@ -1043,7 +1043,7 @@ int tmf_encoder_wgrad(const void* const* t, const float* f, float* dw2, float* d
   }
   p.ntiles = tiles;
   p.nsplit = ceil_div(Mx > Mc ? Mx : Mc, WG_MC);
-  TMF_REQUIRE(tiles <= 64, "encoder_wgrad: too many tiles");
+  TMF_REQUIRE(tiles <= (int)TK_ENC_N / 3, "encoder_wgrad: too many tiles");
   TMF_REQUIRE((size_t)tiles * p.nsplit * (32 * 128 + 32) * sizeof(float) <= TMF_WS_BYTES - TMF_WS_TICKET_BYTES,
               "encoder_wgrad: token count too large for the scratch buffer");
   p.part = enc_partials(ws);

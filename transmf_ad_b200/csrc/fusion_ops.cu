@@ -788,11 +788,11 @@ int tmf_linear_wgrad(const float* dy, const float* x, float* dw, float* dbias, i
     // split-K partial tiles meet in the scratch buffer; the last split of a tile adds them in order (deterministic)
     const int splits = ceil_div(M, p.kchunk);
     const int tiles = gemm_ksplit_eligible(p) ? ceil_div(N, V_TM) * ceil_div(K, V_TN) : ceil_div(N, G_TM) * ceil_div(K, G_TN);
-    if (tiles > 2048 || (size_t)splits * N * K > part_floats) {
+    if (tiles > (int)TK_GEMM_N || (size_t)splits * N * K > part_floats) {
       p.kchunk = 0;                      // too large for the scratch buffer: one CTA per tile walks the whole reduction
     } else {
       p.part = partials;
-      p.tickets = tickets + 1024;
+      p.tickets = tickets + TK_GEMM;
     }
   }
   if (launch_gemm(p, st)) return 3;
@@ -800,9 +800,9 @@ int tmf_linear_wgrad(const float* dy, const float* x, float* dw, float* dbias, i
     int rows = 128;
     while ((size_t)ceil_div(M, rows) * N > part_floats) rows *= 2;
     dim3 grid(ceil_div(N, 32), ceil_div(M, rows), 1);
-    TMF_REQUIRE(grid.x <= 1024, "linear_wgrad: N=%d too wide for the column-sum tickets", N);
+    TMF_REQUIRE(grid.x <= TK_COLSUM_N, "linear_wgrad: N=%d too wide for the column-sum tickets", N);
     // (runs after the GEMM in stream order, so it may reuse the partial area)
-    launch_k(colsum_kernel, grid, 256, 0, st, dy, dbias, M, N, rows, partials, tickets + 3072);
+    launch_k(colsum_kernel, grid, 256, 0, st, dy, dbias, M, N, rows, partials, tickets + TK_COLSUM);
     TMF_LAUNCH_CHECK();
   }
   return 0;
@@ -829,7 +829,7 @@ int tmf_layernorm_bwd(const float* dy, const float* x, const float* gamma, const
   const int grid = max(1, min(ceil_div(rows, 8 * 4), 148));
   launch_k(layernorm_bwd_kernel, grid, 256, 2 * dim * sizeof(float), (cudaStream_t)stream, 
       dy, x, gamma, mean, rstd, dx, dgamma, dbeta, rows, dim, accumulate,
-      reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + TMF_WS_TICKET_BYTES), reinterpret_cast<unsigned*>(ws));
+      reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + TMF_WS_TICKET_BYTES), reinterpret_cast<unsigned*>(ws) + TK_LN);
   TMF_LAUNCH_CHECK();
   return 0;
 }
