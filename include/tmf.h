@@ -401,6 +401,23 @@ int tmf_abl_input(int ng, const float* const* x, const int* mask, int mask_per_s
 int tmf_abl_map(int ng, const float* const* scores, const int* mask, int mask_per_sample, int F, float* const* map, int B,
                 int D, int H, int W, void* stream);
 
+/* ---- Shapley value sampling over the regions of a mask through the sNet towers (DESIGN section 3.13) -----------------------
+ * One pass row n per chain (a permutation's walk from the baseline to x), rows n*B + b; tab as for tmf_abl_input (the
+ * BoxPlan rows of the region each row adds); mask and baselines as for tmf_abl_input, with every mask id in [0, F).  Every
+ * element written once, no atomics, 64-bit offsets.
+ * tmf_shap_input: out[g] fp32 [m*B][Dc][Hc][Wc] = x[g][b] at crop origin + (x, y, z) where rank[perm[n]][id] <= step[n] for
+ * the voxel's mask id (rank: device int32 [P][F], perm / step: device int32 [m]), else the baseline.
+ * tmf_shap_compose: out[g] as for tmf_occ_compose with crop[g] != NULL, except that the base of row n*B + b is
+ * state[g][sidx[n]][b] (state [S][B][D][H][W][C], sidx device int32 [m], distinct, in [0, S)); the same kernel writes out's
+ * values inside [lo, hi) back into state[g][sidx[n]][b]. */
+int tmf_shap_input(int ng, const float* const* x, const int* mask, int mask_per_sample, const float* const* bvol,
+                   const float* bval, int bvol_per_sample, const int* tab, const int* rank, int F, const int* perm,
+                   const int* step, int m, float* const* out, int B, int D, int H, int W, int Dc, int Hc, int Wc,
+                   void* stream);
+int tmf_shap_compose(int ng, void* const* state, const int* sidx, const void* const* crop, const int* tab, int m,
+                     void* const* out, int B, int D, int H, int W, int Dc, int Hc, int Wc, int Dp, int Hp, int Wp, int C,
+                     int fp32, void* stream);
+
 /* ---- attention maps of the fusion transformer (DESIGN section 3.8) ------------------------------------------------------
  * tmf_attn_scores: per-head product of the attention core's operands (q / kv as for tmf_attn_fwd; dh in {16, 32, 64}, any
  * Nq, Nk), written out as fp32 [B, heads, Nq, Nk]:

@@ -51,6 +51,8 @@ SIGNATURES = {
     "tmf_occ_map": [_i, _pp, _pp] + [_i] * 13 + [_vp],
     "tmf_abl_input": [_i, _pp, _vp, _i, _pp, C.POINTER(C.c_float), _i, _vp, _vp, _i, _pp] + [_i] * 7 + [_vp],
     "tmf_abl_map": [_i, _pp, _vp, _i, _i, _pp, _i, _i, _i, _i, _vp],
+    "tmf_shap_input": [_i, _pp, _vp, _i, _pp, C.POINTER(C.c_float), _i, _vp, _vp, _i, _vp, _vp, _i, _pp] + [_i] * 7 + [_vp],
+    "tmf_shap_compose": [_i, _pp, _vp, _pp, _vp, _i, _pp] + [_i] * 12 + [_vp],
     "tmf_attn_scores": [_i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _vp],
     "tmf_attn_relevance": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp],
     "tmf_bn_maxpool_bwd_reduce_kept": [_i, _pp, _i, _pp, _pp, _pp, _i, _i, _i, _i, _i, _f, _vp],

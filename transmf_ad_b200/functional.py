@@ -1531,3 +1531,83 @@ def abl_map(scores, mask):
         L.call("tmf_abl_map", len(scores[i:i + 2]), L.ptrs(scores[i:i + 2]), L.ptr(mask), int(mask.shape[0] > 1), F,
                L.ptrs(maps[i:i + 2]), B, *dims)
     return maps
+
+
+# ==============================================================================================================
+# Shapley value sampling over regions of a mask, with per-chain state   (csrc/shapley.cu; DESIGN section 3.13)
+# ==============================================================================================================
+# Bytes of chain state (per chain: every tower's kept layer 1-6 inputs and its tower output, for all B samples) one group of
+# permutations may hold; a call runs its permutations in groups that fit.  The chains are independent, so the grouping
+# changes the memory and never a bit of the result.
+SHAP_STATE_BYTES = 8 << 30
+
+
+def shap_permutations(ids, n_samples):
+    """``n_samples`` orders of the players ``ids`` (int64 numpy [F']): int64 (n_samples, F'), one ``torch.randperm(F')`` per
+    row from torch's global CPU generator, as captum's ``ShapleyValueSampling`` draws them."""
+    ids = torch.as_tensor(ids, dtype=torch.int64)
+    return torch.stack([ids[torch.randperm(len(ids))] for _ in range(n_samples)])
+
+
+def shap_schedule(perms, cls_of, caps):
+    """Passes of the chains of ``perms`` (int numpy [P, F'], region ids): a pass takes chains whose next region is in one extent
+    class -- the class with the most waiting chains, the smaller class index (``abl_classes`` order) on a tie -- in ascending
+    chain order, at most ``caps[class]`` of them.  cls_of: {id: class index}.  Returns [(class, [(p, k)])]: every (p, k) once,
+    each chain's steps in order, a chain at most once per pass.  Host only; depends on the permutations alone."""
+    P, Fp = perms.shape
+    nxt = [0] * P
+    left = P * Fp
+    passes = []
+    while left:
+        waiting = {}
+        for p in range(P):
+            if nxt[p] < Fp:
+                waiting.setdefault(cls_of[int(perms[p, nxt[p]])], []).append(p)
+        c = min(waiting, key=lambda c: (-len(waiting[c]), c))
+        chains = waiting[c][:caps[c]]
+        passes.append((c, [(p, nxt[p]) for p in chains]))
+        for p in chains:
+            nxt[p] += 1
+        left -= len(chains)
+    return passes
+
+
+def shap_input(xs, mask, baselines, tab, rank, perm, step, m, extent):
+    """fp32 (m*B, 1, Dc, Hc, Wc) layer-0 crops per tower (``tmf_shap_input``): x where the voxel's region comes at or before
+    the row's step in the row's permutation, else the baseline.  xs, mask and baselines as for ``abl_input``; rank: int32
+    contiguous (P, F); perm, step: int32 [m]."""
+    import ctypes
+    B, _, D, H, W = xs[0].shape
+    out = [torch.empty((m * B, 1) + tuple(extent), dtype=torch.float32, device=xs[0].device) for _ in xs]
+    vols = [b if torch.is_tensor(b) else None for b in baselines]
+    vals = (ctypes.c_float * len(xs))(*[0.0 if torch.is_tensor(b) else float(b) for b in baselines])
+    per = sum(1 << g for g, v in enumerate(vols) if v is not None and v.shape[0] > 1)
+    L.call("tmf_shap_input", len(xs), L.ptrs(xs), L.ptr(mask), int(mask.shape[0] > 1), L.ptrs(vols), vals, per, L.ptr(tab),
+           L.ptr(rank), rank.shape[1], L.ptr(perm), L.ptr(step), m, L.ptrs(out), B, D, H, W, *extent)
+    return out
+
+
+def shap_compose(state, sidx, crops, tab, m, extent, out=None, tag=None):
+    """Input crops (m*B, Dc, Hc, Wc, C) per tower (``tmf_shap_compose``), composed as ``occ_compose`` composes them but from the
+    rows' chain states, whose changed region is then overwritten with the crops'.  state: (S*B, D, H, W, C) contiguous, bf16 or
+    fp32, per tower; sidx: int32 [m], distinct chain indices; crops: the previous layer's recomputed outputs."""
+    C = state[0].shape[-1]
+    D, H, W = state[0].shape[1:4]
+    B = crops[0].shape[0] // m
+    if out is None:
+        out = [torch.empty((m * B,) + tuple(extent) + (C,), dtype=state[0].dtype, device=state[0].device) for _ in state]
+    L.call("tmf_shap_compose", len(state), L.ptrs(state), L.ptr(sidx), L.ptrs(crops), L.ptr(tab), m, L.ptrs(out), B, D, H,
+           W, *extent, *crops[0].shape[1:4], C, int(state[0].dtype == torch.float32), tag=tag)
+    return out
+
+
+def shap_crops(spec, hyper, folds, act, state, plan, tabs, sidx, m, out):
+    """One step of m chains through one or two towers of the same shape, as ``occ_crops`` runs a pass, with the chain states in
+    place of the base activations: state[t][l] (l = 1 .. 6: the kept layer input, 7: the fp32 tower output), (S*B, ...) per
+    tower; the composed tower outputs go to ``out`` and every state holds the step's result afterwards."""
+    impl = conv_impl()
+    for l in range(len(spec.layers)):
+        if l > 0:
+            act = shap_compose([s[l] for s in state], sidx, act, tabs[l], m, plan.crop[l], tag=f"tmf_shap_compose@L{l}")
+        act = occ_layer(l, spec, hyper, [f[l] for f in folds], act, plan.crop[l], impl)
+    return shap_compose([s[-1] for s in state], sidx, act, tabs[-1], m, plan.crop[-1], out=out, tag="tmf_shap_compose@out")

@@ -1,7 +1,7 @@
 """Interpretability: Grad-CAM (Selvaraju et al., 2017) on a block of every sNet tower of a model, layer-wise relevance
 propagation (Bach et al., 2015), integrated gradients (Sundararajan et al., 2017), occlusion sensitivity (Zeiler & Fergus,
-2014) and feature ablation over the regions of a mask through the towers, and head-averaged or gradient-weighted (Chefer
-et al., 2021) cross-modal attention maps of the fusion transformer.
+2014), feature ablation and Shapley value sampling (Castro et al., 2009) over the regions of a mask through the towers, and
+head-averaged or gradient-weighted (Chefer et al., 2021) cross-modal attention maps of the fusion transformer.
 
 Input gradients (saliency maps) need nothing from here: ``mri.requires_grad_(True)`` and plain autograd work on every model
 (INTEGRATION.md section 3b).  Module hooks on the sNet blocks work as on the reference modules (section 3c), and so do
@@ -579,27 +579,9 @@ def _ablation_baselines(baselines, nt, shape, device, who):
     return out
 
 
-def feature_ablation(model, inputs, target, feature_mask, baselines=0.0, joint=False, internal_batch_size=None):
-    """Feature ablation over the regions of ``feature_mask`` through every sNet tower of ``model`` (eval mode), for the
-    objective f = ``logits[b, target_b]`` of the model's first output (captum's ``FeatureAblation`` with a feature mask).
-
-    ``feature_mask``: an integer tensor (1|B, 1, D, H, W) on the inputs' device; every id present, 0 included, is one feature,
-    and ids must be >= 0.  It applies to every tower's input (the modalities are co-registered); a per-sample mask ablates
-    each sample's own region.  ``baselines``: a finite Python scalar, or a tuple of one entry per tower, each a finite scalar
-    or an fp32 CUDA tensor (1|B, 1, D, H, W); inside the feature the voxels take the baseline's value.  ``joint``: False
-    ablates a feature in one tower's input at a time; True ablates it in every tower's input at once (captum's
-    ``enable_cross_tensor_attribution``).  ``inputs``, ``target`` and ``internal_batch_size`` (volumes per pass) as for
-    ``occlusion``.
-
-    Returns ``FeatureAblation(maps, scores)``, per tower in tower order: ``scores`` fp32 (B, F), F = max id + 1, f(x) - f(x
-    with feature j ablated) (0 for an id absent from the mask; with ``joint`` every tower has the same scores); ``maps`` fp32
-    (B,1,D,H,W), each voxel holding its feature's score.
-
-    The ablated towers are not run in full (DESIGN section 3.12): as in ``occlusion``, each feature recomputes only what its
-    bounding box changes, on crops of one extent per extent class of features, and the composed tower outputs go through
-    the model's own fusion stack and heads.  No parameter receives a ``.grad``, no weight-gradient kernel runs, BatchNorm
-    buffers and the module mode are untouched and ``requires_grad`` flags are restored."""
-    who = "feature_ablation"
+def _region_args(model, inputs, target, feature_mask, baselines, joint, internal_batch_size, who):
+    """The argument checks of ``feature_ablation`` and ``shapley_sampling``, in order, before any launch.  Returns the towers,
+    the per-tower baselines, the (B,) target rows, the int32 contiguous mask, F = max id + 1 and the fp32 inputs."""
     if not isinstance(joint, bool):
         raise ValueError(f"{who}: joint must be True or False; got {joint!r}")
     if internal_batch_size is not None and not _is_count(internal_batch_size):
@@ -634,6 +616,33 @@ def feature_ablation(model, inputs, target, feature_mask, baselines=0.0, joint=F
     F = hi + 1
     mask = mask.to(torch.int32).contiguous()
     xs = [TF._f32c(x.detach()) for x in inputs]
+    return towers, bls, idx, mask, F, xs
+
+
+def feature_ablation(model, inputs, target, feature_mask, baselines=0.0, joint=False, internal_batch_size=None):
+    """Feature ablation over the regions of ``feature_mask`` through every sNet tower of ``model`` (eval mode), for the
+    objective f = ``logits[b, target_b]`` of the model's first output (captum's ``FeatureAblation`` with a feature mask).
+
+    ``feature_mask``: an integer tensor (1|B, 1, D, H, W) on the inputs' device; every id present, 0 included, is one feature,
+    and ids must be >= 0.  It applies to every tower's input (the modalities are co-registered); a per-sample mask ablates
+    each sample's own region.  ``baselines``: a finite Python scalar, or a tuple of one entry per tower, each a finite scalar
+    or an fp32 CUDA tensor (1|B, 1, D, H, W); inside the feature the voxels take the baseline's value.  ``joint``: False
+    ablates a feature in one tower's input at a time; True ablates it in every tower's input at once (captum's
+    ``enable_cross_tensor_attribution``).  ``inputs``, ``target`` and ``internal_batch_size`` (volumes per pass) as for
+    ``occlusion``.
+
+    Returns ``FeatureAblation(maps, scores)``, per tower in tower order: ``scores`` fp32 (B, F), F = max id + 1, f(x) - f(x
+    with feature j ablated) (0 for an id absent from the mask; with ``joint`` every tower has the same scores); ``maps`` fp32
+    (B,1,D,H,W), each voxel holding its feature's score.
+
+    The ablated towers are not run in full (DESIGN section 3.12): as in ``occlusion``, each feature recomputes only what its
+    bounding box changes, on crops of one extent per extent class of features, and the composed tower outputs go through
+    the model's own fusion stack and heads.  No parameter receives a ``.grad``, no weight-gradient kernel runs, BatchNorm
+    buffers and the module mode are untouched and ``requires_grad`` flags are restored."""
+    who = "feature_ablation"
+    towers, bls, idx, mask, F, xs = _region_args(model, inputs, target, feature_mask, baselines, joint,
+                                                 internal_batch_size, who)
+    B, dims, dev = xs[0].shape[0], tuple(xs[0].shape[2:]), xs[0].device
     spec = towers[0]._spec
     layers = [(ks, pool) for _, _, ks, pool in spec.layers]
     boxes = TF.abl_boxes(mask, F)
@@ -678,3 +687,125 @@ def feature_ablation(model, inputs, target, feature_mask, baselines=0.0, joint=F
     if joint:
         per += [per[0].clone() for _ in range(nt - 1)]
     return FeatureAblation(TF.abl_map(per, mask), per)
+
+
+ShapleySampling = namedtuple("ShapleySampling", ["maps", "scores", "delta", "permutations"])
+
+
+def shapley_sampling(model, inputs, target, feature_mask, baselines=0.0, joint=False, n_samples=25,
+                     internal_batch_size=None):
+    """Shapley value sampling (Castro, Gomez & Tejada, 2009; Strumbelj & Kononenko, 2014) over the regions of
+    ``feature_mask`` through every sNet tower of ``model`` (eval mode), for the objective f = ``logits[b, target_b]`` of the
+    model's first output (captum's ``ShapleyValueSampling`` with a feature mask).
+
+    The players are the ids present in the mask, 0 included.  ``n_samples`` permutations of them are drawn with
+    ``torch.randperm`` from torch's global CPU generator, one per sample draw, shared by all B samples and every tower.  A
+    chain walks one permutation from the start state -- the baseline everywhere in the ablated input(s) -- to x: step k sets
+    the voxels of region pi[k] to x, and its marginal contribution is f(after) - f(before); a region's score is the mean of its
+    contributions over the permutations (positive: the region's real values raise the target logit).  ``joint``: False plays
+    one game per tower (only tower t's input walks, the others see x); True plays one game in which a region enters every
+    tower's input at once, and every tower reports its scores.  ``inputs``, ``target``, ``feature_mask``, ``baselines`` and
+    ``internal_batch_size`` (volumes per pass; it changes the speed only, never the bits) as for ``feature_ablation``.
+
+    Returns ``ShapleySampling(maps, scores, delta, permutations)``, per tower in tower order: ``scores`` fp32 (B, F), F = max
+    id + 1 (0 for an id absent from the mask); ``maps`` fp32 (B,1,D,H,W), each voxel holding its region's score; ``delta`` fp32
+    (B,), sum_j scores[:, j] - (f(x) - f(start)).  The contributions of a chain telescope, so delta is only the rounding of
+    the recomputation, never sampling error.  ``permutations``: int64 (n_samples, F'), the orders of the F' present ids used.
+
+    The towers are not run per step (DESIGN section 3.13): each chain keeps its own copy of every layer's input activation,
+    and a step recomputes only the added region's bounding box on the crops of ``feature_ablation``, writing the result back
+    into the chain's copy.  No parameter receives a ``.grad``, no weight-gradient kernel runs, BatchNorm buffers and the
+    module mode are untouched and ``requires_grad`` flags are restored."""
+    import numpy as np
+    who = "shapley_sampling"
+    if not _is_count(n_samples):
+        raise ValueError(f"{who}: n_samples must be an integer >= 1; got {n_samples!r}")
+    towers, bls, idx, mask, F, xs = _region_args(model, inputs, target, feature_mask, baselines, joint,
+                                                 internal_batch_size, who)
+    B, dims, dev = xs[0].shape[0], tuple(xs[0].shape[2:]), xs[0].device
+    spec = towers[0]._spec
+    layers = [(ks, pool) for _, _, ks, pool in spec.layers]
+    boxes = TF.abl_boxes(mask, F)
+    classes = TF.abl_classes(boxes, dims)
+    plans = [TF.abl_plan(boxes, ids, dims, layers) for _, ids in classes]
+    cls_of = {f: c for c, (_, ids) in enumerate(classes) for f in ids}
+    row_of = {f: n for plan in plans for n, f in enumerate(plan.ids.tolist())}
+    players = np.array(sorted(cls_of), dtype=np.int64)
+    perms = TF.shap_permutations(players, n_samples)
+    P, Fp = perms.shape
+    pn = perms.numpy()
+    rank = np.full((P, F), np.iinfo(np.int32).max, dtype=np.int32)
+    rank[np.arange(P)[:, None], pn] = np.arange(Fp, dtype=np.int32)
+    groups = _tower_groups(towers)
+    nt = len(towers)
+    blocks = 1 if joint else nt
+    chunk = P if internal_batch_size is None else max(1, internal_batch_size // B)
+    caps = [min([chunk] + [TF.occ_pass_limit(plan, towers[g[0]]._spec, B, len(g)) for g in groups]) for plan in plans]
+
+    flags = [(p, p.requires_grad) for p in model.parameters()]
+    try:
+        for p, _ in flags:
+            p.requires_grad_(False)
+        f_x, _, base = _base_forward(model, towers, xs, idx, who)
+        starts = [torch.full_like(x, b) if not torch.is_tensor(b) else b.expand_as(x).contiguous() for x, b in zip(xs, bls)]
+        _, kept, start_out = _base_forward(model, towers, starts, idx, who)
+        # f(start) through the fusion stack as the passes run it: block u holds tower u's start output (joint: every tower's)
+        zero_tab = torch.zeros((1, 3, 4), dtype=torch.int32, device=dev)
+        bufs = [torch.empty((blocks * B,) + tuple(b.shape[1:]), dtype=torch.float32, device=dev) for b in base]
+        for t in range(nt):
+            bufs[t][(0 if joint else t) * B:((0 if joint else t) + 1) * B].copy_(start_out[t])
+        f_start = _through_fusion(model, towers, xs, base, bufs, zero_tab, 1, tuple(base[0].shape[1:4]), idx, blocks)[:, 0]
+        # f along every chain: fv[:, p, k] after step k - 1 of chain p (k = 0: the start state)
+        fv = torch.empty((blocks, P, Fp + 1, B), dtype=torch.float32, device=dev)
+        fv[:, :, 0] = f_start.unsqueeze(1)
+        per_chain = sum(sum(k[l][0].nbytes for l in range(1, len(k))) + o.nbytes for k, o in zip(kept, start_out))
+        Pg = max(1, min(P, TF.SHAP_STATE_BYTES // per_chain))
+        rank_d = torch.from_numpy(rank).to(dev)                                # ordinary host-to-device copies
+        chain, region = torch.arange(P).repeat_interleave(Fp).to(dev), perms.reshape(-1).to(dev)
+        for p0 in range(0, P, Pg):
+            S = min(Pg, P - p0)
+            # every chain starts from the start state: (S*B, ...) copies of the kept layer inputs and the tower output
+            state = [[None] + [a.repeat((S,) + (1,) * (a.dim() - 1)) for a in [kl[0] for kl in k[1:]] + [o]]
+                     for k, o in zip(kept, start_out)]
+            passes = TF.shap_schedule(pn[p0:p0 + S], cls_of, caps)
+            rows = [(c, p, k) for c, steps in passes for p, k in steps]
+            n_at = [row_of[int(pn[p0 + p, k])] for _, p, k in rows]
+            tab_all = [torch.from_numpy(np.stack([plans[c].tab[l][n] for (c, _, _), n in zip(rows, n_at)])).to(dev)
+                       for l in range(len(layers) + 1)]
+            meta = torch.from_numpy(np.array([[p0 + p, k, p] for _, p, k in rows], dtype=np.int32).T.copy()).to(dev)
+            at_all = torch.tensor([(p0 + p) * (Fp + 1) + k + 1 for _, p, k in rows], dtype=torch.int64).to(dev)
+            r0 = 0
+            for c, steps in passes:
+                m, plan = len(steps), plans[c]
+                assert len({p for p, _ in steps}) == m                           # a chain at most once per pass
+                perm, step, sidx = (v[r0:r0 + m] for v in meta)
+                tab = [tb[r0:r0 + m] for tb in tab_all]
+                bufs = [torch.empty((blocks * m * B,) + plan.crop[-1] + (b.shape[-1],), dtype=torch.float32, device=dev)
+                        for b in base]
+                for grp in groups:
+                    act = TF.shap_input([xs[t] for t in grp], mask, [bls[t] for t in grp], tab[0], rank_d, perm, step, m,
+                                        plan.crop[0])
+                    TF.shap_crops(towers[grp[0]]._spec, towers[grp[0]]._hyper(), [towers[t]._folds for t in grp], act,
+                                  [state[t] for t in grp], plan, tab, sidx, m,
+                                  [bufs[t][(0 if joint else t) * m * B:((0 if joint else t) + 1) * m * B] for t in grp])
+                f_new = _through_fusion(model, towers, xs, base, bufs, tab[-1], m, plan.crop[-1], idx, blocks)
+                fv.view(blocks, P * (Fp + 1), B)[:, at_all[r0:r0 + m]] = f_new
+                r0 += m
+            del state
+    finally:
+        for p, f in flags:
+            p.requires_grad_(f)
+        for t in towers:
+            t._lrp_keep = None
+            t._occ_out = None
+    contrib = torch.zeros((blocks, P, F, B), dtype=torch.float32, device=dev)
+    contrib[:, chain, region] = (fv[:, :, 1:] - fv[:, :, :-1]).reshape(blocks, P * Fp, B)
+    total = contrib[:, 0].clone()
+    for p in range(1, P):                                                     # a fixed order, whatever the grouping
+        total += contrib[:, p]
+    scores = [s.t().contiguous() for s in (total / P).unbind(0)]
+    delta = [s.sum(1) - (f_x - fs) for s, fs in zip(scores, f_start.unbind(0))]
+    if joint:
+        scores += [scores[0].clone() for _ in range(nt - 1)]
+        delta += [delta[0].clone() for _ in range(nt - 1)]
+    return ShapleySampling(TF.abl_map(scores, mask), scores, delta, perms)
