@@ -380,6 +380,7 @@ int tmf_line_conv_wgrad(const float* dy, const float* x, float* dw, float* db, i
   const int nb = (int)(lines < 592 ? lines : 592);
   const int nw = LC_CO * Cin * k;
   const size_t smem = sizeof(float) * ((size_t)LC_CO * (L - k + 1) + (size_t)Cin * L);
+  TMF_REQUIRE(smem <= 48 * 1024, "line_conv_wgrad: line too long");
   cudaStream_t st = (cudaStream_t)stream;
   line_conv_wgrad_kernel<<<nb, 256, smem, st>>>(dy, x, (float*)ws, N, Cin, P, L, k);
   TMF_LAUNCH_CHECK();
@@ -390,7 +391,8 @@ int tmf_line_conv_wgrad(const float* dy, const float* x, float* dw, float* db, i
 
 int tmf_conv2d_fwd(const float* x, const float* w, const float* b, float* y, int N, int Cin, int X, int Y, int Cout, int kh, int kw,
                    int stride, void* stream) {
-  TMF_REQUIRE(x && w && b && y && stride >= 1 && X >= kh && Y >= kw, "conv2d_fwd: bad arguments");
+  TMF_REQUIRE(x && w && b && y && N >= 1 && Cin >= 1 && Cout >= 1 && kh >= 1 && kw >= 1 && stride >= 1 && X >= kh && Y >= kw,
+              "conv2d_fwd: bad arguments");
   const int Xo = (X - kh) / stride + 1, Yo = (Y - kw) / stride + 1;
   conv2d_fwd_kernel<<<grid_for((int64_t)N * Cout * Xo * Yo), 256, 0, (cudaStream_t)stream>>>(x, w, b, y, N, Cin, X, Y, Cout, kh, kw, stride, Xo, Yo);
   TMF_LAUNCH_CHECK();
@@ -399,7 +401,8 @@ int tmf_conv2d_fwd(const float* x, const float* w, const float* b, float* y, int
 
 int tmf_conv2d_dgrad(const float* dy, const float* w, float* dx, int N, int Cin, int X, int Y, int Cout, int kh, int kw, int stride,
                      void* stream) {
-  TMF_REQUIRE(dy && w && dx && stride >= 1 && X >= kh && Y >= kw, "conv2d_dgrad: bad arguments");
+  TMF_REQUIRE(dy && w && dx && N >= 1 && Cin >= 1 && Cout >= 1 && kh >= 1 && kw >= 1 && stride >= 1 && X >= kh && Y >= kw,
+              "conv2d_dgrad: bad arguments");
   const int Xo = (X - kh) / stride + 1, Yo = (Y - kw) / stride + 1;
   conv2d_dgrad_kernel<<<grid_for((int64_t)N * Cin * X * Y), 256, 0, (cudaStream_t)stream>>>(dy, w, dx, N, Cin, X, Y, Cout, kh, kw, stride, Xo, Yo);
   TMF_LAUNCH_CHECK();
@@ -408,7 +411,8 @@ int tmf_conv2d_dgrad(const float* dy, const float* w, float* dx, int N, int Cin,
 
 int tmf_conv2d_wgrad(const float* dy, const float* x, float* dw, float* db, int N, int Cin, int X, int Y, int Cout, int kh, int kw,
                      int stride, void* stream) {
-  TMF_REQUIRE(dy && x && dw && stride >= 1 && X >= kh && Y >= kw, "conv2d_wgrad: bad arguments");
+  TMF_REQUIRE(dy && x && dw && N >= 1 && Cin >= 1 && Cout >= 1 && kh >= 1 && kw >= 1 && stride >= 1 && X >= kh && Y >= kw,
+              "conv2d_wgrad: bad arguments");
   const int Xo = (X - kh) / stride + 1, Yo = (Y - kw) / stride + 1;
   const int64_t nwt = (int64_t)Cout * Cin * kh * kw;
   conv2d_wgrad_kernel<<<ceil_div(nwt * 32, 256), 256, 0, (cudaStream_t)stream>>>(dy, x, dw, db, N, Cin, X, Y, Cout, kh, kw, stride, Xo, Yo);
@@ -428,6 +432,7 @@ int tmf_nchw_bn_stats(const float* x, double* rows, int N, int C, int64_t S, voi
 
 int tmf_nchw_bn_relu_fwd(const float* x, const float* coef, float* out, int N, int C, int64_t S, void* stream) {
   TMF_REQUIRE(x && coef && out, "nchw_bn_relu_fwd: NULL pointer");
+  TMF_REQUIRE(N > 0 && C > 0 && S > 0, "nchw_bn_relu_fwd: empty tensor");
   const int64_t total = (int64_t)N * C * S;
   nchw_bn_relu_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(x, coef, out, C, S, total);
   TMF_LAUNCH_CHECK();
@@ -436,6 +441,7 @@ int tmf_nchw_bn_relu_fwd(const float* x, const float* coef, float* out, int N, i
 
 int tmf_nchw_bn_relu_bwd_reduce(const float* dout, const float* x, const float* coef, double* rows, int N, int C, int64_t S, void* stream) {
   TMF_REQUIRE(dout && x && coef && rows, "nchw_bn_relu_bwd_reduce: NULL pointer");
+  TMF_REQUIRE(N > 0 && C > 0 && S > 0, "nchw_bn_relu_bwd_reduce: empty tensor");
   int bx = (int)(((int64_t)N * S + 256 * 8 - 1) / (256 * 8));
   if (bx > TMF_STAT_ROWS) bx = TMF_STAT_ROWS;
   if (bx < 1) bx = 1;
@@ -447,6 +453,7 @@ int tmf_nchw_bn_relu_bwd_reduce(const float* dout, const float* x, const float* 
 int tmf_nchw_bn_relu_bwd_apply(const float* dout, const float* x, const float* coef, const float* bcoef, float* dx, int N, int C,
                                int64_t S, void* stream) {
   TMF_REQUIRE(dout && x && coef && bcoef && dx, "nchw_bn_relu_bwd_apply: NULL pointer");
+  TMF_REQUIRE(N > 0 && C > 0 && S > 0, "nchw_bn_relu_bwd_apply: empty tensor");
   const int64_t total = (int64_t)N * C * S;
   nchw_bn_relu_bwd_apply_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(dout, x, coef, bcoef, dx, C, S, total);
   TMF_LAUNCH_CHECK();
@@ -462,7 +469,7 @@ int tmf_maxpool2d_fwd(const float* x, float* y, void* idx, int64_t NC, int X, in
 }
 
 int tmf_maxpool2d_bwd(const float* dy, const void* idx, float* dx, int64_t NC, int X, int Y, int ph, int pw, void* stream) {
-  TMF_REQUIRE(dy && idx && dx && ph >= 1 && pw >= 1 && X >= ph && Y >= pw, "maxpool2d_bwd: bad arguments");
+  TMF_REQUIRE(dy && idx && dx && ph >= 1 && pw >= 1 && ph * pw <= 255 && X >= ph && Y >= pw, "maxpool2d_bwd: bad arguments");
   const int Xo = X / ph, Yo = Y / pw;
   maxpool2d_bwd_kernel<<<grid_for(NC * X * Y), 256, 0, (cudaStream_t)stream>>>(dy, (const uint8_t*)idx, dx, NC, X, Y, ph, pw, Xo, Yo);
   TMF_LAUNCH_CHECK();
